@@ -26,6 +26,8 @@ of a GPU once.  Streams are independent, so N GPUs = N*S streams, no collective 
           one 4K long-GOP stream cut at key frames into 8 segments over the N GPUs), kernel-only and end to end
 
 --impl reference times that CPU decoder alone (the reference has no GPU path).
+--dump-outputs DIR writes what the timed replay left in the streams after its last step (see dump_outputs), so
+that two builds can be compared output for output: the inputs are the same from run to run for the same arguments.
 """
 import argparse
 import hashlib
@@ -253,6 +255,38 @@ def kernel_only(torch, eng, stream, vp8_b200, payloads, passes, warm):
     return ms, frames_per_pass, sums, dec
 
 
+DUMP_BYTES = 64 * 10**6
+DUMP_SEED = 7122
+
+
+def dump_outputs(out_dir, eng, streams, sums, prefix="", budget=DUMP_BYTES):
+    """After the last timed step every stream holds the last frame it decoded; a caller reads it back as cropped
+    I420 (read_batch_packed).  Writes, at most `budget` bytes in all, each name preceded by `prefix`:
+      last_frame_checksums.npy : float64 (S, 2), the engine's 64-bit checksum of each stream's whole frame as its
+                                 high and low 32 bits
+      last_frame_samples.npy   : float32 (S, K), the I420 bytes at K positions of each stream's frame: all of them
+                                 when the S frames fit, else a sorted sample drawn with a fixed seed
+      last_frame_positions.npy : float64 (K,), those byte positions within the I420 frame"""
+    import numpy as np
+    S = len(streams)
+    k = min(FRAME_BYTES, (budget - 16 * S - 3 * 4096) // (4 * S + 8))  # 4096: room for the three .npy headers
+    if k == FRAME_BYTES:
+        pos = np.arange(FRAME_BYTES)
+    else:
+        pos = np.sort(np.random.default_rng(DUMP_SEED).choice(FRAME_BYTES, k, replace=False))
+    samples = np.empty((S, k), np.float32)
+    chunk = 64
+    buf = np.empty((chunk, FRAME_BYTES), np.uint8)
+    for i in range(0, S, chunk):
+        part = streams[i:i + chunk]
+        eng.read_batch_packed(part, buf.ctypes.data, FRAME_BYTES)
+        samples[i:i + len(part)] = buf[:len(part), pos]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, prefix + "last_frame_checksums.npy"), np.array([[s >> 32, s & 0xFFFFFFFF] for s in sums], np.float64))
+    np.save(os.path.join(out_dir, prefix + "last_frame_samples.npy"), samples)
+    np.save(os.path.join(out_dir, prefix + "last_frame_positions.npy"), pos.astype(np.float64))
+
+
 def small_case(torch, dist, world, eng, stream, vp8_b200, payloads, frame_bytes, passes=3):
     """One of the BASELINE configs on this rank's share `payloads` (may be empty).  Returns the whole-job
     kernel-only and end-to-end frames/s (max time over ranks)."""
@@ -369,7 +403,12 @@ def main():
                     help="mix: share of the streams whose macroblock headers are decoded on the GPU "
                          "(default 1 - 0.4/n_gpus: the host cores are shared by all ranks)")
     ap.add_argument("--serial-setup", action="store_true", help="generate the streams one at a time (for runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one left in the streams to DIR/*.npy "
+                         "(DIR/rank<r>_*.npy per rank when there are several)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -452,6 +491,9 @@ def main():
     clocks = sampler.stop()
     tm = eng.timers(reset=True)
     sums = eng.checksum_batch(dec.streams)  # last frame of every stream, compared below with the e2e pass
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, dec.streams, sums, "" if world == 1 else f"rank{rank}_", DUMP_BYTES // world)
+        eng.timers(reset=True)  # the read-back's pack kernels are not part of the end-to-end pass
     if world > 1:
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -2,6 +2,7 @@
 kernel against the pinned oracle, against the unmodified reference DECODER (what it reconstructs is what a decoder makes
 of its bitstream) and against the source (quality follows the quantiser)."""
 import ctypes as C
+import json
 import os
 import tempfile
 
@@ -9,6 +10,16 @@ import numpy as np
 import pytest
 
 import helpers
+
+SIZES = [(176, 144), (65, 33), (320, 240), (1280, 720)]
+QUANTISERS = ((100, 20), (40, 12), (8, 0))  # (q_index, loop filter level), coarse to fine
+# MD5s of the bitstream the encoder wrote and of the frame it reconstructed, per case, recorded from the encoder itself
+# by tests/golden/make_encoder_goldens.py: they pin its output against regressions, they are not reference output
+ENC_GOLDEN = os.path.join(helpers.ROOT, "tests", "golden", "enc", "encoder_key_frames.json")
+
+
+def golden_key(w, h, bpred, q):
+    return f"{w}x{h}-{'bpred' if bpred else '16x16'}-q{q}"
 
 
 def _image(w, h, seed):
@@ -57,16 +68,18 @@ def test_writer_is_the_inverse_of_the_parser(built):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("bpred", [False, True], ids=["16x16", "bpred"])
-@pytest.mark.parametrize("size", [(176, 144), (65, 33), (320, 240), (1280, 720)], ids=lambda s: f"{s[0]}x{s[1]}")
+@pytest.mark.parametrize("size", SIZES, ids=lambda s: f"{s[0]}x{s[1]}")
 def test_encoder_matches_oracle_and_reference_decoder(built, size, bpred):
     import vp8_b200
     from vp8_b200 import _capi
     w, h = size
+    with open(ENC_GOLDEN) as f:
+        gold = json.load(f)
     eng = vp8_b200.Engine(0)
     orc = C.CDLL(helpers.ORACLE_SO)
     try:
         last_psnr = None
-        for q, lf in ((100, 20), (40, 12), (8, 0)):
+        for q, lf in QUANTISERS:
             img = _image(w, h, 7 + q)
             st = eng.open_stream()
             (fr,) = eng.encode_key_frames([st], [img], w, h, q, loop_filter_level=lf, bpred=bpred)
@@ -92,15 +105,25 @@ def test_encoder_matches_oracle_and_reference_decoder(built, size, bpred):
                 assert (a.flags, a.coef_mask, a.coef_offset, a.aux[0], a.aux[1]) == (b.flags, b.coef_mask, b.coef_offset, b.aux[0], b.aux[1]), (q, m)
                 nb = bin(a.coef_mask).count("1")
                 assert d.payload[a.coef_offset * 16:(a.coef_offset + nb) * 16] == payload[b.coef_offset * 16:(b.coef_offset + nb) * 16], (q, m)
-            # (2) the bitstream, decoded by the UNMODIFIED reference decoder, is the frame the encoder holds
+            # (2) the bitstream and the frame are the recorded ones (ENC_GOLDEN, a regression pin), and the oracle decodes
+            # the bitstream to the frame the encoder holds; the oracle is tied to the reference decoder only through its
+            # golden-vector MD5s.  Where the UNMODIFIED reference decoder has been built (from sources outside the
+            # repository, oracle/Makefile) it has to decode the bitstream to that frame as well
             data = fr.write_bitstream()
-            with tempfile.TemporaryDirectory() as td:
-                path = os.path.join(td, "e.ivf")
-                vp8_b200.write_ivf(path, w, h, [data])
-                ref = helpers.ref_decode_ivf(path)
-            assert ref == recon, (size, q)
-            # (3) our own parser reads the records back
+            want = gold[golden_key(w, h, bpred, q)]
+            assert helpers.md5(data) == want["bitstream_md5"], (size, q)
+            assert helpers.md5(recon) == want["frame_md5"], (size, q)
             back = vp8_b200.Parser().parse(data)
+            oracle = helpers.Oracle()
+            assert oracle.decode(back) == recon, (size, q)
+            oracle.close()
+            if os.path.exists(helpers.REF_DECODE):
+                with tempfile.TemporaryDirectory() as td:
+                    path = os.path.join(td, "e.ivf")
+                    vp8_b200.write_ivf(path, w, h, [data])
+                    ref = helpers.ref_decode_ivf(path)
+                assert ref == recon, (size, q)
+            # (3) our own parser reads the records back
             db = back.desc()
             for m in range(cols * rows):
                 assert (db.mbs[m].flags, db.mbs[m].coef_mask, db.mbs[m].aux[0], db.mbs[m].aux[1]) == \
