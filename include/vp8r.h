@@ -275,6 +275,29 @@ VP8R_API int vp8r_read_batch_packed(vp8r_engine *e, int n, vp8r_stream *const *s
 VP8R_API int vp8r_read_batch_packed_as(vp8r_engine *e, int n, vp8r_stream *const *streams, uint8_t *dst,
                                        size_t stride, int async, int layout);
 
+/* Layouts only the device read-back below writes: BT.601 limited-range RGB of the cropped frame (the matrix of a VP8
+ * stream, color_space 0), 3*w*h bytes, chroma point-sampled (the sample at (x>>1, y>>1) serves its 2x2 pixels).  Per
+ * pixel, c = Y-16, d = U-128, e = V-128, with an arithmetic shift and a clamp to 0..255:
+ *   R = (298c + 409e + 128) >> 8,  G = (298c - 100d - 208e + 128) >> 8,  B = (298c + 516d + 128) >> 8 */
+#define VP8R_LAYOUT_RGB24      2  /* per pixel R,G,B bytes, rows of 3*w bytes (HWC) */
+#define VP8R_LAYOUT_RGB_PLANAR 3  /* R plane, G plane, B plane, each w*h bytes (CHW) */
+/* Writes the most recent frame of streams[i] to dst + i*stride in DEVICE memory of the engine's device, for consumers
+ * on the GPU (nothing crosses PCIe).  layout: VP8R_LAYOUT_I420 / _NV12 (vp8r_stream_frame_bytes(s) bytes, as the packed
+ * read-back writes them) or VP8R_LAYOUT_RGB24 / _RGB_PLANAR (3*w*h bytes).  Asynchronous on the engine's stream, behind
+ * its reconstruction kernels.
+ *
+ * consumer_stream: the cudaStream_t the caller reads dst on (e.g. torch's current stream).  NULL or the engine's own
+ * stream: nothing extra.  Otherwise, without blocking the host:
+ *   1. before the conversion the engine's stream waits for the work submitted to consumer_stream so far, so that dst
+ *      is not overwritten while earlier consumer work may still read it.  This wait also holds back every later
+ *      kernel on the engine's stream (the next time steps' reconstruction) until that consumer work has finished;
+ *   2. after the conversion consumer_stream waits for it, so work submitted there afterwards sees the frames.
+ * VP8R_ERR_INVALID_ARG: null engine / streams / dst, n <= 0, an unknown layout, stride smaller than a frame, dst not
+ * device memory of the engine's device (pinned, pageable and managed memory are refused); VP8R_ERR_STATE: a stream of
+ * another engine or without a frame. */
+VP8R_API int vp8r_read_batch_device(vp8r_engine *e, int n, vp8r_stream *const *streams, void *dst, size_t stride,
+                                    int layout, void *consumer_stream);
+
 /* ---- encoder (SURVEY.md section 8 row f4; the reference only sketches one: src/encode_frame.cc:30-244,
  * src/residual.cc:5-40,96-108, src/dct.cc:5-65, src/quantizer.cc:5-8; its encode.cc does not compile) ----
  *

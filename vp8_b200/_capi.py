@@ -75,6 +75,8 @@ SIGNATURES = {
                                          C.c_int, C.c_int, C.c_uint, C.POINTER(C.c_void_p)]),
     "vp8r_frame_write_bitstream": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "vp8r_read_batch_packed_as": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t, C.c_int, C.c_int]),
+    "vp8r_read_batch_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t, C.c_int,
+                                         C.c_void_p]),
     "vp8r_stream_read_frame": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
     "vp8r_stream_checksum": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "vp8r_checksum_batch": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),

@@ -95,7 +95,7 @@ class BatchDecoder:
     def wait(self, ticket):
         check(self._lib.vp8r_engine_wait(self.engine.handle, ticket))
 
-    def decode(self, payloads, out_ring=None, on_step=None, out_packed=None, shown_only=True, drain=True):
+    def decode(self, payloads, out_ring=None, on_step=None, out_packed=None, shown_only=True, drain=True, out_device=None):
         """payloads[s] = list of compressed frames of stream s.  out_ring: optional list of `depth` lists
         of (ptr, capacity) pinned host buffers, one per stream, that receive the frames of a time step
         (ring of `depth` steps).  out_packed: optional ((ptr0, ptr1, ...), stride): `depth` pinned host
@@ -107,6 +107,10 @@ class BatchDecoder:
         (new streams after reset(), same rings) then starts while they finish, as a server that is handed one set
         of streams after another would run; the ring entry of a step is (steps since the last drain) % depth, and the
         last call has to drain (or the caller calls engine.sync()).
+        out_device: optional (ring, layout): `depth` uint8 CUDA tensors on the engine's device; the frames of a time
+        step stay on the GPU, frame k of the step in row k of its ring entry (same indexing as out_packed), in `layout`
+        ("i420", "nv12", "rgb" or "rgb_planar", Engine.read_batch_device), ordered against torch's current stream.
+        These bytes do not count as d2h.  out_packed and out_device may be given together.
         Returns (frames decoded, frames shown, h2d bytes, d2h bytes)."""
         steps = max(len(p) for p in payloads)
         decoded = shown = h2d = d2h = 0
@@ -147,6 +151,9 @@ class BatchDecoder:
                 (ptrs, stride) = out_packed
                 self.engine.read_batch_packed([streams[k] for k in out_idx], ptrs[g % depth], stride, async_=True)
                 d2h += len(out_idx) * stride
+            if out_device is not None and out_idx:
+                ring, layout = out_device
+                self.engine.read_batch_device([streams[k] for k in out_idx], ring[g % depth], layout)
             tickets[g] = self.fence()
             hs["readback"] += clock() - t0
             if on_step:

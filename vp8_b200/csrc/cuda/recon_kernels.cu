@@ -1600,6 +1600,95 @@ __global__ void __launch_bounds__(256) PackKernel(const DevFrameJob *__restrict_
 }
 
 // ------------------------------------------------------------------------------------------
+// crop + BT.601 limited-range YUV -> RGB (vp8r_read_batch_device, VP8R_LAYOUT_RGB24 / _RGB_PLANAR).
+// Memory-bound (1.5 B read, 3 B written per pixel): one thread converts a strip of 16 x 2 pixels, which share 8
+// chroma samples, so the chroma terms are computed once per sample and every source row is one 128-bit load
+// (surface rows are 16-byte aligned and padded to whole macroblocks, so the loads never leave the surface).
+// ------------------------------------------------------------------------------------------
+constexpr int kRgbStripW = 16;
+
+// Stores the first n of the 4*NW bytes of w[] at d: 128-bit stores for a whole strip at a 16-byte aligned address
+// (every strip of a frame whose width is a multiple of 16, at an aligned destination), 32-bit stores at a 4-byte
+// aligned one, bytes otherwise (odd widths, the last strip of a row).
+template <int NW>
+__device__ __forceinline__ void StoreStrip(uint8_t *d, const unsigned (&w)[NW], int n) {
+  if (n == 4 * NW && ((size_t)d & 15) == 0) {
+#pragma unroll
+    for (int k = 0; k < NW; k += 4) *reinterpret_cast<uint4 *>(d + 4 * k) = make_uint4(w[k], w[k + 1], w[k + 2], w[k + 3]);
+  } else if (n == 4 * NW && ((size_t)d & 3) == 0) {
+#pragma unroll
+    for (int k = 0; k < NW; ++k) *reinterpret_cast<unsigned *>(d + 4 * k) = w[k];
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4 * NW; ++k)
+      if (k < n) d[k] = (uint8_t)(w[k >> 2] >> (8 * (k & 3)));
+  }
+}
+
+__global__ void __launch_bounds__(256) ConvertRgbKernel(const DevFrameJob *__restrict__ jobs) {
+  const DevFrameJob &job = jobs[blockIdx.y];
+  uint8_t *dst = job.pack_dst;
+  if (!dst) return;
+  const bool planar = job.pack_layout == VP8R_LAYOUT_RGB_PLANAR;
+  const int w = job.width, h = job.height;
+  const int strips = (w + kRgbStripW - 1) / kRgbStripW, items = strips * ((h + 1) / 2);
+  const size_t plane = (size_t)w * h;
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < items; t += gridDim.x * blockDim.x) {
+    const int pair = t / strips;
+    const int x = (t - pair * strips) * kRgbStripW, y = 2 * pair;
+    const int n = min(kRgbStripW, w - x);
+    const uint2 u8 = *reinterpret_cast<const uint2 *>(job.cur.u + (size_t)pair * job.pitch_c + x / 2);
+    const uint2 v8 = *reinterpret_cast<const uint2 *>(job.cur.v + (size_t)pair * job.pitch_c + x / 2);
+    // per chroma sample: the rounding constant and the U / V terms of each channel
+    int rc[8], gc[8], bc[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      const int d = (int)(((k < 4 ? u8.x : u8.y) >> (8 * (k & 3))) & 255) - 128;
+      const int e = (int)(((k < 4 ? v8.x : v8.y) >> (8 * (k & 3))) & 255) - 128;
+      rc[k] = 409 * e + 128;
+      gc[k] = 128 - 100 * d - 208 * e;
+      bc[k] = 516 * d + 128;
+    }
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {
+      if (y + r >= h) break;
+      const uint4 yv = *reinterpret_cast<const uint4 *>(job.cur.y + (size_t)(y + r) * job.pitch_y + x);
+      const unsigned yw[4] = {yv.x, yv.y, yv.z, yv.w};
+      int R[16], G[16], B[16];
+#pragma unroll
+      for (int p = 0; p < 16; ++p) {
+        const int c = 298 * ((int)((yw[p >> 2] >> (8 * (p & 3))) & 255) - 16);
+        R[p] = (c + rc[p >> 1]) >> 8;
+        G[p] = (c + gc[p >> 1]) >> 8;
+        B[p] = (c + bc[p >> 1]) >> 8;
+      }
+      const size_t row = (size_t)(y + r) * w + x;
+      if (planar) {
+        unsigned wr[4], wg[4], wb[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          wr[q] = PackSat4(R[4 * q], R[4 * q + 1], R[4 * q + 2], R[4 * q + 3]);
+          wg[q] = PackSat4(G[4 * q], G[4 * q + 1], G[4 * q + 2], G[4 * q + 3]);
+          wb[q] = PackSat4(B[4 * q], B[4 * q + 1], B[4 * q + 2], B[4 * q + 3]);
+        }
+        StoreStrip(dst + row, wr, n);
+        StoreStrip(dst + plane + row, wg, n);
+        StoreStrip(dst + 2 * plane + row, wb, n);
+      } else {
+        unsigned o[12];  // four pixels R,G,B,R G,B,R,G B,R,G,B per three words
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          o[3 * q] = PackSat4(R[4 * q], G[4 * q], B[4 * q], R[4 * q + 1]);
+          o[3 * q + 1] = PackSat4(G[4 * q + 1], B[4 * q + 1], R[4 * q + 2], G[4 * q + 2]);
+          o[3 * q + 2] = PackSat4(B[4 * q + 2], R[4 * q + 3], G[4 * q + 3], B[4 * q + 3]);
+        }
+        StoreStrip(dst + 3 * row, o, 3 * n);
+      }
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // host -> device staging by the SMs (zero-copy reads of pinned host memory)
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) CopyKernel(uint4 *__restrict__ dst, const uint4 *__restrict__ src, size_t n16) {
@@ -1637,6 +1726,13 @@ cudaError_t LaunchGather(const DevFrameJob *jobs, int n_frames, size_t max_bytes
 cudaError_t LaunchPack(const DevFrameJob *jobs, int n_frames, cudaStream_t st) {
   dim3 grid(48, n_frames);
   PackKernel<<<grid, 256, 0, st>>>(jobs);
+  return cudaGetLastError();
+}
+
+cudaError_t LaunchConvertRgb(const DevFrameJob *jobs, int n_frames, int max_w, int max_h, cudaStream_t st) {
+  const int items = (max_w + kRgbStripW - 1) / kRgbStripW * ((max_h + 1) / 2);
+  dim3 grid((unsigned)std::max(1, std::min(48, (items + 255) / 256)), n_frames);
+  ConvertRgbKernel<<<grid, 256, 0, st>>>(jobs);
   return cudaGetLastError();
 }
 

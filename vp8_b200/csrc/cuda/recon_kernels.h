@@ -52,12 +52,12 @@ struct DevFrameJob {
   int16_t dq[4][6];
   uint8_t key_frame, version, filter_type, lf_level, sharpness;
   uint8_t levels_in_one_launch;  // host-built level table walked by IntraLevelsKernel instead of one launch per level
-  uint8_t pack_layout;           // PackKernel: VP8R_LAYOUT_I420 / VP8R_LAYOUT_NV12
+  uint8_t pack_layout;           // PackKernel: VP8R_LAYOUT_I420 / _NV12; ConvertRgbKernel: VP8R_LAYOUT_RGB24 / _RGB_PLANAR
   uint8_t enc_flags;             // K_encode: VP8R_ENC_*
   // output side (crop / checksum)
   int width, height;
   unsigned long long *checksum;  // optional: receives the I420 checksum
-  uint8_t *pack_dst;             // optional: receives the cropped I420 image (device memory)
+  uint8_t *pack_dst;             // optional: receives the cropped image in pack_layout (device memory)
   // deferred tokens (K_tokens): vp8r_token_hdr + raw DCT partitions inside the frame's payload,
   // and the frame's device coefficient area (first block index relative to `payload`)
   const uint8_t *tok_hdr;
@@ -149,6 +149,9 @@ cudaError_t LaunchCopy(void *dst, const void *src_pinned, size_t bytes, cudaStre
 cudaError_t LaunchGather(const DevFrameJob *jobs, int n_frames, size_t max_bytes, cudaStream_t st);
 // Device-side crop + I420 pack of each job's current surface into job.pack_dst.
 cudaError_t LaunchPack(const DevFrameJob *jobs, int n_frames, cudaStream_t st);
+// Device-side crop + BT.601 YUV -> RGB (VP8R_LAYOUT_RGB24 / _RGB_PLANAR, from job.pack_layout) of each job's current
+// surface into job.pack_dst.  max_w, max_h: the largest frame of the batch (sizes the grid).
+cudaError_t LaunchConvertRgb(const DevFrameJob *jobs, int n_frames, int max_w, int max_h, cudaStream_t st);
 // Device-side checksum of the cropped I420 image of each job's current surface.
 cudaError_t LaunchChecksum(const DevFrameJob *jobs, int n_frames, cudaStream_t st);
 

@@ -131,6 +131,8 @@ struct vp8r_engine {
   cudaStream_t st_segments = nullptr;
   cudaEvent_t pack_done[kPackBufs] = {}, copy_done[kPackBufs] = {};
   bool copy_busy[kPackBufs] = {};
+  bool kernel_busy[kPackBufs] = {};  // pack_done of the part marks a device read-back (vp8r_read_batch_device) not yet waited for
+  cudaEvent_t consumer_ev = nullptr;  // vp8r_read_batch_device: the caller's stream, before the conversion
   cudaEvent_t fence_copy_ev[16] = {};
   bool fence_has_copy[16] = {};
   // checksum scratch
@@ -443,6 +445,25 @@ int EnsureScratchJobs(vp8r_engine *e, int n) {
   return VP8R_OK;
 }
 
+// Takes the next of the kPackBufs rotating parts of the scratch job table (and of the packed staging buffer) for a
+// read-back.  LaunchCopy reads a part from pinned host memory while its kernel runs, so the host rewrites the part
+// only after the work that last read it has finished: the D2H copy of a packed read-back (which follows its pack
+// kernel), or the kernel of a device read-back.
+int AcquirePart(vp8r_engine *e, int *part) {
+  e->pack_flip = (e->pack_flip + 1) % vp8r_engine::kPackBufs;
+  const int k = e->pack_flip;
+  if (e->copy_busy[k]) {
+    CU_TRY(cudaEventSynchronize(e->copy_done[k]));
+    e->copy_busy[k] = false;
+  }
+  if (e->kernel_busy[k]) {
+    CU_TRY(cudaEventSynchronize(e->pack_done[k]));
+    e->kernel_busy[k] = false;
+  }
+  *part = k;
+  return VP8R_OK;
+}
+
 // Error words of a batch whose kernels have finished: a stream with a truncated frame stops decoding (its frame
 // was not reconstructed, see JobFailed in the kernels) until its next key frame.  Returns the number of failures
 // and describes the first one.
@@ -548,6 +569,7 @@ VP8R_API int vp8r_engine_create(int device, void *cuda_stream, vp8r_engine **out
     cudaEventCreateWithFlags(&e->pack_done[k], cudaEventDisableTiming);
     cudaEventCreateWithFlags(&e->copy_done[k], cudaEventDisableTiming);
   }
+  cudaEventCreateWithFlags(&e->consumer_ev, cudaEventDisableTiming);
   err = vp8r::InitKernelTables();
   if (err != cudaSuccess) {
     SetError(std::string("kernel table upload: ") + cudaGetErrorString(err));
@@ -575,6 +597,7 @@ VP8R_API void vp8r_engine_destroy(vp8r_engine *e) {
     if (e->pack_done[k]) cudaEventDestroy(e->pack_done[k]);
     if (e->copy_done[k]) cudaEventDestroy(e->copy_done[k]);
   }
+  if (e->consumer_ev) cudaEventDestroy(e->consumer_ev);
   for (auto &ev : e->fence_copy_ev)
     if (ev) cudaEventDestroy(ev);
   for (auto &sl : e->slots) {
@@ -611,6 +634,7 @@ VP8R_API int vp8r_engine_sync(vp8r_engine *e) {
   CU_TRY(cudaStreamSynchronize(e->st));
   CU_TRY(cudaStreamSynchronize(e->st_copy));
   for (bool &b : e->copy_busy) b = false;
+  for (bool &b : e->kernel_busy) b = false;
   for (auto &sl : e->slots) {
     sl.pending = false;
     std::string what;
@@ -1213,6 +1237,7 @@ VP8R_API int vp8r_read_batch_packed_as(vp8r_engine *e, int n, vp8r_stream *const
     CU_TRY(cudaStreamSynchronize(e->st));
     CU_TRY(cudaStreamSynchronize(e->st_copy));
     for (bool &b : e->copy_busy) b = false;
+    for (bool &b : e->kernel_busy) b = false;
     if (e->d_pack) cudaFree(e->d_pack);
     e->d_pack = nullptr;
     const size_t half = (bytes + 255) & ~size_t(255);
@@ -1224,15 +1249,12 @@ VP8R_API int vp8r_read_batch_packed_as(vp8r_engine *e, int n, vp8r_stream *const
   // kPackBufs parts of the job table and of the staging buffer rotate: the pack kernel of this call
   // runs on the engine's stream while the D2H copy of the previous call may still be in flight on
   // the copy stream.
-  e->pack_flip = (e->pack_flip + 1) % vp8r_engine::kPackBufs;
-  const int half = e->pack_flip;
+  int half = 0;
+  rc = AcquirePart(e, &half);
+  if (rc) return rc;
   uint8_t *stage = e->d_pack + size_t(half) * e->pack_cap;
   DevFrameJob *hj = e->h_cjobs + size_t(half) * e->cap_cjobs;
   DevFrameJob *dj = e->d_cjobs + size_t(half) * e->cap_cjobs;
-  if (e->copy_busy[half]) {  // the copy that last read this part (kPackBufs calls ago) must be done
-    CU_TRY(cudaEventSynchronize(e->copy_done[half]));  // host side: hj is about to be rewritten
-    e->copy_busy[half] = false;
-  }
   for (int i = 0; i < n; ++i) {
     DevFrameJob &j = hj[i];
     std::memset(&j, 0, sizeof(j));
@@ -1255,6 +1277,79 @@ VP8R_API int vp8r_read_batch_packed_as(vp8r_engine *e, int n, vp8r_stream *const
     CU_TRY(cudaStreamSynchronize(e->st_copy));
     e->copy_busy[half] = false;
   }
+  return VP8R_OK;
+}
+
+VP8R_API int vp8r_read_batch_device(vp8r_engine *e, int n, vp8r_stream *const *streams, void *dst, size_t stride,
+                                    int layout, void *consumer_stream) {
+  // argument checks that need no device come first
+  if (!e || !streams || !dst) {
+    SetError("vp8r_read_batch_device: null engine, streams or destination");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (n <= 0) {
+    SetError("vp8r_read_batch_device: n <= 0");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
+    SetError("vp8r_read_batch_device: unknown layout " + std::to_string(layout));
+    return VP8R_ERR_INVALID_ARG;
+  }
+  const bool rgb = layout == VP8R_LAYOUT_RGB24 || layout == VP8R_LAYOUT_RGB_PLANAR;
+  int max_w = 0, max_h = 0;
+  for (int i = 0; i < n; ++i) {
+    const vp8r_stream *s = streams[i];
+    if (!s || s->eng != e || !s->have_frame) {
+      SetError("stream has no reconstructed frame");
+      return VP8R_ERR_STATE;
+    }
+    const size_t bytes = rgb ? 3 * size_t(s->width) * s->height : vp8r_stream_frame_bytes(s);
+    if (bytes > stride) {
+      SetError("stride smaller than a frame");
+      return VP8R_ERR_INVALID_ARG;
+    }
+    max_w = std::max(max_w, s->width);
+    max_h = std::max(max_h, s->height);
+  }
+  int rc = EnsureDevice(e);
+  if (rc) return rc;
+  cudaPointerAttributes attr{};
+  if (cudaPointerGetAttributes(&attr, dst) != cudaSuccess) {
+    cudaGetLastError();
+    attr.type = cudaMemoryTypeUnregistered;
+  }
+  if (attr.type != cudaMemoryTypeDevice || attr.device != e->device) {
+    SetError("vp8r_read_batch_device: dst is not device memory of the engine's device (pinned, pageable and managed "
+             "memory are refused)");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  rc = EnsureScratchJobs(e, n);
+  if (rc) return rc;
+  int part = 0;
+  rc = AcquirePart(e, &part);
+  if (rc) return rc;
+  DevFrameJob *hj = e->h_cjobs + size_t(part) * e->cap_cjobs;
+  DevFrameJob *dj = e->d_cjobs + size_t(part) * e->cap_cjobs;
+  for (int i = 0; i < n; ++i) {
+    DevFrameJob &j = hj[i];
+    std::memset(&j, 0, sizeof(j));
+    FillJobSurfaces(streams[i], streams[i]->ref[0], &j);
+    j.pack_dst = static_cast<uint8_t *>(dst) + size_t(i) * stride;
+    j.pack_layout = uint8_t(layout);
+  }
+  cudaStream_t consumer = static_cast<cudaStream_t>(consumer_stream);
+  const bool cross = consumer && consumer != e->st;
+  if (cross) {  // earlier consumer work may still read dst
+    CU_TRY(cudaEventRecord(e->consumer_ev, consumer));
+    CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
+  }
+  CU_TRY(vp8r::LaunchCopy(dj, hj, sizeof(DevFrameJob) * n, e->st));
+  if (rgb) CU_TRY(vp8r::LaunchConvertRgb(dj, n, max_w, max_h, e->st));
+  else CU_TRY(vp8r::LaunchPack(dj, n, e->st));
+  e->acc.launches_other++;
+  CU_TRY(cudaEventRecord(e->pack_done[part], e->st));
+  e->kernel_busy[part] = true;
+  if (cross) CU_TRY(cudaStreamWaitEvent(consumer, e->pack_done[part], 0));
   return VP8R_OK;
 }
 
