@@ -21,5 +21,7 @@ $NVCC $ARCH -shared -o "$OUT/libvp8r.so" vp8_b200/_build/recon_kernels.o vp8_b20
 g++ -O2 -std=c++17 -Wall -Wextra tools/vp8synth.cc -o "$OUT/vp8synth"
 g++ -O2 -std=c++17 -Wall -Wextra -Iinclude tools/vp8dec.cc -o "$OUT/vp8dec" -L"$OUT" -lvp8r -Wl,-rpath,'$ORIGIN'
 make -s -C oracle oracle
+mkdir -p oracle_inter/_build
+gcc -std=c11 -O2 -fPIC -shared -Wall -Wextra -Iinclude -Ioracle -o oracle_inter/_build/liboracle_inter.so oracle_inter/enc_inter_oracle.c
 if [ "${SKIP_REF:-0}" != "1" ]; then make -s -C oracle ref; fi
 echo "built $OUT/libvp8r.so"

@@ -317,9 +317,28 @@ VP8R_API int vp8r_read_batch_device(vp8r_engine *e, int n, vp8r_stream *const *s
 VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
                                     int width, int height, int q_index, int loop_filter_level, int sharpness,
                                     unsigned flags, vp8r_frame *const *out);
-/* The inverse of vp8r_parser_parse for key frames: serialises f (key frame, intra macroblocks, one quantiser) into a
- * VP8 frame with one DCT partition and the default token probabilities.  *size receives the number of bytes needed;
- * VP8R_ERR_INVALID_ARG when cap is too small (call again) or the frame cannot be written. */
+/* vp8r_encode_inter_frames: one INTER frame for each of n different streams, from cropped I420 images in host memory
+ * (the same conventions as vp8r_encode_key_frames).  Every macroblock predicts from the stream's current LAST frame
+ * (made by vp8r_encode_key_frames, by an earlier inter encode or by decoding) with one motion vector; there are no
+ * intra or SPLIT macroblocks.  On the device, one warp per macroblock: full-pel search over +-search_range whole pixels
+ * around the zero vector, then half-pel and quarter-pel refinement, by cost = luma SAD + lambda(q) * bits(vector)
+ * (the lowest candidate index wins a tie), residual, forward DCT / WHT and quantisation; the decoder's own inter
+ * reconstruction, loop filter and border extension then run on the records, so that stream k afterwards holds exactly
+ * the frame a decoder makes of the written bitstream.  The host then gives every vector the cheapest mode consistent
+ * with it (NEAREST / NEAR / ZERO / NEW).  out[k]: complete records (mode bits included, coef_offset = 25*mb) and
+ * coefficient blocks, n_coef_blocks and n_inter_mbs set; header: show_frame 1, refresh_last 1, golden and altref
+ * neither refreshed nor copied, sign biases 0, version 0.  References move as for a decoded inter frame.  Synchronous.
+ * VP8R_ERR_INVALID_ARG: the key-frame call's argument checks, or search_range outside 4..24; VP8R_ERR_STATE: a stream
+ * without a frame, whose frame is not width x height, or that has failed. */
+VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
+                                      int width, int height, int q_index, int loop_filter_level, int sharpness,
+                                      int search_range, vp8r_frame *const *out);
+/* The inverse of vp8r_parser_parse: serialises f into a VP8 frame with one DCT partition and the default token, mode and
+ * motion-vector probabilities.  Key frames: intra macroblocks.  Inter frames: the frame header's refresh, copy,
+ * sign-bias and show_frame fields from f's header, intra macroblocks, and inter macroblocks of any reference coded
+ * NEAREST / NEAR / ZERO / NEW.  Both: no segmentation, no loop-filter deltas, the five quantiser deltas that reproduce
+ * hdr.dq[0] from q_index.  SPLIT macroblocks and a vector that contradicts its mode are refused.  *size receives the
+ * number of bytes needed; VP8R_ERR_INVALID_ARG when cap is too small (call again) or the frame cannot be written. */
 VP8R_API int vp8r_frame_write_bitstream(const vp8r_frame *f, uint8_t *dst, size_t cap, size_t *size);
 
 /* Device-side checksum of the cropped I420 image: low word sum(b_i), high word

@@ -157,7 +157,7 @@ VP8R_API int vp8r_frame_write_bitstream(const vp8r_frame *f, uint8_t *dst, size_
   if (!f || !size) return VP8R_ERR_INVALID_ARG;
   std::vector<uint8_t> bytes;
   std::string err;
-  const int rc = vp8r::WriteKeyFrame(*f, &bytes, &err);
+  const int rc = vp8r::WriteFrame(*f, &bytes, &err);
   if (rc != VP8R_OK) {
     vp8r::SetError(err);
     return rc;

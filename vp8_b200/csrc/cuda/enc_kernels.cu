@@ -14,6 +14,7 @@
 // column c+1).  Lane b < 24 owns 4x4 block b (16 Y raster, 4 U, 4 V), lane 24 the Y2 block.  Everything of a block
 // stays in the lane's registers: source pixels, the four candidate predictions and their errors (summed over the
 // warp with REDUX), residual, forward DCT, quantisation, dequantisation, inverse DCT, reconstruction.
+#include "enc_cost.h"
 #include "recon_kernels.h"
 
 namespace vp8r {
@@ -479,6 +480,267 @@ __global__ void __launch_bounds__(kEncWarps * 32) EncodeIntraKernel(const DevFra
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// K_encode_inter: inter frames whose macroblocks all predict from LAST with one vector each.  No pixel of such a frame
+// depends on another pixel of the same frame, so every macroblock is searched and transformed on its own, one warp
+// each, all frames of the batch in one launch; the reconstruction is the decoder's own K_inter on the records written
+// here (the host assigns the modes afterwards, from the vectors).
+//
+// Per macroblock: the source luma and a window of the LAST luma plane (rows -(R+3) .. 15+R+3, columns -32 .. 47
+// around the macroblock; the surface's 32-pixel border makes any clamp unnecessary for R <= 24) are staged in shared
+// memory by 128-bit loads.  Full-pel search over |dy|, |dx| <= R, candidates split over the lanes, SAD by
+// vabsdiff4-with-accumulate, cost = SAD + lambda * R(v) (enc_cost.h), minimum of (cost << 12) | candidate index by
+// REDUX (ties: the lowest index, index = (dy + R) * (2R + 1) + dx + R).  Then half-pel and quarter-pel refinement:
+// the eight neighbours of the current best (enc_cost.h's ring order, the centre kept on a tie), four lanes per
+// candidate, the prediction computed exactly as the decoder computes it (six-tap, horizontal pass over the rows
+// -2..+3 around each output row, rounding (x + 64) >> 7 and a clamp to 0..255 after each pass; whole-pel
+// positions are the identity filter).  Finally the prediction of luma and of chroma (the decoder's chroma vector
+// of a non-SPLIT macroblock), residual, forward DCT / WHT and quantisation as in K_encode.
+namespace {
+
+constexpr int kEncInterWarps = 4;
+constexpr int kEncSearchMax = 24;
+constexpr int kWinTop = kEncSearchMax + 3;       // window row of the macroblock's first row
+constexpr int kWinRows = 16 + 2 * kWinTop;       // 70
+constexpr int kWinLeft = 32;                     // window column of the macroblock's first column
+constexpr int kWinW = 16 + 2 * kWinLeft;         // 80 bytes: five 128-bit words per row
+
+struct __align__(16) EncInterScratch {
+  unsigned char win[kWinRows][kWinW];
+  unsigned src[64];                 // source luma, row y at words 4y..4y+3
+  unsigned pred[64];                // luma prediction of the chosen vector, same layout
+  unsigned char cpred[2][8][8];     // U, V prediction
+  short y2[16];
+};
+
+__constant__ int c_enc_sixtap[8][6] = {  // RFC 6386 section 14.4 (src/inter_predict.h:18-27)
+    {0, 0, 128, 0, 0, 0},  {0, -6, 123, 12, -1, 0},   {2, -11, 108, 36, -8, 1}, {0, -9, 93, 50, -6, 0},
+    {3, -16, 77, 77, -16, 3}, {0, -6, 50, 93, -9, 0}, {1, -8, 36, 108, -11, 2}, {0, -1, 12, 123, -6, 0}};
+
+__device__ __forceinline__ unsigned Vabsdiff4Add(unsigned a, unsigned b, unsigned c) {
+  unsigned d;
+  asm("vabsdiff4.u32.u32.u32.add %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+  return d;
+}
+
+__device__ __forceinline__ int Tap6(const int *t, int p0, int p1, int p2, int p3, int p4, int p5) {
+  return clamp255e((t[0] * p0 + t[1] * p1 + t[2] * p2 + t[3] * p3 + t[4] * p4 + t[5] * p5 + 64) >> 7);
+}
+
+// Luma prediction of rows y0..y0+NR-1, columns x0..x0+NC-1 (NC a multiple of 4) of the macroblock for the vector
+// (mr, mc) in 1/8 pel, from the staged window.  kStore: into s.pred; otherwise returns the SAD against s.src.
+template <int NR, int NC, bool kStore>
+__device__ __forceinline__ unsigned PredictLuma(EncInterScratch &s, int mr, int mc, int y0, int x0) {
+  int th[6], tv[6];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) {
+    th[k] = c_enc_sixtap[mc & 7][k];
+    tv[k] = c_enc_sixtap[mr & 7][k];
+  }
+  const int row0 = kWinTop + y0 + (mr >> 3) - 2, col0 = kWinLeft + x0 + (mc >> 3) - 2;
+  unsigned sad = 0;
+#pragma unroll 1
+  for (int x4 = 0; x4 < NC; x4 += 4) {
+    unsigned out[NR];
+#pragma unroll
+    for (int y = 0; y < NR; ++y) out[y] = 0;
+#pragma unroll
+    for (int xx = 0; xx < 4; ++xx) {
+      const unsigned char *w = &s.win[row0][col0 + x4 + xx];
+      int h[NR + 5];
+#pragma unroll
+      for (int i = 0; i < NR + 5; ++i) {
+        const unsigned char *q = w + i * kWinW;
+        h[i] = Tap6(th, q[0], q[1], q[2], q[3], q[4], q[5]);
+      }
+#pragma unroll
+      for (int y = 0; y < NR; ++y) out[y] |= (unsigned)Tap6(tv, h[y], h[y + 1], h[y + 2], h[y + 3], h[y + 4], h[y + 5]) << (8 * xx);
+    }
+#pragma unroll
+    for (int y = 0; y < NR; ++y) {
+      const int at = 4 * (y0 + y) + ((x0 + x4) >> 2);
+      if (kStore) s.pred[at] = out[y];
+      else sad = Vabsdiff4Add(out[y], s.src[at], sad);
+    }
+  }
+  return sad;
+}
+
+}  // namespace
+
+__global__ void __launch_bounds__(kEncInterWarps * 32) EncodeInterKernel(const DevFrameJob *__restrict__ jobs) {
+  __shared__ EncInterScratch s_scratch[kEncInterWarps];
+  const DevFrameJob &job = jobs[blockIdx.z];
+  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
+  const int mb_r = blockIdx.y, mb_c = blockIdx.x * kEncInterWarps + warp, cols = job.mb_cols;
+  if (!job.enc_src[0] || mb_r >= job.mb_rows || mb_c >= cols) return;
+  EncInterScratch &s = s_scratch[warp];
+  const int R = job.enc_search_range;
+
+  // ---- stage the source macroblock and the search window ----
+  {
+    const int sp = job.enc_src_pitch_y;
+    if (lane < 16)
+      reinterpret_cast<uint4 *>(s.src)[lane] =
+          *reinterpret_cast<const uint4 *>(job.enc_src[0] + (ptrdiff_t)(mb_r * 16 + lane) * sp + mb_c * 16);
+    const int r_lo = kWinTop - (R + 3), n_rows = 16 + 2 * (R + 3);
+    const uint8_t *ref = job.ref[1].y + (ptrdiff_t)(mb_r * 16 - kWinTop) * job.pitch_y + mb_c * 16 - kWinLeft;
+    for (int i = lane; i < n_rows * 5; i += 32) {
+      const int row = r_lo + i / 5, q = i % 5;
+      reinterpret_cast<uint4 *>(s.win[row])[q] = *reinterpret_cast<const uint4 *>(ref + (ptrdiff_t)row * job.pitch_y + 16 * q);
+    }
+  }
+  __syncwarp();
+  const int lambda = vp8r_enc_lambda(job.dq[0][VP8R_DQ_Y1_AC]);
+
+  // ---- full-pel search ----
+  unsigned best = 0xffffffffu;
+  {
+    const int span = 2 * R + 1, n_cand = span * span;
+#pragma unroll 1
+    for (int i = lane; i < n_cand; i += 32) {
+      const int dy = i / span - R, dx = i - (i / span) * span - R;
+      const int col = kWinLeft + dx;
+      const unsigned sh = (col & 3) * 8;
+      unsigned sad = 0;
+#pragma unroll 4
+      for (int y = 0; y < 16; ++y) {
+        const unsigned *p = reinterpret_cast<const unsigned *>(s.win[kWinTop + dy + y]) + (col >> 2);
+        const unsigned a0 = p[0], a1 = p[1], a2 = p[2], a3 = p[3], a4 = p[4];
+        sad = Vabsdiff4Add(__funnelshift_r(a0, a1, sh), s.src[4 * y + 0], sad);
+        sad = Vabsdiff4Add(__funnelshift_r(a1, a2, sh), s.src[4 * y + 1], sad);
+        sad = Vabsdiff4Add(__funnelshift_r(a2, a3, sh), s.src[4 * y + 2], sad);
+        sad = Vabsdiff4Add(__funnelshift_r(a3, a4, sh), s.src[4 * y + 3], sad);
+      }
+      const unsigned cost = sad + (unsigned)(lambda * vp8r_enc_mv_bits(4 * dy, 4 * dx));
+      best = min(best, (cost << 12) | (unsigned)i);
+    }
+    best = __reduce_min_sync(0xffffffffu, best);
+  }
+  const int span = 2 * R + 1, bi = (int)(best & 4095u);
+  int qr = 4 * (bi / span - R), qc = 4 * (bi % span - R);  // quarter pel
+  unsigned centre = best >> 12;
+
+  // ---- half-pel, then quarter-pel refinement: four lanes per neighbour, rows 4*(lane&3) .. +3 ----
+#pragma unroll 1
+  for (int step = 2; step >= 1; step >>= 1) {
+    const int k = lane >> 2, part = lane & 3;
+    const int cr = qr + step * vp8r_enc_ring_dr(k), cc = qc + step * vp8r_enc_ring_dc(k);
+    unsigned sad = PredictLuma<4, 16, false>(s, 2 * cr, 2 * cc, 4 * part, 0);
+    sad += __shfl_xor_sync(0xffffffffu, sad, 1);
+    sad += __shfl_xor_sync(0xffffffffu, sad, 2);
+    const unsigned cost = sad + (unsigned)(lambda * vp8r_enc_mv_bits(cr, cc));
+    const unsigned key = __reduce_min_sync(0xffffffffu, min((cost << 4) | (unsigned)(k + 1), centre << 4));
+    const int won = (int)(key & 15u);
+    if (won) {
+      qr += step * vp8r_enc_ring_dr(won - 1);
+      qc += step * vp8r_enc_ring_dc(won - 1);
+    }
+    centre = key >> 4;
+  }
+  const int mvr = 2 * qr, mvc = 2 * qc;  // 1/8 pel, as vp8r_mb_info.mv
+
+  // ---- prediction of the chosen vector: luma row lane>>1, half lane&1; chroma plane lane>>4, row, half ----
+  PredictLuma<1, 8, true>(s, mvr, mvc, lane >> 1, 8 * (lane & 1));
+  {
+    // chroma vector of a non-SPLIT macroblock (src/inter_predict.cc:116-144), as K_inter derives it
+    const int sr = s16e(4 * mvr), sc = s16e(4 * mvc);
+    const int ar = (abs(sr) + 4) >> 3, ac = (abs(sc) + 4) >> 3;
+    const int cmr = sr < 0 ? -ar : ar, cmc = sc < 0 ? -ac : ac;
+    const int pl = lane >> 4, y = (lane >> 1) & 7, x0 = 4 * (lane & 1);
+    int th[6], tv[6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+      th[k] = c_enc_sixtap[cmc & 7][k];
+      tv[k] = c_enc_sixtap[cmr & 7][k];
+    }
+    const uint8_t *base = (pl ? job.ref[1].v : job.ref[1].u) + (ptrdiff_t)(mb_r * 8 + y + (cmr >> 3) - 2) * job.pitch_c + mb_c * 8 + x0 +
+                          (cmc >> 3) - 2;
+#pragma unroll
+    for (int xx = 0; xx < 4; ++xx) {
+      int h[6];
+#pragma unroll
+      for (int i = 0; i < 6; ++i) {
+        const uint8_t *q = base + (ptrdiff_t)i * job.pitch_c + xx;
+        h[i] = Tap6(th, __ldg(q), __ldg(q + 1), __ldg(q + 2), __ldg(q + 3), __ldg(q + 4), __ldg(q + 5));
+      }
+      s.cpred[pl][y][x0 + xx] = (unsigned char)Tap6(tv, h[0], h[1], h[2], h[3], h[4], h[5]);
+    }
+  }
+  __syncwarp();
+
+  // ---- residual, forward transform, quantisation (lane b < 24: block b; lane 24: Y2) ----
+  const bool luma = lane < 16, is_block = lane < 24;
+  const int16_t *dq = job.dq[0];
+  const int f_dc = lane == 24 ? dq[VP8R_DQ_Y2_DC] : (luma ? dq[VP8R_DQ_Y1_DC] : dq[VP8R_DQ_UV_DC]);
+  const int f_ac = lane == 24 ? dq[VP8R_DQ_Y2_AC] : (luma ? dq[VP8R_DQ_Y1_AC] : dq[VP8R_DQ_UV_AC]);
+  int m[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) m[i] = 0;
+  if (is_block) {
+    unsigned src[4], pred[4];
+    if (luma) {
+      const int bi4 = lane >> 2, bj = lane & 3;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        src[k] = s.src[4 * (4 * bi4 + k) + bj];
+        pred[k] = s.pred[4 * (4 * bi4 + k) + bj];
+      }
+    } else {
+      const int pl = lane >= 20, b = (lane - 16) & 3, bi2 = b >> 1, bj = b & 1;
+      const int sp = job.enc_src_pitch_c;
+      const uint8_t *sp_base = job.enc_src[1 + pl] + (ptrdiff_t)(mb_r * 8 + 4 * bi2) * sp + mb_c * 8 + 4 * bj;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        src[k] = *reinterpret_cast<const unsigned *>(sp_base + (ptrdiff_t)k * sp);
+        pred[k] = *reinterpret_cast<const unsigned *>(&s.cpred[pl][4 * bi2 + k][4 * bj]);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+#pragma unroll
+      for (int x = 0; x < 4; ++x) m[4 * k + x] = (int)((src[k] >> (8 * x)) & 0xff) - (int)((pred[k] >> (8 * x)) & 0xff);
+    Fdct4x4(m);
+  }
+  if (luma) s.y2[lane] = (short)m[0];
+  __syncwarp();
+  if (lane == 24) {
+#pragma unroll
+    for (int i = 0; i < 16; ++i) m[i] = s.y2[i];
+    Fwht4x4(m);
+  }
+  bool nz = false;
+  if (lane <= 24) {
+    m[0] = luma ? 0 : s16e(m[0] / f_dc);  // a luma block's DC travels in the Y2 block
+#pragma unroll
+    for (int i = 1; i < 16; ++i) m[i] = s16e(m[i] / f_ac);
+#pragma unroll
+    for (int i = 0; i < 16; ++i) nz |= m[i] != 0;
+  }
+  const unsigned lanes_nz = __ballot_sync(0xffffffffu, nz);
+  const unsigned coef_mask = ((lanes_nz & 0x00ffffffu) << 1) | ((lanes_nz >> 24) & 1u);
+  const int mb_index = mb_r * cols + mb_c;
+  const unsigned coef_offset = (unsigned)mb_index * 25u;
+  if (nz) {
+    const int blk = lane < 24 ? lane + 1 : 0;
+    const int at = __popc(coef_mask & ((1u << blk) - 1u));
+    int4 *dst = reinterpret_cast<int4 *>(const_cast<int16_t *>(job.payload) + (size_t)(coef_offset + at) * 16);
+    unsigned w[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) w[i] = ((unsigned)m[2 * i] & 0xffffu) | ((unsigned)m[2 * i + 1] << 16);
+    dst[0] = make_int4((int)w[0], (int)w[1], (int)w[2], (int)w[3]);
+    dst[1] = make_int4((int)w[4], (int)w[5], (int)w[6], (int)w[7]);
+  }
+  if (lane == 0) {
+    const unsigned flags = VP8R_MB_IS_INTER | (1u << VP8R_MB_REF_SHIFT) | VP8R_MB_HAS_Y2 | ((unsigned)job.lf_level << VP8R_MB_LF_SHIFT) |
+                           (coef_mask ? VP8R_MB_LF_INNER : 0u);
+    const unsigned mv = ((unsigned)mvr & 0xffffu) | ((unsigned)mvc << 16);
+    int4 *rec = reinterpret_cast<int4 *>(const_cast<vp8r_mb_info *>(job.mbs) + mb_index);
+    rec[0] = make_int4((int)flags, (int)coef_mask, (int)coef_offset, (int)mv);
+    rec[1] = make_int4(0, 0, 0, 0);
+  }
+}
+
 cudaError_t InitEncodeTables(const unsigned short *bpred_lut) {
   return cudaMemcpyToSymbol(c_enc_bpred_lut, bpred_lut, sizeof(unsigned short) * 160);
 }
@@ -486,6 +748,13 @@ cudaError_t InitEncodeTables(const unsigned short *bpred_lut) {
 cudaError_t LaunchEncodeIntra(const DevFrameJob *jobs, int n_frames, int max_rows, cudaStream_t st) {
   const size_t smem = ((size_t(max_rows) * 4 + 15) & ~size_t(15)) + 320 + sizeof(EncScratch) * kEncWarps;
   EncodeIntraKernel<<<n_frames, kEncWarps * 32, smem, st>>>(jobs);
+  return cudaGetLastError();
+}
+
+cudaError_t LaunchEncodeInter(const DevFrameJob *jobs, int n_frames, int max_cols, int max_rows, cudaStream_t st) {
+  if (max_rows > 65535 || n_frames > 65535) return cudaErrorInvalidValue;
+  dim3 grid((max_cols + kEncInterWarps - 1) / kEncInterWarps, max_rows, n_frames);
+  EncodeInterKernel<<<grid, kEncInterWarps * 32, 0, st>>>(jobs);
   return cudaGetLastError();
 }
 

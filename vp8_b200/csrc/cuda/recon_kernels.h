@@ -81,6 +81,7 @@ struct DevFrameJob {
   // then OUTPUTS (25 coefficient blocks reserved per macroblock)
   const uint8_t *enc_src[3];
   int enc_src_pitch_y, enc_src_pitch_c;
+  int enc_search_range;          // K_encode_inter: full-pel search range (whole pixels, 4..24)
 };
 
 // A frame whose device-side parse ran past the end of a partition: its records are not trustworthy, so no
@@ -122,6 +123,10 @@ cudaError_t LaunchIntraFlat(const DevFrameJob *jobs, int n_frames, int level, in
 // K_encode: closed-loop key-frame encoder (mode decision, forward transform, quantisation, reconstruction) of every
 // job with enc_src set; the loop filter follows as for a decoded frame.
 cudaError_t LaunchEncodeIntra(const DevFrameJob *jobs, int n_frames, int max_rows, cudaStream_t st);
+// K_encode_inter: motion search against LAST (ref[1]), residual, forward transform and quantisation of every
+// macroblock of every job with enc_src set, one warp per macroblock; writes records (vector, coef_mask, flags
+// without mode bits) and coefficient blocks.  K_inter, the loop filter and the border follow as for a decoded frame.
+cudaError_t LaunchEncodeInter(const DevFrameJob *jobs, int n_frames, int max_cols, int max_rows, cudaStream_t st);
 // Up to eight frames with the same geometry and filter type (and a non-zero frame filter level) that one
 // warp of the batch loop filter walks together; unused slots are -1, slot 0 is always used.
 struct FilterGroup {

@@ -1,4 +1,4 @@
-// Key-frame bitstream writer: the inverse of FrameParser for the frames the encoder produces (row f4).
+// Bitstream writer: the inverse of FrameParser for the frames the encoder produces (row f4).
 #ifndef VP8R_HOST_FRAME_WRITER_H_
 #define VP8R_HOST_FRAME_WRITER_H_
 
@@ -10,13 +10,22 @@
 
 namespace vp8r {
 
-// Serialises a parsed-frame structure (key frame, intra macroblocks with 16x16 or B_PRED luma modes, one
-// quantiser, no segmentation, no loop-filter deltas, one DCT partition) into a VP8 frame (RFC 6386 sections 9,
-// 19.2, 19.3, 13): frame tag + start code + dimensions, first partition (headers, "keep the default token
-// probabilities", per-macroblock skip flag and modes), token partition with the default probabilities.
-// Parsing the result with FrameParser gives back the same macroblock records and coefficient blocks.
-// Returns VP8R_OK or an error code with *err set.
-int WriteKeyFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err);
+// Seriali// Serialises a parsed-frame structure into a VP8 frame (RFC 6386 sections 9, 19.2, 19.3, 13): frame tag (+ start
+// code and dimensions of a key frame), first partition (headers, "keep the default token / mode / motion-vector
+// probabilities", per-macroblock skip flag, modes and motion vectors), one token partition with the default
+// probabilities.  Frames it can write: one DCT partition, no segmentation, no loop-filter deltas, quantiser factors
+// that q_index and five deltas reproduce; key frames with intra macroblocks, inter frames with intra macroblocks
+// and inter macroblocks of any reference coded NEAREST / NEAR / ZERO / NEW (SPLIT is refused, and so is a vector
+// that contradicts its mode).  Parsing the result with FrameParser gives back the same macroblock records and
+// coefficient blocks.  Returns VP8R_OK or an error code with *err set.
+int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err);
+
+// Mode bits of the inter macroblocks of a frame whose records carry vectors but no modes (the encoder's): walking
+// the macroblocks in raster order, each vector gets the cheapest mode consistent with it under the mode tree's
+// probabilities (NEAREST if it equals the nearest vector, NEAR if the near one, ZERO if it is zero; the most probable
+// of those that apply, else NEW).  The vector itself is never changed.  Sign biases are taken as 0.
+// VP8R_ERR_INVALID_ARG when a NEW vector lies too far from its predictor (|delta| > 1023 quarter pels).
+int AssignInterModes(vp8r_mb_info *mbs, int cols, int rows, std::string *err);
 
 }  // namespace vp8r
 

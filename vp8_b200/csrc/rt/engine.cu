@@ -16,6 +16,7 @@
 
 #include "../cuda/recon_kernels.h"
 #include "../host/frame_parser.h"
+#include "../host/frame_writer.h"
 #include "../host/parsed_frame.h"
 #include "error.h"
 #include "vp8r.h"
@@ -503,6 +504,27 @@ void FillJobSurfaces(const vp8r_stream *s, int cur, DevFrameJob *j) {
   j->mb_rows = s->mb_rows;
   j->width = s->width;
   j->height = s->height;
+}
+
+// Encoder input: a cropped I420 image padded to whole macroblocks by replicating the last row / column (what an
+// encoder does with the invisible part is its own business; replication keeps its residual small).  dst: Y plane of
+// pitch cols*16, then U and V of pitch cols*8, each rows*16 / rows*8 lines.
+void PadToMacroblocks(const uint8_t *i420, int width, int height, int cols, int rows, uint8_t *dst) {
+  const int sp_y = cols * 16, sp_c = cols * 8;
+  const int cw = (width + 1) / 2, ch = (height + 1) / 2;
+  const uint8_t *py = i420, *pu = py + size_t(width) * height, *pv = pu + size_t(cw) * ch;
+  uint8_t *dy = dst, *du = dy + size_t(sp_y) * rows * 16, *dv = du + size_t(sp_c) * rows * 8;
+  auto pad = [](uint8_t *d, int dp, int dw, int dh, const uint8_t *src, int sw, int sh) {
+    for (int y = 0; y < dh; ++y) {
+      const uint8_t *srow = src + size_t(std::min(y, sh - 1)) * sw;
+      uint8_t *drow = d + size_t(y) * dp;
+      std::memcpy(drow, srow, size_t(sw));
+      std::memset(drow + sw, srow[sw - 1], size_t(dw - sw));
+    }
+  };
+  pad(dy, sp_y, sp_y, rows * 16, py, width, height);
+  pad(du, sp_c, sp_c, rows * 8, pu, cw, ch);
+  pad(dv, sp_c, sp_c, rows * 8, pv, cw, ch);
 }
 
 }  // namespace
@@ -1069,21 +1091,7 @@ VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *s
   int n_groups = 0;
   for (int i = 0; i < n; ++i) {
     vp8r_stream *s = streams[i];
-    // pad the cropped I420 image to whole macroblocks
-    const int cw = (width + 1) / 2, ch = (height + 1) / 2;
-    const uint8_t *py = i420[i], *pu = py + size_t(width) * height, *pv = pu + size_t(cw) * ch;
-    uint8_t *dy = padded.data(), *du = dy + size_t(sp_y) * rows * 16, *dv = du + size_t(sp_c) * rows * 8;
-    auto pad = [](uint8_t *dst, int dp, int dw, int dh, const uint8_t *src, int sw, int sh) {
-      for (int y = 0; y < dh; ++y) {
-        const uint8_t *srow = src + size_t(std::min(y, sh - 1)) * sw;
-        uint8_t *drow = dst + size_t(y) * dp;
-        std::memcpy(drow, srow, size_t(sw));
-        std::memset(drow + sw, srow[sw - 1], size_t(dw - sw));
-      }
-    };
-    pad(dy, sp_y, sp_y, rows * 16, py, width, height);
-    pad(du, sp_c, sp_c, rows * 8, pu, cw, ch);
-    pad(dv, sp_c, sp_c, rows * 8, pv, cw, ch);
+    PadToMacroblocks(i420[i], width, height, cols, rows, padded.data());
     uint8_t *base = sl.d_arena + per_frame * size_t(i);
     CU_TRY(cudaMemcpyAsync(base, padded.data(), src_bytes, cudaMemcpyHostToDevice, e->st));
     CU_TRY(cudaStreamSynchronize(e->st));  // `padded` is reused for the next image
@@ -1163,6 +1171,177 @@ VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *s
     const vp8r_mb_info *mbs = out[i]->mbs();
     for (size_t m = 0; m < n_mb; ++m) blocks += uint32_t(__builtin_popcount(mbs[m].coef_mask));
     out[i]->hdr.n_coef_blocks = blocks;
+  }
+  return VP8R_OK;
+}
+
+// Row f4, inter frames: every macroblock predicts from LAST with one vector (K_encode_inter), the decoder's own
+// K_inter reconstructs from the records, then the loop filter and the border as for a decoded frame.
+VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
+                                      int width, int height, int q_index, int loop_filter_level, int sharpness,
+                                      int search_range, vp8r_frame *const *out) {
+  if (!e || n <= 0 || !streams || !i420 || !out || width < 1 || height < 1 || width > 16383 || height > 16383 || q_index < 0 ||
+      q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 || sharpness > 7 || search_range < 4 ||
+      search_range > 24)
+    return VP8R_ERR_INVALID_ARG;
+  int rc = EnsureDevice(e);
+  if (rc) return rc;
+  {
+    std::vector<const vp8r_stream *> seen(streams, streams + n);
+    std::sort(seen.begin(), seen.end());
+    if (std::adjacent_find(seen.begin(), seen.end()) != seen.end()) {
+      SetError("a stream appears twice in one batch");
+      return VP8R_ERR_INVALID_ARG;
+    }
+  }
+  for (int i = 0; i < n; ++i)
+    if (!streams[i] || streams[i]->eng != e || !i420[i] || !out[i]) {
+      SetError("null stream / image / frame or stream of another engine");
+      return VP8R_ERR_INVALID_ARG;
+    }
+  for (int i = 0; i < n; ++i) {
+    const vp8r_stream *s = streams[i];
+    if (!s->have_frame || s->failed || s->ref[1] < 0) {
+      SetError("inter frame for a stream without a frame to predict from");
+      return VP8R_ERR_STATE;
+    }
+    if (s->width != width || s->height != height) {
+      SetError("inter frame of another size than the stream's frames");
+      return VP8R_ERR_STATE;
+    }
+  }
+  vp8r_frame_hdr h{};
+  h.width = uint16_t(width);
+  h.height = uint16_t(height);
+  h.mb_cols = uint16_t((width + 15) / 16);
+  h.mb_rows = uint16_t((height + 15) / 16);
+  h.key_frame = 0;
+  h.show_frame = 1;
+  h.loop_filter_level = uint8_t(loop_filter_level);
+  h.sharpness_level = uint8_t(sharpness);
+  h.refresh_last = 1;
+  h.q_index = uint8_t(q_index);
+  vp8r::DequantFactorsForIndex(q_index, h.dq[0]);
+  const int cols = h.mb_cols, rows = h.mb_rows;
+  const size_t n_mb = size_t(cols) * rows;
+  const int sp_y = cols * 16, sp_c = cols * 8;
+  const size_t src_bytes = (size_t(sp_y) * rows * 16 + 2 * size_t(sp_c) * rows * 8 + 255) & ~size_t(255);
+  const size_t mb_bytes = (n_mb * sizeof(vp8r_mb_info) + 255) & ~size_t(255);
+  const size_t pay_bytes = n_mb * 25 * 32;
+  const size_t per_frame = src_bytes + mb_bytes + ((pay_bytes + 255) & ~size_t(255));
+  Slot &sl = e->slots[e->cur_slot];
+  e->cur_slot = (e->cur_slot + 1) % vp8r_engine::kSlots;
+  if (sl.pending) {
+    CU_TRY(cudaEventSynchronize(sl.done));
+    sl.pending = false;
+  }
+  {
+    std::string what;
+    HarvestStatus(sl, &what);
+  }
+  rc = GrowSlot(e, sl, n, per_frame * size_t(n));
+  if (rc) return rc;
+
+  std::vector<uint8_t> padded(src_bytes);
+  std::vector<int> cur_idx(static_cast<size_t>(n), -1);
+  bool tma = e->inter_tma;
+  int n_groups = 0;
+  for (int i = 0; i < n; ++i) {
+    vp8r_stream *s = streams[i];
+    PadToMacroblocks(i420[i], width, height, cols, rows, padded.data());
+    uint8_t *base = sl.d_arena + per_frame * size_t(i);
+    CU_TRY(cudaMemcpyAsync(base, padded.data(), src_bytes, cudaMemcpyHostToDevice, e->st));
+    CU_TRY(cudaStreamSynchronize(e->st));  // `padded` is reused for the next image
+
+    int cur = -1;
+    for (int k = 0; k < 5 && cur < 0; ++k)
+      if (k != s->ref[0] && k != s->ref[1] && k != s->ref[2] && k != s->ref[3]) cur = k;
+    cur_idx[size_t(i)] = cur;
+    DevFrameJob &j = sl.h_jobs[i];
+    std::memset(&j, 0, sizeof(j));
+    FillJobSurfaces(s, cur, &j);
+    tma = tma && s->d_tmaps != nullptr;
+    j.mbs = reinterpret_cast<const vp8r_mb_info *>(base + src_bytes);
+    j.payload = reinterpret_cast<const int16_t *>(base + src_bytes + mb_bytes);
+    j.n_inter = int(n_mb);
+    j.n_intra = 0;
+    std::memcpy(j.dq, h.dq, sizeof(j.dq));
+    j.key_frame = 0;
+    j.version = 0;
+    j.lf_level = h.loop_filter_level;
+    j.sharpness = h.sharpness_level;
+    j.enc_src[0] = base;
+    j.enc_src[1] = base + size_t(sp_y) * rows * 16;
+    j.enc_src[2] = j.enc_src[1] + size_t(sp_c) * rows * 8;
+    j.enc_src_pitch_y = sp_y;
+    j.enc_src_pitch_c = sp_c;
+    j.enc_search_range = search_range;
+    e->acc.frames++;
+  }
+  if (loop_filter_level != 0 && (e->filter_mode == 2 || (e->filter_mode == 0 && n >= e->swar_min_frames))) {
+    vp8r::FilterGroup *hg = reinterpret_cast<vp8r::FilterGroup *>(sl.h_jobs + n);
+    for (int at = 0; at < n; at += 8) {
+      vp8r::FilterGroup g;
+      for (int k = 0; k < 8; ++k) g.frame[k] = at + k < n ? at + k : -1;
+      hg[n_groups++] = g;
+    }
+  }
+  CU_TRY(vp8r::LaunchCopy(sl.d_jobs, sl.h_jobs, sizeof(DevFrameJob) * n + sizeof(vp8r::FilterGroup) * n_groups, e->st));
+  {
+    ScopedTimer t(e, 0);
+    CU_TRY(vp8r::LaunchEncodeInter(sl.d_jobs, n, cols, rows, e->st));
+    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st, tma));
+    e->acc.launches_inter += 2;
+  }
+  {
+    ScopedTimer t(e, 2);
+    const int need_sync = vp8r::FilterSyncInts(n);
+    if (need_sync > e->sync_cap) {
+      CU_TRY(cudaStreamSynchronize(e->st));
+      if (e->d_sync) cudaFree(e->d_sync);
+      e->d_sync = nullptr;
+      CU_TRY(cudaMalloc(reinterpret_cast<void **>(&e->d_sync), sizeof(int) * size_t(need_sync) * 2));
+      e->sync_cap = need_sync * 2;
+    }
+    CU_TRY(vp8r::LaunchFilter(sl.d_jobs, n, rows, e->d_sync, e->sync_cap, e->st,
+                              reinterpret_cast<const vp8r::FilterGroup *>(sl.d_jobs + n), n_groups));
+    e->acc.launches_filter++;
+    CU_TRY(vp8r::LaunchBorder(sl.d_jobs, n, e->st));
+  }
+  for (int i = 0; i < n; ++i) {
+    vp8r_frame *f = out[i];
+    f->DropDeviceCopy();
+    f->hdr = h;
+    f->n_mb = n_mb;
+    f->hdr.n_payload_blocks = uint32_t(n_mb * 25);
+    if (!f->Reserve(n_mb * sizeof(vp8r_mb_info) + pay_bytes, 0)) {
+      SetError("out of host memory for the encoded frame");
+      return VP8R_ERR_NOMEM;
+    }
+    const uint8_t *base = sl.d_arena + per_frame * size_t(i);
+    CU_TRY(cudaMemcpyAsync(f->blob, base + src_bytes, n_mb * sizeof(vp8r_mb_info), cudaMemcpyDeviceToHost, e->st));
+    CU_TRY(cudaMemcpyAsync(f->blob + n_mb * sizeof(vp8r_mb_info), base + src_bytes + mb_bytes, pay_bytes, cudaMemcpyDeviceToHost, e->st));
+  }
+  CU_TRY(cudaStreamSynchronize(e->st));
+  // The reconstruction is done; references move as for a decoded inter frame with refresh_last = 1 (golden and
+  // altref stay), even if a mode cannot be assigned below.
+  for (int i = 0; i < n; ++i) {
+    vp8r_stream *s = streams[i];
+    s->ref[1] = s->ref[0] = cur_idx[size_t(i)];
+    s->have_frame = true;
+  }
+  for (int i = 0; i < n; ++i) {
+    vp8r_mb_info *mbs = out[i]->mbs();
+    std::string err;
+    rc = vp8r::AssignInterModes(mbs, cols, rows, &err);
+    if (rc) {
+      SetError(err);
+      return rc;
+    }
+    uint32_t blocks = 0;
+    for (size_t m = 0; m < n_mb; ++m) blocks += uint32_t(__builtin_popcount(mbs[m].coef_mask));
+    out[i]->hdr.n_coef_blocks = blocks;
+    out[i]->hdr.n_inter_mbs = uint32_t(n_mb);
   }
   return VP8R_OK;
 }

@@ -36,7 +36,8 @@ class ParsedFrame:
         return d
 
     def write_bitstream(self):
-        """The frame as a VP8 key frame (the inverse of Parser.parse for what the encoder produces)."""
+        """The frame as a VP8 frame, key or inter (the inverse of Parser.parse for what the encoder produces; see
+        vp8r_frame_write_bitstream for the frames that can be written)."""
         size = C.c_size_t(0)
         rc = self._lib.vp8r_frame_write_bitstream(self.handle, None, 0, C.byref(size))
         if size.value == 0:
@@ -129,6 +130,27 @@ class Engine:
         ia = (C.c_void_p * n)(*[C.cast(b, C.c_void_p) for b in bufs])
         fa = (C.c_void_p * n)(*[f.handle for f in frames])
         check(self._lib.vp8r_encode_key_frames(self.handle, n, sa, ia, width, height, q_index, loop_filter_level, sharpness, 1 if bpred else 0, fa))
+        return frames
+
+    def encode_inter_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, search_range=16):
+        """One inter frame per stream from cropped I420 images (bytes): every macroblock predicts from the stream's
+        current LAST frame with one motion vector, searched on the device over +-search_range whole pixels (4..24) and
+        refined to quarter pel (vp8r_encode_inter_frames).  Returns the ParsedFrame objects (records with modes and
+        vectors, coefficient blocks; .write_bitstream() serialises them); every stream then holds the reconstructed
+        frame a decoder would produce."""
+        n = len(streams)
+        need = width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2)
+        bufs = []
+        for img in images:
+            if len(img) != need:
+                raise ValueError("image is not a cropped I420 frame of the given size")
+            bufs.append((C.c_uint8 * need).from_buffer_copy(img))
+        frames = [ParsedFrame(pinned=False) for _ in range(n)]
+        sa = (C.c_void_p * n)(*[s.handle for s in streams])
+        ia = (C.c_void_p * n)(*[C.cast(b, C.c_void_p) for b in bufs])
+        fa = (C.c_void_p * n)(*[f.handle for f in frames])
+        check(self._lib.vp8r_encode_inter_frames(self.handle, n, sa, ia, width, height, q_index, loop_filter_level, sharpness,
+                                                 search_range, fa))
         return frames
 
     def upload(self, frame, release_host=False):
@@ -286,3 +308,35 @@ def decode_ivf(path_or_bytes, engine=None, layout=None):
     if dims is None:
         raise ValueError("the stream has no shown frame")
     return frames[:len(out)]
+
+
+def encode_ivf(images, width, height, q_index, path=None, key_interval=0, loop_filter_level=0, sharpness=0, bpred=True,
+               search_range=16, engine=None):
+    """Encodes one stream of cropped I420 images (bytes) into an IVF file, the mirror of decode_ivf: a key frame first
+    and then every key_interval frames (0: only the first), inter frames between them.  Returns the IVF bytes and
+    writes them to `path` when one is given."""
+    from .ivf import ivf_bytes
+    if key_interval < 0:
+        raise ValueError("key_interval must be >= 0")
+    own = engine is None
+    engine = engine or Engine()
+    st = engine.open_stream()
+    payloads = []
+    try:
+        for i, img in enumerate(images):
+            if i == 0 or (key_interval and i % key_interval == 0):
+                (f,) = engine.encode_key_frames([st], [img], width, height, q_index, loop_filter_level, sharpness, bpred)
+            else:
+                (f,) = engine.encode_inter_frames([st], [img], width, height, q_index, loop_filter_level, sharpness,
+                                                  search_range)
+            payloads.append(f.write_bitstream())
+            f.close()
+    finally:
+        st.close()
+        if own:
+            engine.close()
+    data = ivf_bytes(width, height, payloads)
+    if path is not None:
+        with open(path, "wb") as fh:
+            fh.write(data)
+    return data

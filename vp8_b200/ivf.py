@@ -20,9 +20,15 @@ def read_ivf(path_or_bytes):
     return {"width": w, "height": h, "rate": rate, "scale": scale, "n_frames": n_frames}, frames
 
 
+def ivf_bytes(width, height, frames, rate=30, scale=1):
+    """An IVF file holding `frames` (payload bytes), as bytes."""
+    out = [b"DKIF" + struct.pack("<HH4sHHIII", 0, 32, b"VP80", width, height, rate, scale, len(frames)) + b"\0\0\0\0"]
+    for i, fr in enumerate(frames):
+        out.append(struct.pack("<IQ", len(fr), i))
+        out.append(bytes(fr))
+    return b"".join(out)
+
+
 def write_ivf(path, width, height, frames, rate=30, scale=1):
     with open(path, "wb") as f:
-        f.write(b"DKIF" + struct.pack("<HH4sHHIII", 0, 32, b"VP80", width, height, rate, scale, len(frames)) + b"\0\0\0\0")
-        for i, fr in enumerate(frames):
-            f.write(struct.pack("<IQ", len(fr), i))
-            f.write(fr)
+        f.write(ivf_bytes(width, height, frames, rate, scale))
