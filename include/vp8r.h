@@ -334,12 +334,22 @@ VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const 
                                       int width, int height, int q_index, int loop_filter_level, int sharpness,
                                       int search_range, vp8r_frame *const *out);
 /* The inverse of vp8r_parser_parse: serialises f into a VP8 frame with one DCT partition and the default token, mode and
- * motion-vector probabilities.  Key frames: intra macroblocks.  Inter frames: the frame header's refresh, copy,
+ * motion-vector probabilities (see vp8r_frame_write_bitstream_in for inter frames of a stream that was decoded).  Key frames: intra macroblocks.  Inter frames: the frame header's refresh, copy,
  * sign-bias and show_frame fields from f's header, intra macroblocks, and inter macroblocks of any reference coded
  * NEAREST / NEAR / ZERO / NEW.  Both: no segmentation, no loop-filter deltas, the five quantiser deltas that reproduce
  * hdr.dq[0] from q_index.  SPLIT macroblocks and a vector that contradicts its mode are refused.  *size receives the
  * number of bytes needed; VP8R_ERR_INVALID_ARG when cap is too small (call again) or the frame cannot be written. */
 VP8R_API int vp8r_frame_write_bitstream(const vp8r_frame *f, uint8_t *dst, size_t cap, size_t *size);
+/* The same, with the token, motion-vector and 16x16 / chroma mode probabilities of `context`: the parser that parsed
+ * the stream so far, whose state a decoder holds when it reaches this frame.  Write with it when the stream's LAST
+ * frame came from decoding: the probability updates a stream carries persist until its next key frame, and a frame
+ * coded with the defaults does not decode in such a stream.  context == NULL gives vp8r_frame_write_bitstream's bytes;
+ * a key frame ignores context (it resets the decoder's probabilities).  The written frame carries no updates and sets
+ * refresh_entropy_probs, so the context is the same after it: consecutive frames can all be written against the same
+ * parser without feeding them through it.  VP8R_ERR_STATE: for an inter frame, a context that has not parsed a key
+ * frame or whose frame size is not f's. */
+VP8R_API int vp8r_frame_write_bitstream_in(const vp8r_frame *f, const vp8r_parser *context, uint8_t *dst, size_t cap,
+                                           size_t *size);
 
 /* Device-side checksum of the cropped I420 image: low word sum(b_i), high word
  * sum((i+1)*b_i), both mod 2^32, i = byte index in the Y,U,V stream.  For parity checks at sizes

@@ -13,6 +13,8 @@
 
 int oracle_encode_inter_frame(const oracle_decoder *d, const uint8_t *sy, const uint8_t *su, const uint8_t *sv, int cols, int rows,
                               const int16_t dq[6], int q_index, int lf_level, int search_range, vp8r_mb_info *mbs, int16_t *payload);
+int oracle_search_full_pel(const oracle_decoder *d, const uint8_t *sy, int cols, int rows, int y1_ac, int search_range,
+                           int16_t *mv);
 
 /* Six-tap prediction of the 16x16 luma block of macroblock (r, c) for the vector (mvr, mvc) in 1/8 pel, as the
  * decoder predicts it (predict_inter4x4 per 4x4 block, reference clamped at the plane's edges). */
@@ -20,6 +22,25 @@ static void enc_predict_luma(const ofrm *ref, int r, int c, int mvr, int mvc, ui
   for (int b = 0; b < 16; b++)
     predict_inter4x4(pred + (b >> 2) * 64 + (b & 3) * 4, 16, ref->y, ref->ys, ref->yh, ref->ys, 16 * r + 4 * (b >> 2),
                      16 * c + 4 * (b & 3), mvr, mvc, k_sixtap);
+}
+
+/* Full-pel search of macroblock (r, c) over |dy|, |dx| <= R: the minimum of (cost << 12) | index with
+ * index = (dy + R) * (2R + 1) + dx + R, reference pixels clamped to the MB-aligned plane. */
+static uint32_t enc_full_pel(const ofrm *ref, const uint8_t *src, int ys, int r, int c, int R, int lambda) {
+  const int span = 2 * R + 1;
+  uint32_t best = 0xffffffffu;
+  for (int i = 0; i < span * span; i++) {
+    const int dy = i / span - R, dx = i % span - R;
+    uint32_t sad = 0;
+    for (int y = 0; y < 16; y++)
+      for (int x = 0; x < 16; x++) {
+        int dd = (int)src[y * ys + x] - ref_px(ref->y, ref->ys, ref->yh, ref->ys, 16 * r + y + dy, 16 * c + x + dx);
+        sad += (uint32_t)(dd < 0 ? -dd : dd);
+      }
+    const uint32_t key = ((sad + (uint32_t)(lambda * vp8r_enc_mv_bits(4 * dy, 4 * dx))) << 12) | (uint32_t)i;
+    if (key < best) best = key;
+  }
+  return best;
 }
 
 static uint32_t enc_sad16(const uint8_t *src, int ss, const uint8_t pred[256]) {
@@ -52,19 +73,7 @@ int oracle_encode_inter_frame(const oracle_decoder *d, const uint8_t *sy, const 
     for (int c = 0; c < cols; c++) {
       const int m = r * cols + c;
       const uint8_t *src = sy + (size_t)(16 * r) * ys + 16 * c;
-      /* full pel */
-      uint32_t best = 0xffffffffu;
-      for (int i = 0; i < span * span; i++) {
-        const int dy = i / span - R, dx = i % span - R;
-        uint32_t sad = 0;
-        for (int y = 0; y < 16; y++)
-          for (int x = 0; x < 16; x++) {
-            int dd = (int)src[y * ys + x] - ref_px(ref->y, ref->ys, ref->yh, ref->ys, 16 * r + y + dy, 16 * c + x + dx);
-            sad += (uint32_t)(dd < 0 ? -dd : dd);
-          }
-        const uint32_t key = ((sad + (uint32_t)(lambda * vp8r_enc_mv_bits(4 * dy, 4 * dx))) << 12) | (uint32_t)i;
-        if (key < best) best = key;
-      }
+      const uint32_t best = enc_full_pel(ref, src, ys, r, c, R, lambda);
       int qr = 4 * ((int)(best & 4095u) / span - R), qc = 4 * ((int)(best & 4095u) % span - R);
       uint32_t centre = best >> 12;
       /* half pel, quarter pel */
@@ -138,6 +147,22 @@ int oracle_encode_inter_frame(const oracle_decoder *d, const uint8_t *sy, const 
                   (mb->coef_mask ? VP8R_MB_LF_INNER : 0u);
       mb->mv[0] = (int16_t)mvr;
       mb->mv[1] = (int16_t)mvc;
+    }
+  return 0;
+}
+
+/* The full-pel stage alone, as oracle_encode_inter_frame runs it (lambda from the luma AC factor y1_ac): mv[2m],
+ * mv[2m+1] = (dy, dx) in whole pixels of macroblock m.  Returns 0, or -1 when d has no LAST frame of this size. */
+int oracle_search_full_pel(const oracle_decoder *d, const uint8_t *sy, int cols, int rows, int y1_ac, int search_range,
+                           int16_t *mv) {
+  const ofrm *ref = d->ref[1];
+  if (!d->have_frame || !ref || ref->cols != cols || ref->rows != rows) return -1;
+  const int ys = cols * 16, R = search_range, span = 2 * R + 1, lambda = vp8r_enc_lambda(y1_ac);
+  for (int r = 0; r < rows; r++)
+    for (int c = 0; c < cols; c++) {
+      const int i = (int)(enc_full_pel(ref, sy + (size_t)(16 * r) * ys + 16 * c, ys, r, c, R, lambda) & 4095u);
+      mv[2 * (r * cols + c)] = (int16_t)(i / span - R);
+      mv[2 * (r * cols + c) + 1] = (int16_t)(i % span - R);
     }
   return 0;
 }

@@ -76,6 +76,7 @@ SIGNATURES = {
     "vp8r_encode_inter_frames": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int, C.c_int,
                                            C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "vp8r_frame_write_bitstream": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "vp8r_frame_write_bitstream_in": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "vp8r_read_batch_packed_as": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t, C.c_int, C.c_int]),
     "vp8r_read_batch_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t, C.c_int,
                                          C.c_void_p]),

@@ -154,10 +154,15 @@ VP8R_API int vp8r_parse_batch(int n, vp8r_parser *const *parsers, const uint8_t 
 }
 
 VP8R_API int vp8r_frame_write_bitstream(const vp8r_frame *f, uint8_t *dst, size_t cap, size_t *size) {
+  return vp8r_frame_write_bitstream_in(f, nullptr, dst, cap, size);
+}
+
+VP8R_API int vp8r_frame_write_bitstream_in(const vp8r_frame *f, const vp8r_parser *context, uint8_t *dst, size_t cap,
+                                           size_t *size) {
   if (!f || !size) return VP8R_ERR_INVALID_ARG;
   std::vector<uint8_t> bytes;
   std::string err;
-  const int rc = vp8r::WriteFrame(*f, &bytes, &err);
+  const int rc = vp8r::WriteFrame(*f, context ? &context->impl : nullptr, &bytes, &err);
   if (rc != VP8R_OK) {
     vp8r::SetError(err);
     return rc;

@@ -47,6 +47,14 @@ class FrameParser {
   // too (vp8r_frame_hdr.modes_deferred).  Implies deferred tokens.
   void set_defer_modes(bool on) { want_defer_modes_ = on; }
 
+  // The context the next frame of the stream is parsed in (read by the bitstream writer): whether a key frame has
+  // been seen, the size it set, and the token / motion-vector / mode probabilities (after a frame with
+  // refresh_entropy_probs = 0, those from before that frame).
+  bool have_key() const { return have_key_; }
+  int width() const { return width_; }
+  int height() const { return height_; }
+  const EntropyTables &probs() const { return probs_; }
+
  private:
   int Fail(int code, const std::string &msg) {
     error_ = msg;

@@ -38,12 +38,13 @@ const int kCatBits[6] = {1, 2, 3, 4, 5, 11};
 // One block of tokens (RFC 6386 section 13; the mirror of FrameParser::ReadCoefTokens): `blk` holds the quantised
 // coefficients in raster order, scan position n is blk[kZigzag[n]].  No end-of-block right after a zero token.
 // Returns whether any coefficient from `first` on is non-zero.  A magnitude above DCT_CAT6's range cannot be coded.
-bool WriteBlock(BoolWriter &bw, int type, int ctx, int first, const int16_t *blk, bool *too_large) {
+// `coef` holds the token probabilities of the frame's context.
+bool WriteBlock(BoolWriter &bw, const uint8_t (*coef)[8][3][11], int type, int ctx, int first, const int16_t *blk,
+                bool *too_large) {
   int last = -1;
   for (int n = first; n < 16; ++n)
     if (blk[kZigzag[n]]) last = n;
-  const uint8_t *base = &kCoefDefault[size_t(type) * 8 * 3 * 11];
-  auto probs = [&](int n, int cx) { return base + (size_t(kBand[n]) * 3 + size_t(cx)) * 11; };
+  auto probs = [&](int n, int cx) { return coef[type][kBand[n]][cx]; };
   bool prev_zero = false;
   int n = first;
   for (; n <= last; ++n) {
@@ -117,6 +118,17 @@ void WriteMvComponent(BoolWriter &bw, const uint8_t *p, int v) {
   if (x) bw.Put(p[1], v < 0);
 }
 
+// The context of a stream right after a key frame: the default token, motion-vector and 16x16 / chroma mode
+// probabilities (FrameParser::LoadDefaults).
+EntropyTables DefaultTables() {
+  EntropyTables t;
+  std::memcpy(t.coef, kCoefDefault, sizeof(t.coef));
+  std::memcpy(t.mv, kMvDefault, sizeof(t.mv));
+  std::memcpy(t.ymode, kProbYModeDefault, sizeof(t.ymode));
+  std::memcpy(t.uvmode, kProbUvModeDefault, sizeof(t.uvmode));
+  return t;
+}
+
 // P(bit == 0) out of 256 for `zeros` of `total` decisions, kept inside 1..255 (how prob_skip_false is chosen).
 int ProbOf(size_t zeros, size_t total) {
   const int p = int(256 * zeros / (total ? total : 1));
@@ -184,11 +196,11 @@ int AssignInterModes(vp8r_mb_info *mbs, int cols, int rows, std::string *err) {
   return VP8R_OK;
 }
 
-int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err) {
+int WriteFrame(const vp8r_frame &f, const FrameParser *context, std::vector<uint8_t> *out, std::string *err) {
   const vp8r_frame_hdr &h = f.hdr;
-  auto fail = [&](const char *what) {
+  auto fail = [&](const char *what, int code = VP8R_ERR_INVALID_ARG) {
     if (err) *err = what;
-    return VP8R_ERR_INVALID_ARG;
+    return code;
   };
   if (!f.blob) return fail("vp8r_frame_write_bitstream: the frame has no host arrays");
   if (h.tokens_deferred || h.modes_deferred) return fail("vp8r_frame_write_bitstream: the frame holds raw partitions, not macroblock records");
@@ -196,6 +208,15 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
   if (cols <= 0 || rows <= 0 || size_t(cols) * rows != f.n_mb) return fail("vp8r_frame_write_bitstream: inconsistent frame size");
   if (h.version > 3) return fail("vp8r_frame_write_bitstream: unknown bitstream version");
   const bool key = h.key_frame != 0;
+  // A key frame resets the decoder's context to the defaults; an inter frame is coded in the one it is decoded in.
+  static const EntropyTables kDefaults = DefaultTables();
+  const EntropyTables *probs = &kDefaults;
+  if (context && !key) {
+    if (!context->have_key()) return fail("vp8r_frame_write_bitstream_in: the context parser has not parsed a key frame", VP8R_ERR_STATE);
+    if (context->width() != h.width || context->height() != h.height)
+      return fail("vp8r_frame_write_bitstream_in: the context parser's frame size differs from the frame's", VP8R_ERR_STATE);
+    probs = &context->probs();
+  }
   const vp8r_mb_info *mbs = f.mbs();
   const int16_t *payload = f.payload();
   int qdelta[5];
@@ -244,16 +265,16 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
   }
   hdr.Lit(1, 1);  // refresh_entropy_probs
   if (!key) hdr.Lit(1, h.refresh_last ? 1u : 0u);
-  for (int i = 0; i < 1056; ++i) hdr.Put(kCoefUpdate[i], 0);  // keep the default token probabilities
+  for (int i = 0; i < 1056; ++i) hdr.Put(kCoefUpdate[i], 0);  // keep the context's token probabilities
   hdr.Lit(1, 1);                                             // mb_no_skip_coeff
   hdr.Lit(8, uint32_t(prob_skip));
   if (!key) {
     hdr.Lit(8, uint32_t(prob_intra));
     hdr.Lit(8, uint32_t(prob_last));
     hdr.Lit(8, uint32_t(prob_gf));
-    hdr.Lit(1, 0);                                         // keep the 16x16 luma mode probabilities
-    hdr.Lit(1, 0);                                         // keep the chroma mode probabilities
-    for (int i = 0; i < 38; ++i) hdr.Put(kMvUpdate[i], 0);  // keep the motion-vector probabilities
+    hdr.Lit(1, 0);                                         // keep the context's 16x16 luma mode probabilities
+    hdr.Lit(1, 0);                                         // ... its chroma mode probabilities
+    for (int i = 0; i < 38; ++i) hdr.Put(kMvUpdate[i], 0);  // ... and its motion-vector probabilities
   }
 
   const bool sign_bias[4] = {false, false, h.sign_bias_golden != 0, h.sign_bias_altref != 0};
@@ -303,12 +324,12 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
         for (int i = 0; i < 4; ++i) p[i] = kProbMvRef[nm.cnt[i]][i];
         hdr.Tree(kTreeMvRef, 8, p, ymode);
         if (ymode == MV_NEW) {
-          WriteMvComponent(hdr, &kMvDefault[0], dr / 2);
-          WriteMvComponent(hdr, &kMvDefault[19], dc / 2);
+          WriteMvComponent(hdr, probs->mv[0], dr / 2);
+          WriteMvComponent(hdr, probs->mv[1], dc / 2);
         }
         ctx[size_t(idx)] = MbCtx{1, uint8_t(ref), uint8_t(ymode), v};
       } else {
-        hdr.Tree(key ? kTreeYModeKey : kTreeYMode, 8, key ? kProbYModeKey : kProbYModeDefault, ymode);
+        hdr.Tree(key ? kTreeYModeKey : kTreeYMode, 8, key ? kProbYModeKey : probs->ymode, ymode);
         if (ymode == B_PRED) {
           for (int i = 0; i < 4; ++i)
             for (int j = 0; j < 4; ++j) {
@@ -325,7 +346,7 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
           static const uint8_t implied[4] = {0, 2, 3, 1};  // DC->B_DC, V->B_VE, H->B_HE, TM->B_TM (RFC 6386 11.3)
           for (int i = 0; i < 4; ++i) above_b[size_t(c) * 4 + i] = left_b[i] = implied[ymode];
         }
-        hdr.Tree(kTreeUvMode, 6, key ? kProbUvModeKey : kProbUvModeDefault, uvmode);
+        hdr.Tree(kTreeUvMode, 6, key ? kProbUvModeKey : probs->uvmode, uvmode);
       }
 
       if (!skip) {
@@ -351,7 +372,7 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
         };
         uint32_t raw = 0, nz = 0;  // bit 0: Y2, 1..16: Y, 17..20: U, 21..24: V
         if (has_y2) {
-          if (WriteBlock(tok, 1, nz_ay2[size_t(c)] + nz_ly2, 0, blk[0], &too_large)) raw |= 1;
+          if (WriteBlock(tok, probs->coef, 1, nz_ay2[size_t(c)] + nz_ly2, 0, blk[0], &too_large)) raw |= 1;
           if (dq_nz(blk[0], 0, dq[VP8R_DQ_Y2_DC], dq[VP8R_DQ_Y2_AC])) nz |= 1;
           nz_ay2[size_t(c)] = nz_ly2 = uint8_t(nz & 1);
         }
@@ -359,7 +380,7 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
           const int i = b >> 2, j = b & 3;
           const int a = i ? int((raw >> (b - 3)) & 1) : nz_ay[size_t(c) * 4 + j];
           const int l = j ? int((raw >> b) & 1) : nz_ly[i];
-          if (WriteBlock(tok, has_y2 ? 0 : 3, a + l, has_y2 ? 1 : 0, blk[1 + b], &too_large)) raw |= 2u << b;
+          if (WriteBlock(tok, probs->coef, has_y2 ? 0 : 3, a + l, has_y2 ? 1 : 0, blk[1 + b], &too_large)) raw |= 2u << b;
           if (dq_nz(blk[1 + b], has_y2 ? 1 : 0, dq[VP8R_DQ_Y1_DC], dq[VP8R_DQ_Y1_AC])) nz |= 2u << b;
         }
         for (int pl = 0; pl < 2; ++pl) {
@@ -370,7 +391,7 @@ int WriteFrame(const vp8r_frame &f, std::vector<uint8_t> *out, std::string *err)
             const int i = b >> 1, j = b & 1;
             const int a = i ? int((raw >> (base + b - 2)) & 1) : na[j];
             const int l = j ? int((raw >> (base + b - 1)) & 1) : nl[i];
-            if (WriteBlock(tok, 2, a + l, 0, blk[base + b], &too_large)) raw |= 1u << (base + b);
+            if (WriteBlock(tok, probs->coef, 2, a + l, 0, blk[base + b], &too_large)) raw |= 1u << (base + b);
             if (dq_nz(blk[base + b], 0, dq[VP8R_DQ_UV_DC], dq[VP8R_DQ_UV_AC])) nz |= 1u << (base + b);
           }
         }

@@ -35,15 +35,18 @@ class ParsedFrame:
         check(self._lib.vp8r_frame_get_desc(self.handle, C.byref(d)))
         return d
 
-    def write_bitstream(self):
+    def write_bitstream(self, context=None):
         """The frame as a VP8 frame, key or inter (the inverse of Parser.parse for what the encoder produces; see
-        vp8r_frame_write_bitstream for the frames that can be written)."""
+        vp8r_frame_write_bitstream for the frames that can be written).  context: the Parser that parsed the stream so
+        far; an inter frame is then coded with that stream's current probabilities instead of the defaults, which it
+        must be when the stream's LAST frame came from decoding (vp8r_frame_write_bitstream_in)."""
+        ctx = context.handle if context is not None else None
         size = C.c_size_t(0)
-        rc = self._lib.vp8r_frame_write_bitstream(self.handle, None, 0, C.byref(size))
+        rc = self._lib.vp8r_frame_write_bitstream_in(self.handle, ctx, None, 0, C.byref(size))
         if size.value == 0:
             check(rc)
         buf = (C.c_uint8 * size.value)()
-        check(self._lib.vp8r_frame_write_bitstream(self.handle, buf, size.value, C.byref(size)))
+        check(self._lib.vp8r_frame_write_bitstream_in(self.handle, ctx, buf, size.value, C.byref(size)))
         return bytes(buf[:size.value])
 
     def close(self):
