@@ -566,19 +566,24 @@ def test_passes_without_draining_and_resident_replays(engine):
     dec.close()
 
 
+def _truncated_key_frame():
+    """A 320x192 key frame whose declared first partition is cut to half: the start code and headers are kept, the
+    macroblock headers then run past the partition's end while the DCT partition (the bytes behind it) is present."""
+    import vp8_b200
+    ivf = helpers.synth_stream("--width 320 --height 192 --frames 2 --seed 9 --log2-parts 0")
+    key = vp8_b200.read_ivf(ivf)[1][0]
+    first_size = (key[0] | key[1] << 8 | key[2] << 16) >> 5
+    cut = first_size // 2
+    tag = (key[0] | key[1] << 8 | key[2] << 16) & 0x1f | (cut << 5)
+    return bytes([tag & 0xff, (tag >> 8) & 0xff, (tag >> 16) & 0xff]) + key[3:10 + cut] + key[10 + first_size:]
+
+
 def test_device_parse_truncated_first_partition(engine):
     """Deferred modes: a first partition that ends early is reported by vp8r_engine_sync
     (VP8R_ERR_TRUNCATED), like the host parser does for the same bytes."""
     import vp8_b200
     from vp8_b200._capi import Vp8rError
-    ivf = helpers.synth_stream("--width 320 --height 192 --frames 2 --seed 9 --log2-parts 0")
-    key = vp8_b200.read_ivf(ivf)[1][0]
-    first_size = (key[0] | key[1] << 8 | key[2] << 16) >> 5
-    # keep the start code and headers, shorten the declared first partition: the macroblock headers
-    # then run past its end while the DCT partition (the bytes behind it) is still present
-    cut = first_size // 2
-    tag = (key[0] | key[1] << 8 | key[2] << 16) & 0x1f | (cut << 5)
-    bad = bytes([tag & 0xff, (tag >> 8) & 0xff, (tag >> 16) & 0xff]) + key[3:10 + cut] + key[10 + first_size:]
+    bad = _truncated_key_frame()
     host = vp8_b200.Parser()
     with pytest.raises(Vp8rError) as e0:
         host.parse(bad)
@@ -595,6 +600,29 @@ def test_device_parse_truncated_first_partition(engine):
     fr.close()
     st.close()
 
+
+def test_device_parse_failure_survives_encoder_calls(engine):
+    """A device-parse failure not yet reported is still reported by vp8r_engine_sync after encoder calls have reused
+    the slot of its batch (the encoders harvest the slot's error words as decoded batches do)."""
+    import vp8_b200
+    from vp8_b200._capi import Vp8rError
+    ps = vp8_b200.Parser()
+    ps.set_defer_modes(True)
+    st, enc = engine.open_stream(), engine.open_stream()
+    fr = ps.parse(_truncated_key_frame(), pinned=True)
+    engine.reconstruct_batch([st], [fr])
+    w, h = 64, 48
+    image = bytes(range(256)) * ((w * h * 3 // 2) // 256)
+    for _ in range(16):  # more calls than the engine has slots
+        for f in engine.encode_key_frames([enc], [image], w, h, q_index=40):
+            f.close()
+    with pytest.raises(Vp8rError) as e:
+        engine.sync()
+    assert e.value.code == 4
+    engine.sync()
+    fr.close()
+    st.close()
+    enc.close()
 
 def test_device_parse_survives_corrupted_streams(engine):
     """Bit flips / garbage in the partitions (the frame header kept valid): the device-side parse must

@@ -121,19 +121,8 @@ class Engine:
         Returns the ParsedFrame objects (macroblock records + coefficient blocks; .write_bitstream() serialises them);
         every stream then holds the reconstructed frame a decoder would produce.  bpred: B_PRED (sixteen 4x4 modes per
         macroblock) competes with the four 16x16 modes (VP8R_ENC_BPRED)."""
-        n = len(streams)
-        need = width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2)
-        bufs = []
-        for img in images:
-            if len(img) != need:
-                raise ValueError("image is not a cropped I420 frame of the given size")
-            bufs.append((C.c_uint8 * need).from_buffer_copy(img))
-        frames = [ParsedFrame(pinned=False) for _ in range(n)]
-        sa = (C.c_void_p * n)(*[s.handle for s in streams])
-        ia = (C.c_void_p * n)(*[C.cast(b, C.c_void_p) for b in bufs])
-        fa = (C.c_void_p * n)(*[f.handle for f in frames])
-        check(self._lib.vp8r_encode_key_frames(self.handle, n, sa, ia, width, height, q_index, loop_filter_level, sharpness, 1 if bpred else 0, fa))
-        return frames
+        return self._encode(self._lib.vp8r_encode_key_frames, streams, images, width, height, q_index, loop_filter_level,
+                            sharpness, 1 if bpred else 0)
 
     def encode_inter_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, search_range=16):
         """One inter frame per stream from cropped I420 images (bytes): every macroblock predicts from the stream's
@@ -141,6 +130,12 @@ class Engine:
         refined to quarter pel (vp8r_encode_inter_frames).  Returns the ParsedFrame objects (records with modes and
         vectors, coefficient blocks; .write_bitstream() serialises them); every stream then holds the reconstructed
         frame a decoder would produce."""
+        return self._encode(self._lib.vp8r_encode_inter_frames, streams, images, width, height, q_index, loop_filter_level,
+                            sharpness, search_range)
+
+    def _encode(self, fn, streams, images, width, height, *params):
+        """Calls the C encoder entry point fn(engine, n, streams, images, width, height, *params, frames) on one cropped
+        I420 image (bytes) per stream; returns the new ParsedFrame objects."""
         n = len(streams)
         need = width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2)
         bufs = []
@@ -152,8 +147,7 @@ class Engine:
         sa = (C.c_void_p * n)(*[s.handle for s in streams])
         ia = (C.c_void_p * n)(*[C.cast(b, C.c_void_p) for b in bufs])
         fa = (C.c_void_p * n)(*[f.handle for f in frames])
-        check(self._lib.vp8r_encode_inter_frames(self.handle, n, sa, ia, width, height, q_index, loop_filter_level, sharpness,
-                                                 search_range, fa))
+        check(fn(self.handle, n, sa, ia, width, height, *params, fa))
         return frames
 
     def upload(self, frame, release_host=False):
