@@ -333,6 +333,42 @@ VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *s
 VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
                                       int width, int height, int q_index, int loop_filter_level, int sharpness,
                                       int search_range, vp8r_frame *const *out);
+/* ---- encoder input from device memory ----
+ * Frames already on the GPU (decoded frames, a model's output, rendered images) encode without crossing PCIe.  The
+ * source layouts are the VP8R_LAYOUT_* constants read as input formats: VP8R_LAYOUT_I420 (cropped Y, U, V planes back to
+ * back: the bytes of the host path and of vp8r_read_batch_device), VP8R_LAYOUT_NV12 (Y plane, then interleaved U,V
+ * pairs), VP8R_LAYOUT_RGB24 (HWC) and VP8R_LAYOUT_RGB_PLANAR (CHW), 3*w*h bytes.  RGB becomes I420 by BT.601 limited
+ * range in integers, with arithmetic shifts and no clamp (Y lands in 16..235, U and V in 16..240):
+ *   Y = ((66R + 129G + 25B + 128) >> 8) + 16                 per pixel
+ *   U = ((-38R' - 74G' + 112B' + 128) >> 8) + 128            per chroma sample
+ *   V = ((112R' - 94G' - 18B' + 128) >> 8) + 128
+ * where R', G', B' are the channel means (s + 2) >> 2 over the pixels (2i+a, 2j+b), a, b in {0, 1}, of chroma sample
+ * (i, j), pixel coordinates clamped to w-1 / h-1 (odd sizes replicate the edge pixels).  Each component is within 1 of
+ * the rounded floating-point BT.601 matrix.  Whatever the layout, the encoder codes exactly what the host path codes for
+ * the cropped I420 image of the frame (vp8r_convert_to_i420_device returns it).
+ *
+ * vp8r_encode_key_frames_device / vp8r_encode_inter_frames_device: vp8r_encode_key_frames / vp8r_encode_inter_frames
+ * (same checks, outputs, reference updates; synchronous) with frame i of the batch at src + i*stride in device memory
+ * of the engine's device, any byte alignment, stride at least one frame of the layout.  producer_stream: the
+ * cudaStream_t src was written on.  NULL or the engine's own stream: nothing extra; otherwise the engine's stream waits,
+ * before it reads src, for the work submitted to producer_stream so far (without blocking the host).  src may be reused
+ * once the call returns.  VP8R_ERR_INVALID_ARG: null engine / streams / src / out, n <= 0, an unknown layout, a stride
+ * smaller than a frame, src not device memory of the engine's device (pinned, pageable and managed memory are refused),
+ * and the host calls' argument checks; the checks that need no device come first. */
+VP8R_API int vp8r_encode_key_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
+                                           int layout, void *producer_stream, int width, int height, int q_index,
+                                           int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out);
+VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
+                                             int layout, void *producer_stream, int width, int height, int q_index,
+                                             int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out);
+/* The cropped I420 image (w*h + 2*ceil(w/2)*ceil(h/2) bytes) the encoder codes for each of n frames at src + i*src_stride
+ * in `layout`, written to dst + i*dst_stride; src and dst device memory of the engine's device.  For PSNR against the
+ * reconstruction of an RGB / NV12 source.  Asynchronous on the engine's stream, ordered against `stream` (the caller's
+ * cudaStream_t, e.g. torch's current stream; NULL or the engine's own: nothing extra) as vp8r_read_batch_device orders
+ * against its consumer stream: the conversion waits for the work submitted to `stream` so far, and work submitted there
+ * afterwards sees dst.  VP8R_ERR_INVALID_ARG as for the encoder calls, and dst_stride smaller than an I420 frame. */
+VP8R_API int vp8r_convert_to_i420_device(vp8r_engine *e, int n, const void *src, size_t src_stride, int layout, int width,
+                                         int height, void *dst, size_t dst_stride, void *stream);
 /* The inverse of vp8r_parser_parse: serialises f into a VP8 frame with one DCT partition and the default token, mode and
  * motion-vector probabilities (see vp8r_frame_write_bitstream_in for inter frames of a stream that was decoded).  Key frames: intra macroblocks.  Inter frames: the frame header's refresh, copy,
  * sign-bias and show_frame fields from f's header, intra macroblocks, and inter macroblocks of any reference coded

@@ -15,6 +15,10 @@ Reports, in one JSON document (--out):
     --compare-streams streams, encoded as key frames on streams of their own);
   - PSNR (Y, whole frame) of the reconstructions of --compare-streams streams against their source;
   - the card's name and power limit (nvidia-smi).
+--input selects where the pictures come from: "host" (cropped I420 bytes, the default), "i420" (a CUDA tensor of the
+same bytes) or "rgb" (a CUDA tensor of RGB24 pictures, made from the I420 pictures in numpy by include/vp8r.h's
+YUV -> RGB formula).  A device input is uploaded before each call, outside the timed window; with "rgb" the PSNR is
+measured against the I420 the encoder codes (Engine.convert_to_i420).
 --dry-run builds the pictures of the first two time steps and prints the plan without touching a device.
 """
 import argparse
@@ -64,6 +68,17 @@ def gpu_info():
     return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else f"nvidia-smi failed: {q.stderr.strip()}"
 
 
+def rgb_from_i420(img, w, h):
+    """Cropped I420 bytes -> (h, w, 3) RGB by include/vp8r.h's BT.601 formula (chroma point-sampled)."""
+    a = np.frombuffer(img, np.uint8)
+    cw, ch = (w + 1) // 2, (h + 1) // 2
+    y = a[:w * h].reshape(h, w).astype(np.int32) - 16
+    u = a[w * h:w * h + cw * ch].reshape(ch, cw).repeat(2, 0).repeat(2, 1)[:h, :w].astype(np.int32) - 128
+    v = a[w * h + cw * ch:].reshape(ch, cw).repeat(2, 0).repeat(2, 1)[:h, :w].astype(np.int32) - 128
+    rgb = np.stack([(298 * y + 409 * v + 128) >> 8, (298 * y - 100 * u - 208 * v + 128) >> 8, (298 * y + 516 * u + 128) >> 8], -1)
+    return np.clip(rgb, 0, 255).astype(np.uint8)
+
+
 def psnr_y(a, b, n):
     a = np.frombuffer(a, np.uint8)[:n].astype(np.float64)
     b = np.frombuffer(b, np.uint8)[:n].astype(np.float64)
@@ -83,6 +98,7 @@ def main():
     ap.add_argument("--search-range", type=int, default=16)
     ap.add_argument("--compare-streams", type=int, default=4, help="streams whose key-frame sizes and PSNR are measured")
     ap.add_argument("--profile-steps", type=int, default=3)
+    ap.add_argument("--input", choices=("host", "i420", "rgb"), default="host", help="where the pictures come from")
     ap.add_argument("--out", default=None)
     ap.add_argument("--dry-run", action="store_true", help="build the pictures of two steps and print the plan; no device")
     args = ap.parse_args()
@@ -92,7 +108,8 @@ def main():
     scene = Scene(n, w, h, args.inter + 1)
     ncmp = min(args.compare_streams, n)
     plan = {"streams": n, "width": w, "height": h, "inter_frames_per_stream": args.inter, "timed_steps": args.inter - args.warmup,
-            "q_index": args.q, "loop_filter_level": args.lf, "search_range": args.search_range, "compare_streams": ncmp}
+            "q_index": args.q, "loop_filter_level": args.lf, "search_range": args.search_range, "compare_streams": ncmp,
+            "input": args.input}
     if args.dry_run:
         t0 = time.perf_counter()
         pics = [scene.picture(s, t) for t in range(2) for s in range(n)]
@@ -107,17 +124,32 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("no CUDA device: the encoder benchmark runs on the GPU only")
     eng = vp8_b200.Engine(0)
+
+    def source(pics):
+        """The encoder's input for one step and the I420 pictures it codes (bytes)."""
+        if args.input == "host":
+            return pics, pics, "i420"
+        if args.input == "i420":
+            dev = torch.from_numpy(np.frombuffer(b"".join(pics), np.uint8).reshape(n, -1)).cuda()
+            torch.cuda.synchronize()
+            return dev, pics, "i420"
+        dev = torch.from_numpy(np.stack([rgb_from_i420(p, w, h) for p in pics])).cuda()
+        coded = [bytes(r) for r in eng.convert_to_i420(dev, "rgb", w, h).cpu().numpy()]
+        torch.cuda.synchronize()
+        return dev, coded, "rgb"
+
     streams = [eng.open_stream() for _ in range(n)]
     key_streams = [eng.open_stream() for _ in range(ncmp)]
     fb_y = w * h
     step_s, inter_bytes, key_bytes, psnr = [], [], [], []
     try:
-        for f in eng.encode_key_frames(streams, [scene.picture(s, 0) for s in range(n)], w, h, args.q, args.lf):
+        src, _, layout = source([scene.picture(s, 0) for s in range(n)])
+        for f in eng.encode_key_frames(streams, src, w, h, args.q, args.lf, layout=layout):
             f.close()
         for t in range(1, args.inter + 1):
-            pics = [scene.picture(s, t) for s in range(n)]
+            src, pics, layout = source([scene.picture(s, t) for s in range(n)])
             t0 = time.perf_counter()
-            frames = eng.encode_inter_frames(streams, pics, w, h, args.q, args.lf, search_range=args.search_range)
+            frames = eng.encode_inter_frames(streams, src, w, h, args.q, args.lf, search_range=args.search_range, layout=layout)
             dt = time.perf_counter() - t0
             if t > args.warmup:
                 step_s.append(dt)
@@ -133,11 +165,12 @@ def main():
                 f.close()
         # separate run under the profiler: kernel times of --profile-steps inter calls
         from torch.profiler import ProfilerActivity, profile
-        pics = [scene.picture(s, args.inter + 1) for s in range(n)]
+        src, _, layout = source([scene.picture(s, args.inter + 1) for s in range(n)])
         with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
             t0 = time.perf_counter()
             for _ in range(args.profile_steps):
-                for f in eng.encode_inter_frames(streams, pics, w, h, args.q, args.lf, search_range=args.search_range):
+                for f in eng.encode_inter_frames(streams, src, w, h, args.q, args.lf, search_range=args.search_range,
+                                                 layout=layout):
                     f.close()
             prof_wall = time.perf_counter() - t0
         kernels, copies = {}, {}
@@ -162,7 +195,8 @@ def main():
         "profile": {"calls": args.profile_steps, "wall_ms_per_call_under_profiler": 1e3 * prof_wall / args.profile_steps,
                     "kernel_ms_per_call": kernels, "kernels_total_ms_per_call": kernel_ms, "copy_ms_per_call": copies,
                     "rest_ms_per_call": 1e3 * prof_wall / args.profile_steps - kernel_ms,
-                    "note": "rest = host padding, staging and read-back copies, mode assignment (wall under the profiler minus kernel time)"},
+                    "note": "rest = host padding and staging copies (host input), read-back copies, mode assignment (wall under the "
+                            "profiler minus kernel time)"},
         "bytes_per_inter_frame": float(np.mean(inter_bytes)),
         "bytes_per_key_frame_same_pictures": float(np.mean(key_bytes)),
         "inter_over_key": float(np.mean(inter_bytes) / np.mean(key_bytes)),

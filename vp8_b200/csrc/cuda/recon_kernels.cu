@@ -1557,11 +1557,14 @@ constexpr int kRgbStripW = 16;
 // Stores the first n of the 4*NW bytes of w[] at d: 128-bit stores for a whole strip at a 16-byte aligned address
 // (every strip of a frame whose width is a multiple of 16, at an aligned destination), 32-bit stores at a 4-byte
 // aligned one, bytes otherwise (odd widths, the last strip of a row).
+// A strip of two words (StageSourceKernel's chroma) takes one 64-bit store at an 8-byte aligned address instead.
 template <int NW>
 __device__ __forceinline__ void StoreStrip(uint8_t *d, const unsigned (&w)[NW], int n) {
-  if (n == 4 * NW && ((size_t)d & 15) == 0) {
+  if (NW % 4 == 0 && n == 4 * NW && ((size_t)d & 15) == 0) {
 #pragma unroll
-    for (int k = 0; k < NW; k += 4) *reinterpret_cast<uint4 *>(d + 4 * k) = make_uint4(w[k], w[k + 1], w[k + 2], w[k + 3]);
+    for (int k = 0; k + 3 < NW; k += 4) *reinterpret_cast<uint4 *>(d + 4 * k) = make_uint4(w[k], w[k + 1], w[k + 2], w[k + 3]);
+  } else if (NW == 2 && n == 8 && ((size_t)d & 7) == 0) {
+    *reinterpret_cast<uint2 *>(d) = make_uint2(w[0], w[NW - 1]);
   } else if (n == 4 * NW && ((size_t)d & 3) == 0) {
 #pragma unroll
     for (int k = 0; k < NW; ++k) *reinterpret_cast<unsigned *>(d + 4 * k) = w[k];
@@ -1636,6 +1639,192 @@ __global__ void __launch_bounds__(256) ConvertRgbKernel(const DevFrameJob *__res
 }
 
 // ------------------------------------------------------------------------------------------
+// Encoder input from device memory (vp8r_encode_*_device, vp8r_convert_to_i420_device): each job's source frame
+// (job.stage_src: width x height in job.pack_layout, any byte alignment) becomes I420 by the BT.601 formula of
+// include/vp8r.h, written to the planes enc_src[0..2] (pitches enc_src_pitch_y / _c) over stage_w x stage_h luma
+// pixels.  Source coordinates are clamped to the picture: with stage_w x stage_h the macroblock-aligned size this is
+// PadToMacroblocks (rt/engine.cu) of the cropped I420 image, with the cropped size it is that image.  Same mapping as
+// ConvertRgbKernel: one thread per 16 x 2 luma strip and its 8 chroma samples.  Memory-bound (I420 / NV12: about
+// 1.5 B read and written per pixel; RGB: 3 B read, 1.5 B written).
+// ------------------------------------------------------------------------------------------
+// 4*NW bytes at p, any alignment: 128-bit loads at a 16-byte aligned address, 32-bit loads at a 4-byte aligned one,
+// otherwise NW+1 aligned words joined by funnel shifts.  Every word read holds at least one of the 4*NW bytes, so the
+// loads stay inside the pages of the buffer that holds them.
+template <int NW>
+__device__ __forceinline__ void LoadBytes(const uint8_t *p, unsigned (&w)[NW]) {
+  const unsigned r = (unsigned)(size_t)p & 3;
+  if (NW % 4 == 0 && ((size_t)p & 15) == 0) {
+#pragma unroll
+    for (int k = 0; k + 3 < NW; k += 4) {
+      const uint4 v = *reinterpret_cast<const uint4 *>(p + 4 * k);
+      w[k] = v.x, w[k + 1] = v.y, w[k + 2] = v.z, w[k + 3] = v.w;
+    }
+  } else if (r == 0) {
+#pragma unroll
+    for (int k = 0; k < NW; ++k) w[k] = reinterpret_cast<const unsigned *>(p)[k];
+  } else {
+    const unsigned *a = reinterpret_cast<const unsigned *>(p - r);
+    unsigned lo = a[0];
+#pragma unroll
+    for (int k = 0; k < NW; ++k) {
+      const unsigned hi = a[k + 1];
+      w[k] = __funnelshift_r(lo, hi, 8 * r);
+      lo = hi;
+    }
+  }
+}
+
+__device__ __forceinline__ int ByteOf(const unsigned *w, int i) { return (int)((w[i >> 2] >> (8 * (i & 3))) & 255); }
+
+// BT.601 limited range (include/vp8r.h): luma of one pixel, chroma of the sums of a 2x2 block's channels.
+__device__ __forceinline__ int LumaOf(int r, int g, int b) { return ((66 * r + 129 * g + 25 * b + 128) >> 8) + 16; }
+__device__ __forceinline__ int ChromaU(int sr, int sg, int sb) {
+  return ((-38 * ((sr + 2) >> 2) - 74 * ((sg + 2) >> 2) + 112 * ((sb + 2) >> 2) + 128) >> 8) + 128;
+}
+__device__ __forceinline__ int ChromaV(int sr, int sg, int sb) {
+  return ((112 * ((sr + 2) >> 2) - 94 * ((sg + 2) >> 2) - 18 * ((sb + 2) >> 2) + 128) >> 8) + 128;
+}
+
+__device__ __forceinline__ void RgbAt(const uint8_t *src, bool planar, int w, int h, int x, int y, int &r, int &g, int &b) {
+  const size_t o = (size_t)y * w + x;
+  if (planar) {
+    const size_t plane = (size_t)w * h;
+    r = src[o], g = src[plane + o], b = src[2 * plane + o];
+  } else {
+    r = src[3 * o], g = src[3 * o + 1], b = src[3 * o + 2];
+  }
+}
+
+// One instance per layout (a batch has one): each path gets the registers it needs.
+template <int kLayout>
+__global__ void __launch_bounds__(256) StageSourceKernel(const DevFrameJob *__restrict__ jobs) {
+  const DevFrameJob &job = jobs[blockIdx.y];
+  const uint8_t *src = job.stage_src;
+  if (!src) return;
+  constexpr int layout = kLayout;
+  const int w = job.width, h = job.height, cw = (w + 1) / 2, ch = (h + 1) / 2;
+  const int dw = job.stage_w, dh = job.stage_h, dcw = (dw + 1) / 2;
+  uint8_t *dy = const_cast<uint8_t *>(job.enc_src[0]), *du = const_cast<uint8_t *>(job.enc_src[1]),
+          *dv = const_cast<uint8_t *>(job.enc_src[2]);
+  const int py = job.enc_src_pitch_y, pc = job.enc_src_pitch_c;
+  const size_t plane = (size_t)w * h, cplane = (size_t)cw * ch;
+  const int strips = (dw + 15) / 16, items = strips * ((dh + 1) / 2);
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < items; t += gridDim.x * blockDim.x) {
+    const int pair = t / strips;
+    const int x = (t - pair * strips) * 16, y = 2 * pair, cx = x / 2;
+    // no coordinate of the strip, its 2x2 blocks or its chroma samples needs a clamp
+    const bool inside = x + 16 <= w && y + 1 < h;
+    const int cy = min(pair, ch - 1);
+    unsigned yw[2][4], uw[2], vw[2];
+    if constexpr (layout == VP8R_LAYOUT_I420 || layout == VP8R_LAYOUT_NV12) {
+      if (inside) {
+        LoadBytes(src + (size_t)y * w + x, yw[0]);
+        LoadBytes(src + (size_t)(y + 1) * w + x, yw[1]);
+        if constexpr (layout == VP8R_LAYOUT_I420) {
+          LoadBytes(src + plane + (size_t)cy * cw + cx, uw);
+          LoadBytes(src + plane + cplane + (size_t)cy * cw + cx, vw);
+        } else {
+          unsigned uv[4];
+          LoadBytes(src + plane + 2 * ((size_t)cy * cw + cx), uv);
+          uw[0] = __byte_perm(uv[0], uv[1], 0x6420), vw[0] = __byte_perm(uv[0], uv[1], 0x7531);
+          uw[1] = __byte_perm(uv[2], uv[3], 0x6420), vw[1] = __byte_perm(uv[2], uv[3], 0x7531);
+        }
+      } else {
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {
+          const uint8_t *row = src + (size_t)min(y + r, h - 1) * w;
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            unsigned v = 0;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) v |= (unsigned)row[min(x + 4 * q + k, w - 1)] << (8 * k);
+            yw[r][q] = v;
+          }
+        }
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+          unsigned u = 0, v = 0;
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const size_t o = (size_t)cy * cw + min(cx + 4 * q + k, cw - 1);
+            const size_t ou = layout == VP8R_LAYOUT_I420 ? plane + o : plane + 2 * o;
+            const size_t ov = layout == VP8R_LAYOUT_I420 ? plane + cplane + o : plane + 2 * o + 1;
+            u |= (unsigned)src[ou] << (8 * k);
+            v |= (unsigned)src[ov] << (8 * k);
+          }
+          uw[q] = u, vw[q] = v;
+        }
+      }
+    } else {
+      constexpr bool planar = layout == VP8R_LAYOUT_RGB_PLANAR;
+      int sr[8], sg[8], sb[8];  // channel sums of the strip's 2x2 blocks (inside only)
+#pragma unroll
+      for (int k = 0; k < 8; ++k) sr[k] = sg[k] = sb[k] = 0;
+#pragma unroll
+      for (int r = 0; r < 2; ++r) {
+        int Y[16];
+        if (inside) {
+          const size_t o = (size_t)(y + r) * w + x;
+          unsigned a[12];  // RGB24: the strip's 48 bytes; planar: its 16 R, then 16 G, then 16 B bytes
+          if (planar) {
+            unsigned t[4];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+              LoadBytes(src + c * plane + o, t);
+#pragma unroll
+              for (int k = 0; k < 4; ++k) a[4 * c + k] = t[k];
+            }
+          } else {
+            LoadBytes(src + 3 * o, a);
+          }
+#pragma unroll
+          for (int p = 0; p < 16; ++p) {
+            const int R = ByteOf(a, planar ? p : 3 * p), G = ByteOf(a, planar ? 16 + p : 3 * p + 1),
+                      B = ByteOf(a, planar ? 32 + p : 3 * p + 2);
+            sr[p >> 1] += R, sg[p >> 1] += G, sb[p >> 1] += B;
+            Y[p] = LumaOf(R, G, B);
+          }
+        } else {
+#pragma unroll
+          for (int p = 0; p < 16; ++p) {
+            int R, G, B;
+            RgbAt(src, planar, w, h, min(x + p, w - 1), min(y + r, h - 1), R, G, B);
+            Y[p] = LumaOf(R, G, B);
+          }
+        }
+#pragma unroll
+        for (int q = 0; q < 4; ++q) yw[r][q] = PackSat4(Y[4 * q], Y[4 * q + 1], Y[4 * q + 2], Y[4 * q + 3]);
+      }
+      if (!inside) {  // chroma sample (i, j) averages pixels (2i+a, 2j+b), i and j clamped first, then the pixels
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+          const int i = min(cx + k, cw - 1);
+          sr[k] = sg[k] = sb[k] = 0;
+#pragma unroll
+          for (int a = 0; a < 4; ++a) {
+            int r, g, b;
+            RgbAt(src, planar, w, h, min(2 * i + (a & 1), w - 1), min(2 * cy + (a >> 1), h - 1), r, g, b);
+            sr[k] += r, sg[k] += g, sb[k] += b;
+          }
+        }
+      }
+#pragma unroll
+      for (int q = 0; q < 2; ++q) {
+        uw[q] = PackSat4(ChromaU(sr[4 * q], sg[4 * q], sb[4 * q]), ChromaU(sr[4 * q + 1], sg[4 * q + 1], sb[4 * q + 1]),
+                         ChromaU(sr[4 * q + 2], sg[4 * q + 2], sb[4 * q + 2]), ChromaU(sr[4 * q + 3], sg[4 * q + 3], sb[4 * q + 3]));
+        vw[q] = PackSat4(ChromaV(sr[4 * q], sg[4 * q], sb[4 * q]), ChromaV(sr[4 * q + 1], sg[4 * q + 1], sb[4 * q + 1]),
+                         ChromaV(sr[4 * q + 2], sg[4 * q + 2], sb[4 * q + 2]), ChromaV(sr[4 * q + 3], sg[4 * q + 3], sb[4 * q + 3]));
+      }
+    }
+    const int n = min(16, dw - x), nc = min(8, dcw - cx);
+    StoreStrip(dy + (size_t)y * py + x, yw[0], n);
+    if (y + 1 < dh) StoreStrip(dy + (size_t)(y + 1) * py + x, yw[1], n);
+    StoreStrip(du + (size_t)pair * pc + cx, uw, nc);
+    StoreStrip(dv + (size_t)pair * pc + cx, vw, nc);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // host -> device staging by the SMs (zero-copy reads of pinned host memory)
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) CopyKernel(uint4 *__restrict__ dst, const uint4 *__restrict__ src, size_t n16) {
@@ -1680,6 +1869,19 @@ cudaError_t LaunchConvertRgb(const DevFrameJob *jobs, int n_frames, int max_w, i
   const int items = (max_w + kRgbStripW - 1) / kRgbStripW * ((max_h + 1) / 2);
   dim3 grid((unsigned)std::max(1, std::min(48, (items + 255) / 256)), n_frames);
   ConvertRgbKernel<<<grid, 256, 0, st>>>(jobs);
+  return cudaGetLastError();
+}
+
+cudaError_t LaunchStageSource(const DevFrameJob *jobs, int n_frames, int layout, int max_w, int max_h, cudaStream_t st) {
+  const int items = (max_w + 15) / 16 * ((max_h + 1) / 2);
+  dim3 grid((unsigned)std::max(1, std::min(48, (items + 255) / 256)), n_frames);
+  switch (layout) {
+    case VP8R_LAYOUT_I420: StageSourceKernel<VP8R_LAYOUT_I420><<<grid, 256, 0, st>>>(jobs); break;
+    case VP8R_LAYOUT_NV12: StageSourceKernel<VP8R_LAYOUT_NV12><<<grid, 256, 0, st>>>(jobs); break;
+    case VP8R_LAYOUT_RGB24: StageSourceKernel<VP8R_LAYOUT_RGB24><<<grid, 256, 0, st>>>(jobs); break;
+    case VP8R_LAYOUT_RGB_PLANAR: StageSourceKernel<VP8R_LAYOUT_RGB_PLANAR><<<grid, 256, 0, st>>>(jobs); break;
+    default: return cudaErrorInvalidValue;
+  }
   return cudaGetLastError();
 }
 

@@ -52,7 +52,8 @@ struct DevFrameJob {
   int16_t dq[4][6];
   uint8_t key_frame, version, filter_type, lf_level, sharpness;
   uint8_t levels_in_one_launch;  // host-built level table walked by IntraLevelsKernel instead of one launch per level
-  uint8_t pack_layout;           // PackKernel: VP8R_LAYOUT_I420 / _NV12; ConvertRgbKernel: VP8R_LAYOUT_RGB24 / _RGB_PLANAR
+  uint8_t pack_layout;           // PackKernel: VP8R_LAYOUT_I420 / _NV12; ConvertRgbKernel: VP8R_LAYOUT_RGB24 / _RGB_PLANAR;
+                                 // StageSourceKernel: the layout of stage_src (any of the four)
   uint8_t enc_flags;             // K_encode: VP8R_ENC_*
   // output side (crop / checksum)
   int width, height;
@@ -82,6 +83,10 @@ struct DevFrameJob {
   const uint8_t *enc_src[3];
   int enc_src_pitch_y, enc_src_pitch_c;
   int enc_search_range;          // K_encode_inter: full-pel search range (whole pixels, 4..24)
+  // StageSourceKernel: a width x height frame in pack_layout at stage_src (device memory, any alignment) becomes the
+  // I420 planes enc_src[0..2] over stage_w x stage_h luma pixels (source coordinates clamped to the frame)
+  const uint8_t *stage_src;
+  int stage_w, stage_h;
 };
 
 // A frame whose device-side parse ran past the end of a partition: its records are not trustworthy, so no
@@ -157,6 +162,10 @@ cudaError_t LaunchPack(const DevFrameJob *jobs, int n_frames, cudaStream_t st);
 // Device-side crop + BT.601 YUV -> RGB (VP8R_LAYOUT_RGB24 / _RGB_PLANAR, from job.pack_layout) of each job's current
 // surface into job.pack_dst.  max_w, max_h: the largest frame of the batch (sizes the grid).
 cudaError_t LaunchConvertRgb(const DevFrameJob *jobs, int n_frames, int max_w, int max_h, cudaStream_t st);
+// Device-side layout / BT.601 conversion + edge padding of each job's stage_src into its enc_src planes
+// (StageSourceKernel).  layout: the pack_layout of every job; max_w, max_h: the largest stage_w x stage_h of the batch
+// (sizes the grid).
+cudaError_t LaunchStageSource(const DevFrameJob *jobs, int n_frames, int layout, int max_w, int max_h, cudaStream_t st);
 // Device-side checksum of the cropped I420 image of each job's current surface.
 cudaError_t LaunchChecksum(const DevFrameJob *jobs, int n_frames, cudaStream_t st);
 

@@ -635,21 +635,85 @@ void RefreshRefs(vp8r_stream *s, const vp8r_frame_hdr &h, int cur) {
   s->have_frame = true;
 }
 
+// Where an encoder batch's pictures come from: cropped I420 images in host memory, one per frame (host), or n frames
+// in device memory of the engine's device, frame i at dev + i*stride in `layout` (StageSourceKernel converts them).
+struct EncoderSource {
+  const uint8_t *const *host = nullptr;
+  const uint8_t *dev = nullptr;
+  size_t stride = 0;
+  int layout = VP8R_LAYOUT_I420;
+  cudaStream_t producer = nullptr;  // the stream dev was written on (nullptr: nothing to wait for)
+};
+
+// Bytes of one width x height frame in a source / device layout.
+size_t LayoutBytes(int layout, int width, int height) {
+  if (layout == VP8R_LAYOUT_RGB24 || layout == VP8R_LAYOUT_RGB_PLANAR) return 3 * size_t(width) * height;
+  return size_t(width) * height + 2 * size_t((width + 1) / 2) * ((height + 1) / 2);
+}
+
+// A pointer into device memory of the engine's device (pinned, pageable and managed memory are not).
+bool IsEngineDeviceMemory(const vp8r_engine *e, const void *p) {
+  cudaPointerAttributes attr{};
+  if (cudaPointerGetAttributes(&attr, p) != cudaSuccess) {
+    cudaGetLastError();
+    return false;
+  }
+  return attr.type == cudaMemoryTypeDevice && attr.device == e->device;
+}
+
 // The arguments both encoders take.
-int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420, vp8r_frame *const *out,
+int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, vp8r_frame *const *out,
                      int width, int height, int q_index, int loop_filter_level, int sharpness) {
-  if (!e || n <= 0 || !streams || !i420 || !out || width < 1 || height < 1 || width > 16383 || height > 16383 || q_index < 0 ||
-      q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 || sharpness > 7)
+  if (!e || n <= 0 || !streams || !(src.host || src.dev) || !out || width < 1 || height < 1 || width > 16383 ||
+      height > 16383 || q_index < 0 || q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 ||
+      sharpness > 7)
     return VP8R_ERR_INVALID_ARG;
   int rc = EnsureDevice(e);
   if (rc) return rc;
   rc = CheckBatchStreams(e, n, streams);
   if (rc) return rc;
   for (int i = 0; i < n; ++i)
-    if (!i420[i] || !out[i]) {
+    if ((src.host && !src.host[i]) || !out[i]) {
       SetError("null image or frame");
       return VP8R_ERR_INVALID_ARG;
     }
+  if (src.dev && !IsEngineDeviceMemory(e, src.dev)) {
+    SetError("src is not device memory of the engine's device (pinned, pageable and managed memory are refused)");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  return VP8R_OK;
+}
+
+// The checks of an encoder call with its source in device memory that need no device, with a message for each;
+// `what` names the call.  The encoder's other argument checks follow in CheckEncoderArgs.
+int CheckDeviceSourceArgs(const char *what, const vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src,
+                          size_t stride, int layout, vp8r_frame *const *out, int width, int height, int q_index,
+                          int loop_filter_level, int sharpness) {
+  const std::string call(what);
+  if (!e || !streams || !src || !out) {
+    SetError(call + ": null engine, streams, src or out");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (n <= 0) {
+    SetError(call + ": n <= 0");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
+    SetError(call + ": unknown layout " + std::to_string(layout));
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (width < 1 || height < 1 || width > 16383 || height > 16383) {
+    SetError(call + ": frame size outside 1..16383");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (q_index < 0 || q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 || sharpness > 7) {
+    SetError(call + ": q_index, loop_filter_level or sharpness out of range");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (stride < LayoutBytes(layout, width, height)) {
+    SetError(call + ": stride smaller than a frame");
+    return VP8R_ERR_INVALID_ARG;
+  }
   return VP8R_OK;
 }
 
@@ -683,20 +747,24 @@ EncodeLayout MakeEncodeLayout(int width, int height, int q_index, int loop_filte
   return L;
 }
 
-// Pads each image and uploads it into its frame's part of the slot arena, then fills the job fields both encoders
-// set; cur[i] is the surface frame i is reconstructed into.
-int StageEncoderSources(vp8r_engine *e, Slot &sl, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
+// Fills the job fields both encoders set and stages each frame's source picture, padded to whole macroblocks, in its
+// part of the slot arena: a host image is padded here and uploaded; a device source is converted and padded there by
+// StageSourceKernel, which SubmitEncoderJobs launches once the job table is on the device.  cur[i] is the surface
+// frame i is reconstructed into.
+int StageEncoderSources(vp8r_engine *e, Slot &sl, int n, vp8r_stream *const *streams, const EncoderSource &src,
                         const EncodeLayout &L, std::vector<int> *cur) {
   const vp8r_frame_hdr &h = L.h;
   const int cols = h.mb_cols, rows = h.mb_rows, sp_y = cols * 16, sp_c = cols * 8;
-  std::vector<uint8_t> padded(L.src_bytes);
+  std::vector<uint8_t> padded(src.host ? L.src_bytes : 0);
   cur->assign(size_t(n), -1);
   for (int i = 0; i < n; ++i) {
     vp8r_stream *s = streams[i];
-    PadToMacroblocks(i420[i], h.width, h.height, cols, rows, padded.data());
     uint8_t *base = sl.d_arena + L.per_frame * size_t(i);
-    CU_TRY(cudaMemcpyAsync(base, padded.data(), L.src_bytes, cudaMemcpyHostToDevice, e->st));
-    CU_TRY(cudaStreamSynchronize(e->st));  // `padded` is reused for the next image
+    if (src.host) {
+      PadToMacroblocks(src.host[i], h.width, h.height, cols, rows, padded.data());
+      CU_TRY(cudaMemcpyAsync(base, padded.data(), L.src_bytes, cudaMemcpyHostToDevice, e->st));
+      CU_TRY(cudaStreamSynchronize(e->st));  // `padded` is reused for the next image
+    }
     (*cur)[size_t(i)] = PickCurrent(s);
     DevFrameJob &j = sl.h_jobs[i];
     std::memset(&j, 0, sizeof(j));
@@ -712,8 +780,30 @@ int StageEncoderSources(vp8r_engine *e, Slot &sl, int n, vp8r_stream *const *str
     j.enc_src[2] = j.enc_src[1] + size_t(sp_c) * rows * 8;
     j.enc_src_pitch_y = sp_y;
     j.enc_src_pitch_c = sp_c;
+    if (src.dev) {
+      j.stage_src = src.dev + size_t(i) * src.stride;
+      j.pack_layout = uint8_t(src.layout);
+      j.stage_w = sp_y;
+      j.stage_h = rows * 16;
+    }
     e->acc.frames++;
   }
+  return VP8R_OK;
+}
+
+// Builds the batch's filter groups and puts its job table on the device; for a device source, the engine's stream
+// then waits for the producer stream and StageSourceKernel stages the pictures.  *n_groups: the filter groups.
+int SubmitEncoderJobs(vp8r_engine *e, Slot &sl, int n, const EncoderSource &src, const EncodeLayout &L, int *n_groups) {
+  *n_groups = BuildFilterGroups(e, sl, n);
+  CU_TRY(vp8r::LaunchCopy(sl.d_jobs, sl.h_jobs, sizeof(DevFrameJob) * n + sizeof(vp8r::FilterGroup) * *n_groups, e->st));
+  if (!src.dev) return VP8R_OK;
+  if (src.producer && src.producer != e->st) {
+    CU_TRY(cudaEventRecord(e->consumer_ev, src.producer));
+    CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
+  }
+  ScopedTimer t(e, 3);
+  CU_TRY(vp8r::LaunchStageSource(sl.d_jobs, n, src.layout, L.h.mb_cols * 16, L.h.mb_rows * 16, e->st));
+  e->acc.launches_other++;
   return VP8R_OK;
 }
 
@@ -743,6 +833,102 @@ int FinishEncoderBatch(vp8r_engine *e, const Slot &sl, int n, vp8r_stream *const
     const vp8r_mb_info *mbs = out[i]->mbs();
     for (size_t m = 0; m < L.n_mb; ++m) blocks += uint32_t(__builtin_popcount(mbs[m].coef_mask));
     out[i]->hdr.n_coef_blocks = blocks;
+  }
+  return VP8R_OK;
+}
+
+// Row f4: closed-loop key-frame encoder (vp8r_encode_key_frames, _device).
+int EncodeKeyFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, int width, int height,
+                    int q_index, int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out) {
+  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness);
+  if (rc) return rc;
+  EncodeLayout L = MakeEncodeLayout(width, height, q_index, loop_filter_level, sharpness);
+  L.h.key_frame = 1;
+  L.h.refresh_golden = L.h.refresh_altref = 1;
+  for (int i = 0; i < n; ++i) {
+    rc = ConfigureStream(streams[i], L.h);
+    if (rc) return rc;
+    streams[i]->failed = false;
+  }
+  int slot_index;
+  rc = TakeSlot(e, n, L.per_frame * size_t(n), &slot_index, nullptr);
+  if (rc) return rc;
+  Slot &sl = e->slots[slot_index];
+  std::vector<int> cur;
+  rc = StageEncoderSources(e, sl, n, streams, src, L, &cur);
+  if (rc) return rc;
+  for (int i = 0; i < n; ++i) {
+    sl.h_jobs[i].n_intra = int(L.n_mb);
+    sl.h_jobs[i].enc_flags = uint8_t(flags);
+  }
+  int n_groups = 0;
+  rc = SubmitEncoderJobs(e, sl, n, src, L, &n_groups);
+  if (rc) return rc;
+  {
+    ScopedTimer t(e, 1);
+    CU_TRY(vp8r::LaunchEncodeIntra(sl.d_jobs, n, L.h.mb_rows, e->st));
+    e->acc.launches_intra++;
+  }
+  rc = LaunchFilterAndBorder(e, sl, n, L.h.mb_rows, n_groups);
+  if (rc) return rc;
+  return FinishEncoderBatch(e, sl, n, streams, cur, L, out);
+}
+
+// Row f4, inter frames: every macroblock predicts from LAST with one vector (K_encode_inter), the decoder's own
+// K_inter reconstructs from the records, then the loop filter and the border as for a decoded frame.
+int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, int width, int height,
+                      int q_index, int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out) {
+  if (search_range < 4 || search_range > 24) return VP8R_ERR_INVALID_ARG;
+  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness);
+  if (rc) return rc;
+  for (int i = 0; i < n; ++i) {
+    const vp8r_stream *s = streams[i];
+    if (!s->have_frame || s->failed || s->ref[1] < 0) {
+      SetError("inter frame for a stream without a frame to predict from");
+      return VP8R_ERR_STATE;
+    }
+    if (s->width != width || s->height != height) {
+      SetError("inter frame of another size than the stream's frames");
+      return VP8R_ERR_STATE;
+    }
+  }
+  const EncodeLayout L = MakeEncodeLayout(width, height, q_index, loop_filter_level, sharpness);
+  const int cols = L.h.mb_cols, rows = L.h.mb_rows;
+  int slot_index;
+  rc = TakeSlot(e, n, L.per_frame * size_t(n), &slot_index, nullptr);
+  if (rc) return rc;
+  Slot &sl = e->slots[slot_index];
+  std::vector<int> cur;
+  rc = StageEncoderSources(e, sl, n, streams, src, L, &cur);
+  if (rc) return rc;
+  bool tma = e->inter_tma;
+  for (int i = 0; i < n; ++i) {
+    sl.h_jobs[i].n_inter = int(L.n_mb);
+    sl.h_jobs[i].enc_search_range = search_range;
+    tma = tma && streams[i]->d_tmaps != nullptr;
+  }
+  int n_groups = 0;
+  rc = SubmitEncoderJobs(e, sl, n, src, L, &n_groups);
+  if (rc) return rc;
+  {
+    ScopedTimer t(e, 0);
+    CU_TRY(vp8r::LaunchEncodeInter(sl.d_jobs, n, cols, rows, e->st));
+    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st, tma));
+    e->acc.launches_inter += 2;
+  }
+  rc = LaunchFilterAndBorder(e, sl, n, rows, n_groups);
+  if (rc) return rc;
+  // The references move with the reconstruction (golden and altref stay), even if a mode cannot be assigned below.
+  rc = FinishEncoderBatch(e, sl, n, streams, cur, L, out);
+  if (rc) return rc;
+  for (int i = 0; i < n; ++i) {
+    std::string err;
+    rc = vp8r::AssignInterModes(out[i]->mbs(), cols, rows, &err);
+    if (rc) {
+      SetError(err);
+      return rc;
+    }
+    out[i]->hdr.n_inter_mbs = uint32_t(L.n_mb);
   }
   return VP8R_OK;
 }
@@ -1173,95 +1359,119 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
 // Row f4: closed-loop key-frame encoder.
 VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420, int width,
                                     int height, int q_index, int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out) {
-  int rc = CheckEncoderArgs(e, n, streams, i420, out, width, height, q_index, loop_filter_level, sharpness);
-  if (rc) return rc;
-  EncodeLayout L = MakeEncodeLayout(width, height, q_index, loop_filter_level, sharpness);
-  L.h.key_frame = 1;
-  L.h.refresh_golden = L.h.refresh_altref = 1;
-  for (int i = 0; i < n; ++i) {
-    rc = ConfigureStream(streams[i], L.h);
-    if (rc) return rc;
-    streams[i]->failed = false;
-  }
-  int slot_index;
-  rc = TakeSlot(e, n, L.per_frame * size_t(n), &slot_index, nullptr);
-  if (rc) return rc;
-  Slot &sl = e->slots[slot_index];
-  std::vector<int> cur;
-  rc = StageEncoderSources(e, sl, n, streams, i420, L, &cur);
-  if (rc) return rc;
-  for (int i = 0; i < n; ++i) {
-    sl.h_jobs[i].n_intra = int(L.n_mb);
-    sl.h_jobs[i].enc_flags = uint8_t(flags);
-  }
-  const int n_groups = BuildFilterGroups(e, sl, n);
-  CU_TRY(vp8r::LaunchCopy(sl.d_jobs, sl.h_jobs, sizeof(DevFrameJob) * n + sizeof(vp8r::FilterGroup) * n_groups, e->st));
-  {
-    ScopedTimer t(e, 1);
-    CU_TRY(vp8r::LaunchEncodeIntra(sl.d_jobs, n, L.h.mb_rows, e->st));
-    e->acc.launches_intra++;
-  }
-  rc = LaunchFilterAndBorder(e, sl, n, L.h.mb_rows, n_groups);
-  if (rc) return rc;
-  return FinishEncoderBatch(e, sl, n, streams, cur, L, out);
+  EncoderSource src;
+  src.host = i420;
+  return EncodeKeyFrames(e, n, streams, src, width, height, q_index, loop_filter_level, sharpness, flags, out);
 }
 
-// Row f4, inter frames: every macroblock predicts from LAST with one vector (K_encode_inter), the decoder's own
-// K_inter reconstructs from the records, then the loop filter and the border as for a decoded frame.
+VP8R_API int vp8r_encode_key_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
+                                           int layout, void *producer_stream, int width, int height, int q_index,
+                                           int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out) {
+  int rc = CheckDeviceSourceArgs("vp8r_encode_key_frames_device", e, n, streams, src, stride, layout, out, width, height,
+                                 q_index, loop_filter_level, sharpness);
+  if (rc) return rc;
+  EncoderSource s;
+  s.dev = static_cast<const uint8_t *>(src);
+  s.stride = stride;
+  s.layout = layout;
+  s.producer = static_cast<cudaStream_t>(producer_stream);
+  return EncodeKeyFrames(e, n, streams, s, width, height, q_index, loop_filter_level, sharpness, flags, out);
+}
+
 VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
                                       int width, int height, int q_index, int loop_filter_level, int sharpness,
                                       int search_range, vp8r_frame *const *out) {
-  if (search_range < 4 || search_range > 24) return VP8R_ERR_INVALID_ARG;
-  int rc = CheckEncoderArgs(e, n, streams, i420, out, width, height, q_index, loop_filter_level, sharpness);
+  EncoderSource src;
+  src.host = i420;
+  return EncodeInterFrames(e, n, streams, src, width, height, q_index, loop_filter_level, sharpness, search_range, out);
+}
+
+VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
+                                             int layout, void *producer_stream, int width, int height, int q_index,
+                                             int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out) {
+  int rc = CheckDeviceSourceArgs("vp8r_encode_inter_frames_device", e, n, streams, src, stride, layout, out, width, height,
+                                 q_index, loop_filter_level, sharpness);
   if (rc) return rc;
+  if (search_range < 4 || search_range > 24) {
+    SetError("vp8r_encode_inter_frames_device: search_range outside 4..24");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  EncoderSource s;
+  s.dev = static_cast<const uint8_t *>(src);
+  s.stride = stride;
+  s.layout = layout;
+  s.producer = static_cast<cudaStream_t>(producer_stream);
+  return EncodeInterFrames(e, n, streams, s, width, height, q_index, loop_filter_level, sharpness, search_range, out);
+}
+
+VP8R_API int vp8r_convert_to_i420_device(vp8r_engine *e, int n, const void *src, size_t src_stride, int layout, int width,
+                                         int height, void *dst, size_t dst_stride, void *stream) {
+  // argument checks that need no device come first
+  if (!e || !src || !dst) {
+    SetError("vp8r_convert_to_i420_device: null engine, src or dst");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (n <= 0) {
+    SetError("vp8r_convert_to_i420_device: n <= 0");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
+    SetError("vp8r_convert_to_i420_device: unknown layout " + std::to_string(layout));
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (width < 1 || height < 1 || width > 16383 || height > 16383) {
+    SetError("vp8r_convert_to_i420_device: frame size outside 1..16383");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (src_stride < LayoutBytes(layout, width, height)) {
+    SetError("vp8r_convert_to_i420_device: stride smaller than a frame");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (dst_stride < LayoutBytes(VP8R_LAYOUT_I420, width, height)) {
+    SetError("vp8r_convert_to_i420_device: dst_stride smaller than an I420 frame");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  int rc = EnsureDevice(e);
+  if (rc) return rc;
+  if (!IsEngineDeviceMemory(e, src) || !IsEngineDeviceMemory(e, dst)) {
+    SetError("vp8r_convert_to_i420_device: src or dst is not device memory of the engine's device (pinned, pageable "
+             "and managed memory are refused)");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  rc = EnsureScratchJobs(e, n);
+  if (rc) return rc;
+  int part = 0;
+  rc = AcquirePart(e, &part);
+  if (rc) return rc;
+  DevFrameJob *hj = e->h_cjobs + size_t(part) * e->cap_cjobs;
+  DevFrameJob *dj = e->d_cjobs + size_t(part) * e->cap_cjobs;
+  const size_t cw = size_t(width + 1) / 2, ch = size_t(height + 1) / 2;
   for (int i = 0; i < n; ++i) {
-    const vp8r_stream *s = streams[i];
-    if (!s->have_frame || s->failed || s->ref[1] < 0) {
-      SetError("inter frame for a stream without a frame to predict from");
-      return VP8R_ERR_STATE;
-    }
-    if (s->width != width || s->height != height) {
-      SetError("inter frame of another size than the stream's frames");
-      return VP8R_ERR_STATE;
-    }
+    DevFrameJob &j = hj[i];
+    std::memset(&j, 0, sizeof(j));
+    uint8_t *d = static_cast<uint8_t *>(dst) + size_t(i) * dst_stride;
+    j.stage_src = static_cast<const uint8_t *>(src) + size_t(i) * src_stride;
+    j.pack_layout = uint8_t(layout);
+    j.width = j.stage_w = width;
+    j.height = j.stage_h = height;
+    j.enc_src[0] = d;
+    j.enc_src[1] = d + size_t(width) * height;
+    j.enc_src[2] = j.enc_src[1] + cw * ch;
+    j.enc_src_pitch_y = width;
+    j.enc_src_pitch_c = int(cw);
   }
-  const EncodeLayout L = MakeEncodeLayout(width, height, q_index, loop_filter_level, sharpness);
-  const int cols = L.h.mb_cols, rows = L.h.mb_rows;
-  int slot_index;
-  rc = TakeSlot(e, n, L.per_frame * size_t(n), &slot_index, nullptr);
-  if (rc) return rc;
-  Slot &sl = e->slots[slot_index];
-  std::vector<int> cur;
-  rc = StageEncoderSources(e, sl, n, streams, i420, L, &cur);
-  if (rc) return rc;
-  bool tma = e->inter_tma;
-  for (int i = 0; i < n; ++i) {
-    sl.h_jobs[i].n_inter = int(L.n_mb);
-    sl.h_jobs[i].enc_search_range = search_range;
-    tma = tma && streams[i]->d_tmaps != nullptr;
+  cudaStream_t user = static_cast<cudaStream_t>(stream);
+  const bool cross = user && user != e->st;
+  if (cross) {  // the source is written, and earlier work may still read dst, on the caller's stream
+    CU_TRY(cudaEventRecord(e->consumer_ev, user));
+    CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
   }
-  const int n_groups = BuildFilterGroups(e, sl, n);
-  CU_TRY(vp8r::LaunchCopy(sl.d_jobs, sl.h_jobs, sizeof(DevFrameJob) * n + sizeof(vp8r::FilterGroup) * n_groups, e->st));
-  {
-    ScopedTimer t(e, 0);
-    CU_TRY(vp8r::LaunchEncodeInter(sl.d_jobs, n, cols, rows, e->st));
-    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st, tma));
-    e->acc.launches_inter += 2;
-  }
-  rc = LaunchFilterAndBorder(e, sl, n, rows, n_groups);
-  if (rc) return rc;
-  // The references move with the reconstruction (golden and altref stay), even if a mode cannot be assigned below.
-  rc = FinishEncoderBatch(e, sl, n, streams, cur, L, out);
-  if (rc) return rc;
-  for (int i = 0; i < n; ++i) {
-    std::string err;
-    rc = vp8r::AssignInterModes(out[i]->mbs(), cols, rows, &err);
-    if (rc) {
-      SetError(err);
-      return rc;
-    }
-    out[i]->hdr.n_inter_mbs = uint32_t(L.n_mb);
-  }
+  CU_TRY(vp8r::LaunchCopy(dj, hj, sizeof(DevFrameJob) * n, e->st));
+  CU_TRY(vp8r::LaunchStageSource(dj, n, layout, width, height, e->st));
+  e->acc.launches_other++;
+  CU_TRY(cudaEventRecord(e->pack_done[part], e->st));
+  e->kernel_busy[part] = true;
+  if (cross) CU_TRY(cudaStreamWaitEvent(user, e->pack_done[part], 0));
   return VP8R_OK;
 }
 

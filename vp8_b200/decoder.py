@@ -15,6 +15,11 @@ from ._capi import check
 DEVICE_LAYOUTS = {"i420": 0, "nv12": 1, "rgb": 2, "rgb_planar": 3}  # VP8R_LAYOUT_*
 
 
+def _is_tensor(x):
+    """A torch.Tensor, without importing torch for callers that never pass one."""
+    return type(x).__module__.startswith("torch") and hasattr(x, "data_ptr")
+
+
 def _layout_bytes(stream, layout):
     """Bytes of the stream's latest frame in a device read-back layout (0 before its first frame)."""
     if layout in ("i420", "nv12") or stream.frame_bytes() == 0:
@@ -116,27 +121,42 @@ class Engine:
         fa = (C.c_void_p * n)(*[f.handle for f in frames])
         check(self._lib.vp8r_reconstruct_batch(self.handle, n, sa, fa))
 
-    def encode_key_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, bpred=True):
+    def encode_key_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, bpred=True,
+                          layout="i420"):
         """Row f4: one key frame per stream from cropped I420 images (bytes), encoded in a closed loop on the device.
         Returns the ParsedFrame objects (macroblock records + coefficient blocks; .write_bitstream() serialises them);
         every stream then holds the reconstructed frame a decoder would produce.  bpred: B_PRED (sixteen 4x4 modes per
-        macroblock) competes with the four 16x16 modes (VP8R_ENC_BPRED)."""
-        return self._encode(self._lib.vp8r_encode_key_frames, streams, images, width, height, q_index, loop_filter_level,
-                            sharpness, 1 if bpred else 0)
+        macroblock) competes with the four 16x16 modes (VP8R_ENC_BPRED).  `images` may instead be a contiguous
+        torch.uint8 CUDA tensor on the engine's device with one frame per stream along its first dimension, in `layout`
+        (see _device_source); it is read on the device, ordered behind the work queued on torch's current stream."""
+        return self._encode(self._lib.vp8r_encode_key_frames, self._lib.vp8r_encode_key_frames_device, streams, images,
+                            layout, width, height, q_index, loop_filter_level, sharpness, 1 if bpred else 0)
 
-    def encode_inter_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, search_range=16):
+    def encode_inter_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, search_range=16,
+                            layout="i420"):
         """One inter frame per stream from cropped I420 images (bytes): every macroblock predicts from the stream's
         current LAST frame with one motion vector, searched on the device over +-search_range whole pixels (4..24) and
         refined to quarter pel (vp8r_encode_inter_frames).  Returns the ParsedFrame objects (records with modes and
         vectors, coefficient blocks; .write_bitstream() serialises them); every stream then holds the reconstructed
-        frame a decoder would produce."""
-        return self._encode(self._lib.vp8r_encode_inter_frames, streams, images, width, height, q_index, loop_filter_level,
-                            sharpness, search_range)
+        frame a decoder would produce.  `images` and `layout` as for encode_key_frames."""
+        return self._encode(self._lib.vp8r_encode_inter_frames, self._lib.vp8r_encode_inter_frames_device, streams, images,
+                            layout, width, height, q_index, loop_filter_level, sharpness, search_range)
 
-    def _encode(self, fn, streams, images, width, height, *params):
-        """Calls the C encoder entry point fn(engine, n, streams, images, width, height, *params, frames) on one cropped
-        I420 image (bytes) per stream; returns the new ParsedFrame objects."""
+    def _encode(self, fn, fn_device, streams, images, layout, width, height, *params):
+        """Calls the C encoder entry point on one picture per stream: fn(engine, n, streams, images, width, height,
+        *params, frames) for cropped I420 images (bytes), fn_device(engine, n, streams, src, stride, layout, producer,
+        width, height, *params, frames) for a CUDA tensor; returns the new ParsedFrame objects."""
         n = len(streams)
+        if _is_tensor(images):
+            src, stride, code, producer = self._device_source(images, n, layout, width, height)
+            frames = [ParsedFrame(pinned=False) for _ in range(n)]
+            sa = (C.c_void_p * n)(*[s.handle for s in streams])
+            fa = (C.c_void_p * n)(*[f.handle for f in frames])
+            check(fn_device(self.handle, n, sa, C.c_void_p(src), stride, code, C.c_void_p(producer), width, height, *params,
+                            fa))
+            return frames
+        if layout != "i420":
+            raise ValueError(f"layout {layout!r} needs a CUDA tensor: images in host memory are cropped I420 bytes")
         need = width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2)
         bufs = []
         for img in images:
@@ -149,6 +169,42 @@ class Engine:
         fa = (C.c_void_p * n)(*[f.handle for f in frames])
         check(fn(self.handle, n, sa, ia, width, height, *params, fa))
         return frames
+
+    def _device_source(self, src, n, layout, width, height):
+        """Checks a tensor of n source frames: torch.uint8, contiguous, on the engine's device, of shape (n, frame bytes)
+        for "i420" / "nv12", (n, H, W, 3) for "rgb", (n, 3, H, W) for "rgb_planar".  Returns (address, stride, layout
+        code, producer stream): the producer is torch's current stream, named by cudaStreamLegacy (1) when it is the
+        default stream, whose handle 0 the C calls read as "no stream"."""
+        import torch
+        if layout not in DEVICE_LAYOUTS:
+            raise ValueError(f"unknown layout {layout!r}: one of {sorted(DEVICE_LAYOUTS)}")
+        if src.dtype != torch.uint8:
+            raise ValueError("source tensor must be torch.uint8")
+        if src.device != torch.device("cuda", self.device):
+            raise ValueError(f"source tensor is on {src.device}, the engine on cuda:{self.device}")
+        if not src.is_contiguous():
+            raise ValueError("source tensor must be contiguous")
+        shape = {"rgb": (height, width, 3), "rgb_planar": (3, height, width)}.get(
+            layout, (width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2),))
+        if tuple(src.shape) != (n,) + shape:
+            raise ValueError(f"source tensor has shape {tuple(src.shape)}, {layout} frames of {width}x{height} for {n} "
+                             f"streams need {(n,) + shape}")
+        producer = torch.cuda.current_stream(src.device).cuda_stream or 1
+        return src.data_ptr(), src[0].numel(), DEVICE_LAYOUTS[layout], producer
+
+    def convert_to_i420(self, src, layout, width, height):
+        """The cropped I420 images the encoder codes for a CUDA tensor of n frames in `layout` (as encode_key_frames
+        takes it): returns an (n, frame bytes) torch.uint8 CUDA tensor, computed on torch's current stream's order
+        (vp8r_convert_to_i420_device)."""
+        import torch
+        n = src.shape[0] if src.dim() else 0
+        s, stride, code, stream = self._device_source(src, n, layout, width, height)
+        fb = width * height + 2 * ((width + 1) // 2) * ((height + 1) // 2)
+        out = torch.empty((n, fb), dtype=torch.uint8, device=src.device)
+        if n:
+            check(self._lib.vp8r_convert_to_i420_device(self.handle, n, C.c_void_p(s), stride, code, width, height,
+                                                        C.c_void_p(out.data_ptr()), fb, C.c_void_p(stream)))
+        return out
 
     def upload(self, frame, release_host=False):
         """Copies the frame's arrays to HBM; release_host frees the host copy afterwards."""
@@ -308,10 +364,11 @@ def decode_ivf(path_or_bytes, engine=None, layout=None):
 
 
 def encode_ivf(images, width, height, q_index, path=None, key_interval=0, loop_filter_level=0, sharpness=0, bpred=True,
-               search_range=16, engine=None):
+               search_range=16, engine=None, layout="i420"):
     """Encodes one stream of cropped I420 images (bytes) into an IVF file, the mirror of decode_ivf: a key frame first
     and then every key_interval frames (0: only the first), inter frames between them.  Returns the IVF bytes and
-    writes them to `path` when one is given."""
+    writes them to `path` when one is given.  `images` may instead be a (T, ...) torch.uint8 CUDA tensor of T frames in
+    `layout` (see Engine.encode_key_frames), such as decode_ivf(..., layout="i420") returns: no pixel then crosses PCIe."""
     from .ivf import ivf_bytes
     if key_interval < 0:
         raise ValueError("key_interval must be >= 0")
@@ -320,12 +377,14 @@ def encode_ivf(images, width, height, q_index, path=None, key_interval=0, loop_f
     st = engine.open_stream()
     payloads = []
     try:
-        for i, img in enumerate(images):
+        pictures = (images[i:i + 1] for i in range(len(images))) if _is_tensor(images) else ([img] for img in images)
+        for i, img in enumerate(pictures):
             if i == 0 or (key_interval and i % key_interval == 0):
-                (f,) = engine.encode_key_frames([st], [img], width, height, q_index, loop_filter_level, sharpness, bpred)
+                (f,) = engine.encode_key_frames([st], img, width, height, q_index, loop_filter_level, sharpness, bpred,
+                                                layout=layout)
             else:
-                (f,) = engine.encode_inter_frames([st], [img], width, height, q_index, loop_filter_level, sharpness,
-                                                  search_range)
+                (f,) = engine.encode_inter_frames([st], img, width, height, q_index, loop_filter_level, sharpness,
+                                                  search_range, layout=layout)
             payloads.append(f.write_bitstream())
             f.close()
     finally:
