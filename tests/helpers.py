@@ -135,3 +135,165 @@ def synth_stream(args):
 
 def synth_golden(name):
     return [l.split()[0] for l in open(os.path.join(SYN_DIR, name + ".md5"))]
+
+
+# ---- randomised generator settings and the decode paths they run on ----------------------------------------------
+def randomised_configs():
+    """vp8synth settings of the randomised parity matrix.  The first 60 draws are the original matrix (all four
+    versions, both filters, every sharpness, 1-8 partitions, odd sizes, SPLIT / intra / B_PRED mixes, GOP lengths);
+    the 40 after them add the syntax extremes (DCT_CAT6 magnitudes, vectors beyond the frame, probability updates,
+    no skip flag) and frames of 1, 12, 13, 24 and 25 macroblock rows, across the 12-row bands of the loop filter.
+    The 1-row frames use 8 partitions, so some partitions own no row."""
+    import random
+    rng = random.Random(20261018)
+    cfgs = []
+    for k in range(60):
+        w, h = rng.choice([(16, 16), (17, 33), (48, 64), (96, 80), (130, 98), (176, 144), (250, 120), (320, 16)])
+        cfgs.append(f"--width {w} --height {h} --frames {rng.randint(3, 9)} --seed {1000 + k} "
+                    f"--version {rng.randint(0, 3)} --filter-type {rng.randint(0, 1)} --sharpness {rng.randint(0, 7)} "
+                    f"--lf {rng.choice([0, 1, 8, 24, 40, 63])} --q {rng.choice([0, 10, 40, 90, 127])} "
+                    f"--log2-parts {rng.randint(0, 3)} --key-interval {rng.choice([0, 2, 4])} "
+                    f"--segmentation {rng.randint(0, 1)} --lf-deltas {rng.randint(0, 1)} "
+                    f"--pct-intra {rng.choice([0, 8, 40, 100])} --pct-split {rng.choice([0, 10, 60])} "
+                    f"--pct-new {rng.choice([10, 30])} --pct-skip {rng.choice([0, 35, 90])} "
+                    f"--pct-bpred {rng.choice([0, 25, 100])} --coef-density {rng.randint(1, 8)} "
+                    f"--pct-empty-block {rng.choice([0, 45, 90])} --golden-period {rng.choice([0, 2, 5])} "
+                    f"--altref-period {rng.choice([0, 3, 4])} --hidden-altref {rng.randint(0, 1)}")
+    for k in range(40):
+        rows = [1, 12, 13, 24, 25][k % 5]
+        h = rows * 16 - rng.choice([0, 0, 5, 15])
+        w = rng.choice([16, 40, 96, 130, 176])
+        parts = 3 if rows == 1 else rng.randint(0, 3)
+        cfgs.append(f"--width {w} --height {h} --frames {rng.randint(3, 6)} --seed {2000 + k} "
+                    f"--version {rng.randint(0, 3)} --filter-type {rng.randint(0, 1)} --sharpness {rng.choice([0, 3, 7])} "
+                    f"--lf {rng.choice([8, 40, 63])} --q {rng.choice([0, 28, 57, 87, 127])} "
+                    f"--log2-parts {parts} --key-interval {rng.choice([0, 3])} "
+                    f"--segmentation {rng.randint(0, 1)} --lf-deltas {rng.randint(0, 1)} "
+                    f"--pct-intra {rng.choice([0, 8, 40, 100])} --pct-split {rng.choice([0, 10, 60])} "
+                    f"--pct-new {rng.choice([10, 30, 60])} --pct-skip {rng.choice([0, 35, 90])} "
+                    f"--pct-bpred {rng.choice([0, 25, 100])} --coef-density {rng.randint(1, 8)} "
+                    f"--pct-empty-block {rng.choice([0, 45, 90])} --golden-period {rng.choice([0, 2, 5])} "
+                    f"--altref-period {rng.choice([0, 3, 4])} --hidden-altref {rng.randint(0, 1)} "
+                    f"--pct-big-coef {rng.choice([0, 5, 30, 100])} --pct-long-mv {rng.choice([0, 10, 40])} "
+                    f"--prob-updates {rng.choice([0, 3, 20])}" + (" --no-skip-flag" if rng.random() < 0.3 else ""))
+    return cfgs
+
+
+# Decode paths of the parity tests: engine settings (read when the engine is created), how the frames are parsed
+# (BatchDecoder's tokens_on_device / device_parse / depth) and VP8R_TOKENS (read at every launch of the token kernel).
+DECODE_PATHS = {
+    "auto": dict(env={}),
+    "swar": dict(env={"VP8R_FILTER": "swar"}),
+    "ldg-one-launch": dict(env={"VP8R_INTER": "ldg", "VP8R_INTRA_ONE_LAUNCH": "1"}),
+    "tokens-swar": dict(env={"VP8R_FILTER": "swar"}, tokens_on_device=True),
+    "modes-swar": dict(env={"VP8R_FILTER": "swar"}, device_parse=True, depth=3),
+    "modes-warp": dict(env={"VP8R_FILTER": "swar"}, device_parse=True, depth=3, tokens="warp"),
+    "modes-lanes": dict(env={"VP8R_FILTER": "swar"}, device_parse=True, depth=3, tokens="lanes"),
+    "half-device": dict(env={}, device_parse=0.5),
+}
+
+
+class Engines:
+    """One engine per set of engine settings, created on first use (the settings are environment variables the
+    engine reads when it is created)."""
+
+    def __init__(self):
+        self._by_env = {}
+
+    def get(self, env):
+        import vp8_b200
+        key = tuple(sorted(env.items()))
+        if key not in self._by_env:
+            names = ("VP8R_FILTER", "VP8R_INTER", "VP8R_INTRA_ONE_LAUNCH", "VP8R_FILTER_SWAR_MIN")
+            old = {k: os.environ.get(k) for k in names}
+            for k in names:
+                os.environ.pop(k, None)
+            os.environ.update(env)
+            try:
+                self._by_env[key] = vp8_b200.Engine(0)
+            finally:
+                for k, v in old.items():
+                    if v is None:
+                        os.environ.pop(k, None)
+                    else:
+                        os.environ[k] = v
+        return self._by_env[key]
+
+    def close(self):
+        for e in self._by_env.values():
+            e.close()
+        self._by_env.clear()
+
+
+def oracle_frames(payloads):
+    """Every frame (shown or not) of one stream through host parser -> oracle: [(I420 bytes, width, height)]."""
+    import vp8_b200
+    ps, orc = vp8_b200.Parser(), Oracle()
+    out = []
+    for p in payloads:
+        fr = ps.parse(p)
+        img = orc.decode(fr)
+        d = fr.desc().hdr
+        out.append((img, d.width, d.height))
+        fr.close()
+    orc.close()
+    ps.close()
+    return out
+
+
+def oracle_checksums(lib, payloads):
+    return [lib.vp8r_checksum_i420(img, w, h) for img, w, h in oracle_frames(payloads)]
+
+
+def first_difference(got, want, w, h):
+    """(plane, x, y) of the first differing byte of two I420 pictures, or None."""
+    if got == want:
+        return None
+    cw, ch = (w + 1) // 2, (h + 1) // 2
+    planes = [("Y", 0, w, h), ("U", w * h, cw, ch), ("V", w * h + cw * ch, cw, ch)]
+    for i in range(min(len(got), len(want))):
+        if got[i] != want[i]:
+            for name, at, pw, ph in reversed(planes):
+                if i >= at:
+                    return name, (i - at) % pw, (i - at) // pw
+    return "size", len(got), len(want)
+
+
+def decode_on_path(engine, payloads, want, path, names, last_frames=None):
+    """Decodes the streams `payloads` as one lock-step batch on decode path `path` (a DECODE_PATHS entry) and compares
+    every frame's device checksum with `want` (oracle checksums per stream) and, given `last_frames`, each stream's
+    last frame byte for byte with last_frames[i].  Returns a list of mismatch descriptions
+    naming the stream, the frame and the plane and (x, y) of the first differing sample."""
+    import vp8_b200
+    tokens = path.get("tokens")
+    old = os.environ.get("VP8R_TOKENS")
+    if tokens:
+        os.environ["VP8R_TOKENS"] = tokens
+    else:
+        os.environ.pop("VP8R_TOKENS", None)
+    bad = []
+    try:
+        dec = vp8_b200.BatchDecoder(engine, len(payloads), pinned=True, tokens_on_device=path.get("tokens_on_device", False),
+                                    device_parse=path.get("device_parse", False), depth=path.get("depth", 2))
+
+        def on_step(t, live, frames):
+            sums = engine.checksum_batch([dec.streams[i] for i in live])
+            for i, s in zip(live, sums):
+                if s != want[i][t]:
+                    where = ""
+                    if len(bad) < 4:  # read the first few back and say where they differ
+                        img, w, h = oracle_frames(payloads[i][:t + 1])[t]
+                        where = f", first difference (plane, x, y) {first_difference(dec.streams[i].read_frame(), img, w, h)}"
+                    bad.append(f"{names[i]}: frame {t}{where}")
+
+        dec.decode(payloads, on_step=on_step)
+        for i, img in enumerate(last_frames or []):
+            if dec.streams[i].read_frame() != img:
+                bad.append(f"{names[i]}: last frame differs byte for byte")
+        dec.close()
+    finally:
+        if old is None:
+            os.environ.pop("VP8R_TOKENS", None)
+        else:
+            os.environ["VP8R_TOKENS"] = old
+    return bad

@@ -273,53 +273,47 @@ def test_many_streams_lockstep_checksums(engine_forms):
     assert got == want
 
 
-def test_randomised_streams_against_oracle(engine_forms):
-    """60 small streams with randomised generator settings (all four bitstream versions, both loop
-    filters, every sharpness, 1-8 partitions, odd sizes, dense SPLIT / intra / B_PRED mixes, GOP
-    lengths) decoded as one lock-step batch; every frame of every stream must equal the oracle's
-    picture (device checksum vs host checksum of the oracle output)."""
-    engine = engine_forms
-    import random
+@pytest.fixture(scope="module")
+def path_engines(built):
+    e = helpers.Engines()
+    yield e
+    e.close()
+
+
+@pytest.fixture(scope="module")
+def randomised_streams(built):
+    """The streams of helpers.randomised_configs() and the oracle's checksum of each of their frames."""
     import vp8_b200
-    rng = random.Random(20261018)
-    cfgs = []
-    for k in range(60):
-        w, h = rng.choice([(16, 16), (17, 33), (48, 64), (96, 80), (130, 98), (176, 144), (250, 120), (320, 16)])
-        cfgs.append(f"--width {w} --height {h} --frames {rng.randint(3, 9)} --seed {1000 + k} "
-                    f"--version {rng.randint(0, 3)} --filter-type {rng.randint(0, 1)} --sharpness {rng.randint(0, 7)} "
-                    f"--lf {rng.choice([0, 1, 8, 24, 40, 63])} --q {rng.choice([0, 10, 40, 90, 127])} "
-                    f"--log2-parts {rng.randint(0, 3)} --key-interval {rng.choice([0, 2, 4])} "
-                    f"--segmentation {rng.randint(0, 1)} --lf-deltas {rng.randint(0, 1)} "
-                    f"--pct-intra {rng.choice([0, 8, 40, 100])} --pct-split {rng.choice([0, 10, 60])} "
-                    f"--pct-new {rng.choice([10, 30])} --pct-skip {rng.choice([0, 35, 90])} "
-                    f"--pct-bpred {rng.choice([0, 25, 100])} --coef-density {rng.randint(1, 8)} "
-                    f"--pct-empty-block {rng.choice([0, 45, 90])} --golden-period {rng.choice([0, 2, 5])} "
-                    f"--altref-period {rng.choice([0, 3, 4])} --hidden-altref {rng.randint(0, 1)}")
+    cfgs = helpers.randomised_configs()
+    from vp8_b200 import _capi
     payloads = [vp8_b200.read_ivf(helpers.synth_stream(c))[1] for c in cfgs]
-    lib = engine._lib
-    want = []
-    for pl in payloads:
-        ps, orc = vp8_b200.Parser(), helpers.Oracle()
-        sums = []
-        for p in pl:
-            fr = ps.parse(p)
-            img = orc.decode(fr)
-            d = fr.desc().hdr
-            sums.append(lib.vp8r_checksum_i420(img, d.width, d.height))
-            fr.close()
-        orc.close()
-        want.append(sums)
-    dec = vp8_b200.BatchDecoder(engine, len(cfgs), pinned=True)
-    got = [[] for _ in cfgs]
+    return cfgs, payloads, [helpers.oracle_checksums(_capi.load(), p) for p in payloads]
 
-    def on_step(t, live, frames):
-        for i, s in zip(live, engine.checksum_batch([dec.streams[i] for i in live])):
-            got[i].append(s)
 
-    dec.decode(payloads, on_step=on_step)
-    dec.close()
-    bad = [cfgs[i] for i in range(len(cfgs)) if got[i] != want[i]]
-    assert not bad, bad[:3]
+DEVICE_PATHS = [k for k, v in helpers.DECODE_PATHS.items() if v.get("tokens_on_device") or v.get("device_parse")]
+
+
+@pytest.mark.parametrize("path", list(helpers.DECODE_PATHS) + [p + "-by-parts" for p in DEVICE_PATHS])
+def test_randomised_streams_against_oracle(path_engines, randomised_streams, path):
+    """100 small streams with randomised generator settings (helpers.randomised_configs: all four bitstream versions,
+    both loop filters, every sharpness, 1-8 partitions, odd sizes, dense SPLIT / intra / B_PRED mixes, GOP lengths,
+    DCT_CAT6 magnitudes, vectors far beyond the frame, probability updates, no skip flag, 1 to 25 macroblock rows)
+    decoded as one lock-step batch on each decode path; every frame of every stream must equal the oracle's picture
+    (device checksum against the checksum of the oracle's output).  The token kernel's instance follows the largest
+    partition count of the batch, so the "-by-parts" rows decode the set again as four batches of one partition
+    count each."""
+    cfgs, payloads, want = randomised_streams
+    by_parts = path.endswith("-by-parts")
+    row = helpers.DECODE_PATHS[path[:-len("-by-parts")] if by_parts else path]
+    engine = path_engines.get(row["env"])
+    groups = [list(range(len(cfgs)))]
+    if by_parts:
+        groups = [[i for i, c in enumerate(cfgs) if f"--log2-parts {lp} " in c] for lp in range(4)]
+        assert sorted(i for g in groups for i in g) == list(range(len(cfgs)))
+    bad = []
+    for g in groups:
+        bad += helpers.decode_on_path(engine, [payloads[i] for i in g], [want[i] for i in g], row, [cfgs[i] for i in g])
+    assert not bad, f"{len(bad)} frames differ: {bad[:4]}"
 
 
 def test_packed_readback_equals_pitched_readback(engine_forms):

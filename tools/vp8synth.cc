@@ -6,8 +6,8 @@
 // It is an OPEN-LOOP synthesiser, not a video encoder: every decision (modes, motion vectors,
 // coefficients, reference updates) is drawn from std::mt19937 (seed 7122 by default, the seed the
 // reference's unit tests use, test/dct_test.h:19) with tunable statistics, and written with the
-// default entropy tables.  What makes a stream a valid test input is that the unmodified reference
-// decoder decodes it; its output is then the golden (tests/golden/synthetic/*.md5).
+// default entropy tables (or, with --prob-updates, with the tables its own header updates).  What
+// makes a stream a valid test input is that the unmodified reference decoder decodes it; its output is then the golden (tests/golden/synthetic/*.md5).
 //
 // Stand-alone on purpose: links neither the product parser nor anything under oracle/.
 #include <algorithm>
@@ -61,6 +61,24 @@ const uint8_t kCat6[] = {254, 254, 243, 230, 196, 177, 153, 140, 133, 130, 129, 
 const uint8_t *const kCatProbs[6] = {kCat1, kCat2, kCat3, kCat4, kCat5, kCat6};
 const int kCatBase[7] = {5, 7, 11, 19, 35, 67, 2115};
 const int kCatBits[6] = {1, 2, 3, 4, 5, 11};
+// Quantiser lookup tables (RFC 6386 section 14.1): the writer derives the above / left token contexts from the
+// dequantised values, as the decoder does.
+const uint8_t kDcQ[128] = {
+    4,   5,   6,   7,   8,   9,   10,  10,  11,  12,  13,  14,  15,  16,  17,  17,  18,  19,  20,
+    20,  21,  21,  22,  22,  23,  23,  24,  25,  25,  26,  27,  28,  29,  30,  31,  32,  33,  34,
+    35,  36,  37,  37,  38,  39,  40,  41,  42,  43,  44,  45,  46,  46,  47,  48,  49,  50,  51,
+    52,  53,  54,  55,  56,  57,  58,  59,  60,  61,  62,  63,  64,  65,  66,  67,  68,  69,  70,
+    71,  72,  73,  74,  75,  76,  76,  77,  78,  79,  80,  81,  82,  83,  84,  85,  86,  87,  88,
+    89,  91,  93,  95,  96,  98,  100, 101, 102, 104, 106, 108, 110, 112, 114, 116, 118, 122, 124,
+    126, 128, 130, 132, 134, 136, 138, 140, 143, 145, 148, 151, 154, 157};
+const uint16_t kAcQ[128] = {
+    4,   5,   6,   7,   8,   9,   10,  11,  12,  13,  14,  15,  16,  17,  18,  19,  20,  21,  22,
+    23,  24,  25,  26,  27,  28,  29,  30,  31,  32,  33,  34,  35,  36,  37,  38,  39,  40,  41,
+    42,  43,  44,  45,  46,  47,  48,  49,  50,  51,  52,  53,  54,  55,  56,  57,  58,  60,  62,
+    64,  66,  68,  70,  72,  74,  76,  78,  80,  82,  84,  86,  88,  90,  92,  94,  96,  98,  100,
+    102, 104, 106, 108, 110, 112, 114, 116, 119, 122, 125, 128, 131, 134, 137, 140, 143, 146, 149,
+    152, 155, 158, 161, 164, 167, 170, 173, 177, 181, 185, 189, 193, 197, 201, 205, 209, 213, 217,
+    221, 225, 229, 234, 239, 245, 249, 254, 259, 264, 269, 274, 279, 284};
 
 struct Mv {
   int r = 0, c = 0;
@@ -77,6 +95,12 @@ struct Options {
   int pct_intra = 8, pct_split = 10, pct_new = 30, pct_skip = 35, pct_bpred = 25;
   int coef_density = 6;  // expected non-zero coefficients per coded block (x2)
   int pct_empty_block = 45;  // blocks without any coefficient inside a non-skipped macroblock
+  // Syntax extremes, all off by default (an option at 0 draws nothing from the RNG, so the streams of
+  // the manifest stay byte-identical):
+  int pct_big_coef = 0;   // share of the non-zero coefficients made DCT_CAT6 magnitudes (67..2114, 512*k)
+  int pct_long_mv = 0;    // share of the NEW deltas aimed 64 px beyond a frame corner
+  int prob_updates = 0;   // per-probability update chance (coefficients, MVs), mode updates, non-refreshed frames
+  int no_skip_flag = 0;   // mb_no_skip_coeff = 0: every macroblock carries its tokens
   std::string out = "synth.ivf";
 };
 
@@ -90,6 +114,7 @@ class Synth {
   std::vector<uint8_t> Frame(int index) {
     const bool key = index == 0 || (opt_.key_interval > 0 && index % opt_.key_interval == 0);
     key_ = key;
+    if (key) probs_ = Probs();
     BoolWriter hdr;
     const int n_parts = 1 << opt_.log2_parts;
     std::vector<BoolWriter> parts(n_parts);
@@ -162,7 +187,17 @@ class Synth {
       hdr.Lit(1, deltas[i] != 0);
       if (deltas[i]) hdr.SignedLit(4, deltas[i]);
     }
-    bool show = true;
+    for (int s = 0; s < 4; ++s) {  // dequantisation factors per segment: Y1 DC, AC, Y2 DC, AC, UV DC, AC
+      const int q = Clamp(seg ? (seg_abs_ ? seg_q_[s] : opt_.q + seg_q_[s]) : opt_.q, 0, 127);
+      auto qi = [&](int d) { return Clamp(q + d, 0, 127); };
+      dq_[s][0] = kDcQ[qi(deltas[0])];
+      dq_[s][1] = kAcQ[q];
+      dq_[s][2] = kDcQ[qi(deltas[1])] * 2;
+      dq_[s][3] = std::max(8, int(kAcQ[qi(deltas[2])]) * 155 / 100);
+      dq_[s][4] = std::min(132, int(kDcQ[qi(deltas[3])]));
+      dq_[s][5] = kAcQ[qi(deltas[4])];
+    }
+    bool show = true, refresh_entropy = true;
     bool sign_bias[4] = {false, false, false, false};
     if (key) {
       hdr.Lit(1, 1);  // refresh_entropy_probs
@@ -185,13 +220,23 @@ class Synth {
       if (!refresh_a) hdr.Lit(2, uint32_t(copy_a));
       hdr.Lit(1, sign_bias[2]);
       hdr.Lit(1, sign_bias[3]);
-      hdr.Lit(1, 1);  // refresh_entropy_probs
+      refresh_entropy = !(opt_.prob_updates && Pct(opt_.prob_updates));
+      hdr.Lit(1, refresh_entropy);
       hdr.Lit(1, refresh_last);
     }
-    for (int i = 0; i < 1056; ++i) hdr.Put(kCoefUpdate[i], 0);  // keep the default token probabilities
+    // The updates of a frame that does not refresh the entropy context last for that frame only.
+    const Probs saved = probs_;
+    for (int i = 0; i < 1056; ++i) {
+      const bool upd = opt_.prob_updates && Pct(opt_.prob_updates);
+      hdr.Put(kCoefUpdate[i], upd);
+      if (upd) {
+        probs_.coef[i] = uint8_t(Range(1, 255));
+        hdr.Lit(8, probs_.coef[i]);
+      }
+    }
     const int prob_skip = 255 - (opt_.pct_skip * 255) / 100;
-    hdr.Lit(1, 1);  // mb_no_skip_coeff
-    hdr.Lit(8, uint32_t(Clamp(prob_skip, 1, 255)));
+    hdr.Lit(1, !opt_.no_skip_flag);  // mb_no_skip_coeff
+    if (!opt_.no_skip_flag) hdr.Lit(8, uint32_t(Clamp(prob_skip, 1, 255)));
     // prob_intra = P(bit == 0) = P(macroblock is intra), out of 256.
     const int prob_intra = Clamp((opt_.pct_intra * 256) / 100, 1, 255);
     const int prob_last = 200, prob_gf = 128;
@@ -199,9 +244,22 @@ class Synth {
       hdr.Lit(8, uint32_t(prob_intra));
       hdr.Lit(8, prob_last);
       hdr.Lit(8, prob_gf);
-      hdr.Lit(1, 0);
-      hdr.Lit(1, 0);
-      for (int i = 0; i < 38; ++i) hdr.Put(kMvUpdate[i], 0);
+      const bool upd_y = opt_.prob_updates && Pct(50), upd_uv = opt_.prob_updates && Pct(50);
+      hdr.Lit(1, upd_y);
+      if (upd_y)
+        for (int i = 0; i < 4; ++i) hdr.Lit(8, probs_.ymode[i] = uint8_t(Range(1, 255)));
+      hdr.Lit(1, upd_uv);
+      if (upd_uv)
+        for (int i = 0; i < 3; ++i) hdr.Lit(8, probs_.uvmode[i] = uint8_t(Range(1, 255)));
+      for (int i = 0; i < 38; ++i) {
+        const bool upd = opt_.prob_updates && Pct(opt_.prob_updates);
+        hdr.Put(kMvUpdate[i], upd);
+        if (upd) {
+          const int v = Range(0, 127);
+          hdr.Lit(7, uint32_t(v));
+          probs_.mv[i] = uint8_t(v ? v << 1 : 1);
+        }
+      }
     }
 
     // ---- macroblocks ----
@@ -214,6 +272,10 @@ class Synth {
     nz_ay2_.assign(size_t(cols_), 0);
     // a smooth global motion for this frame plus per-macroblock jitter, quarter-pel units
     const int pan_r = Range(-12, 12), pan_c = Range(-16, 16);
+    if (opt_.pct_long_mv) {  // the point the long deltas aim at: 64 px beyond one corner of the frame
+      far_r_ = Pct(50) ? -64 : rows_ * 16 + 64;
+      far_c_ = Pct(50) ? -64 : cols_ * 16 + 64;
+    }
 
     for (int r = 0; r < rows_; ++r) {
       uint8_t left_b[4] = {0, 0, 0, 0};
@@ -226,8 +288,8 @@ class Synth {
           seg_map_[idx] = uint8_t(s);
           hdr.Tree(kTreeSegment, 6, seg_tree_probs_, s);
         }
-        const bool skip = Pct(opt_.pct_skip);
-        hdr.Put(Clamp(prob_skip, 1, 255), skip);
+        const bool skip = !opt_.no_skip_flag && Pct(opt_.pct_skip);
+        if (!opt_.no_skip_flag) hdr.Put(Clamp(prob_skip, 1, 255), skip);
         bool inter = false;
         if (!key) {
           inter = !Pct(opt_.pct_intra);
@@ -243,7 +305,7 @@ class Synth {
         } else {
           int ymode = Pct(opt_.pct_bpred) ? B_PRED : int(rng_() % 4);
           if (key) hdr.Tree(kTreeYModeKey, 8, kProbYModeKey, ymode);
-          else hdr.Tree(kTreeYMode, 8, kProbYMode, ymode);
+          else hdr.Tree(kTreeYMode, 8, probs_.ymode, ymode);
           if (ymode == B_PRED) {
             has_y2 = false;
             for (int i = 0; i < 4; ++i)
@@ -261,17 +323,21 @@ class Synth {
             for (int i = 0; i < 4; ++i) above_b_[c * 4 + i] = left_b[i] = implied[ymode];
           }
           int uvmode = int(rng_() % 4);
-          hdr.Tree(kTreeUvMode, 6, key ? kProbUvModeKey : kProbUvMode, uvmode);
+          hdr.Tree(kTreeUvMode, 6, key ? kProbUvModeKey : probs_.uvmode, uvmode);
         }
 
         // ---- residual tokens ----
         if (!skip) {
-          uint32_t nz = 0;  // bit 0: Y2, 1..16: Y, 17..20: U, 21..24: V
+          // Inside the macroblock the contexts follow the coded tokens; the ones handed to the next macroblocks
+          // follow the dequantised int16 values (a product that wraps to 0 counts as zero).
+          uint32_t nz = 0, dnz = 0;  // bit 0: Y2, 1..16: Y, 17..20: U, 21..24: V
+          const int *dq = dq_[seg ? seg_map_[idx] : 0];
           if (has_y2) {
             int coefs[16];
             MakeCoefs(coefs, 0, /*dc_bias=*/true, 3);
             if (WriteBlock(tok, 1, nz_ay2_[c] + nz_ly2, 0, coefs)) nz |= 1;
-            nz_ay2_[c] = nz_ly2 = uint8_t(nz & 1);
+            if (DequantNz(coefs, dq[2], dq[3])) dnz |= 1;
+            nz_ay2_[c] = nz_ly2 = uint8_t(dnz & 1);
           }
           for (int b = 0; b < 16; ++b) {
             int i = b >> 2, j = b & 3;
@@ -280,6 +346,7 @@ class Synth {
             int coefs[16];
             MakeCoefs(coefs, has_y2 ? 1 : 0, !has_y2, 2);
             if (WriteBlock(tok, has_y2 ? 0 : 3, a + l, has_y2 ? 1 : 0, coefs)) nz |= 2u << b;
+            if (DequantNz(coefs, dq[0], dq[1])) dnz |= 2u << b;
           }
           for (int pl = 0; pl < 2; ++pl) {
             uint8_t *na = pl ? &nz_av_[c * 2] : &nz_au_[c * 2];
@@ -292,17 +359,18 @@ class Synth {
               int coefs[16];
               MakeCoefs(coefs, 0, true, 2);
               if (WriteBlock(tok, 2, a + l, 0, coefs)) nz |= 1u << (base + b);
+              if (DequantNz(coefs, dq[4], dq[5])) dnz |= 1u << (base + b);
             }
           }
-          for (int j = 0; j < 4; ++j) nz_ay_[c * 4 + j] = uint8_t((nz >> (13 + j)) & 1);
-          for (int i = 0; i < 4; ++i) nz_ly[i] = uint8_t((nz >> (4 + i * 4)) & 1);
+          for (int j = 0; j < 4; ++j) nz_ay_[c * 4 + j] = uint8_t((dnz >> (13 + j)) & 1);
+          for (int i = 0; i < 4; ++i) nz_ly[i] = uint8_t((dnz >> (4 + i * 4)) & 1);
           for (int j = 0; j < 2; ++j) {
-            nz_au_[c * 2 + j] = uint8_t((nz >> (19 + j)) & 1);
-            nz_av_[c * 2 + j] = uint8_t((nz >> (23 + j)) & 1);
+            nz_au_[c * 2 + j] = uint8_t((dnz >> (19 + j)) & 1);
+            nz_av_[c * 2 + j] = uint8_t((dnz >> (23 + j)) & 1);
           }
           for (int i = 0; i < 2; ++i) {
-            nz_lu[i] = uint8_t((nz >> (18 + i * 2)) & 1);
-            nz_lv[i] = uint8_t((nz >> (22 + i * 2)) & 1);
+            nz_lu[i] = uint8_t((dnz >> (18 + i * 2)) & 1);
+            nz_lv[i] = uint8_t((dnz >> (22 + i * 2)) & 1);
           }
         } else {
           if (has_y2) nz_ay2_[c] = nz_ly2 = 0;
@@ -316,6 +384,7 @@ class Synth {
     std::vector<uint8_t> first = hdr.Finish();
     std::vector<std::vector<uint8_t>> pb;
     for (auto &p : parts) pb.push_back(p.Finish());
+    if (!refresh_entropy) probs_ = saved;
     std::vector<uint8_t> out;
     uint32_t tag = (key ? 0u : 1u) | (uint32_t(opt_.version) << 1) | (uint32_t(show) << 4) | (uint32_t(first.size()) << 5);
     out.push_back(uint8_t(tag));
@@ -341,6 +410,15 @@ class Synth {
   }
 
  private:
+  struct Probs {  // the entropy context: token, motion-vector and inter-frame 16x16 / chroma mode probabilities
+    uint8_t coef[1056], mv[38], ymode[4], uvmode[3];
+    Probs() {
+      std::memcpy(coef, kCoefDefault, sizeof(coef));
+      std::memcpy(mv, kMvDefault, sizeof(mv));
+      std::memcpy(ymode, kProbYMode, sizeof(ymode));
+      std::memcpy(uvmode, kProbUvMode, sizeof(uvmode));
+    }
+  };
   struct MbCtx {
     bool inter = false;
     int ref = 0, mode = 0;
@@ -351,7 +429,9 @@ class Synth {
   bool Pct(int p) { return int(rng_() % 100) < p; }
   int Range(int lo, int hi) { return lo + int(rng_() % uint32_t(hi - lo + 1)); }
 
-  // Sparse, low-frequency-weighted coefficients in zig-zag order; no int16 wrap after dequant.
+  // Sparse, low-frequency-weighted coefficients in zig-zag order; no int16 wrap after dequant unless
+  // --pct-big-coef asks for DCT_CAT6 magnitudes: half of them over the whole 11-bit range, half multiples
+  // of 512, whose product with a factor that is a multiple of 128 (or 1024 with 64, 2048 with 32) wraps to 0.
   void MakeCoefs(int *z, int first, bool allow_dc, int amp) {
     std::memset(z, 0, sizeof(int) * 16);
     if (Pct(opt_.pct_empty_block)) return;  // uncoded block
@@ -363,8 +443,16 @@ class Synth {
       int mag = 1 + int(rng_() % uint32_t(amp));
       if (Pct(3)) mag += int(rng_() % 40);  // occasionally exercise the DCT_CAT tokens
       if (Pct(1)) mag = 67 + int(rng_() % 200);
+      if (opt_.pct_big_coef && Pct(opt_.pct_big_coef)) mag = Pct(50) ? Range(67, 2114) : 512 * Range(1, 4);
       z[pos] = Pct(50) ? mag : -mag;
     }
+  }
+
+  // Whether any coefficient of a block is non-zero after dequantisation in int16 (z in zig-zag order, z[0] the DC).
+  static bool DequantNz(const int *z, int dc_f, int ac_f) {
+    for (int n = 0; n < 16; ++n)
+      if (int16_t(z[n] * (n ? ac_f : dc_f)) != 0) return true;
+    return false;
   }
 
   // Writes one block; returns whether any coefficient is non-zero.  No trailing zero tokens.
@@ -372,7 +460,7 @@ class Synth {
     int last = -1;
     for (int n = first; n < 16; ++n)
       if (z[n]) last = n;
-    const uint8_t *base = &kCoefDefault[size_t(type) * 8 * 3 * 11];
+    const uint8_t *base = &probs_.coef[size_t(type) * 8 * 3 * 11];
     auto probs = [&](int n, int cx) { return base + (size_t(kBand[n]) * 3 + cx) * 11; };
     bool prev_zero = false;
     int n = first;
@@ -508,13 +596,17 @@ class Synth {
     for (int i = 0; i < 4; ++i) p[i] = kProbMvRef[cnt[i]][i];
     bw.Tree(kTreeMvRef, 8, p, mode);
 
-    const uint8_t *mvp_r = &kMvDefault[0], *mvp_c = &kMvDefault[19];
+    const uint8_t *mvp_r = &probs_.mv[0], *mvp_c = &probs_.mv[19];
     // A delta that steers the final vector towards the frame's global pan (quarter-pel units).
     auto new_delta = [&](const Mv &base_mv, int *dr, int *dc) {
       int want_r = pan_r + Range(-6, 6), want_c = pan_c + Range(-6, 6);
       if (Pct(3)) {  // occasional long vectors: exercise the border clamps
         want_r += Range(-400, 400);
         want_c += Range(-400, 400);
+      }
+      if (opt_.pct_long_mv && Pct(opt_.pct_long_mv)) {  // at the frame's far point, as far as one delta gets
+        want_r = 4 * (far_r_ - r * 16);
+        want_c = 4 * (far_c_ - c * 16);
       }
       *dr = Clamp(want_r - base_mv.r / 2, -1023, 1023);
       *dc = Clamp(want_c - base_mv.c / 2, -1023, 1023);
@@ -576,8 +668,11 @@ class Synth {
   std::vector<uint8_t> seg_map_;
   bool have_seg_data_ = false;
   int seg_abs_ = 0, seg_q_[4] = {0, 0, 0, 0};
+  int dq_[4][6] = {};
   uint8_t seg_tree_probs_[3] = {128, 128, 128};
   int ref_lf_delta_[4], mode_lf_delta_[4];
+  Probs probs_;
+  int far_r_ = 0, far_c_ = 0;
   std::vector<MbCtx> ctx_;
   std::vector<Mv> sub_mvs_;
   std::vector<uint8_t> above_b_, nz_ay_, nz_au_, nz_av_, nz_ay2_;
@@ -623,6 +718,10 @@ int main(int argc, char **argv) {
     else if (a == "--pct-bpred") o.pct_bpred = std::atoi(next());
     else if (a == "--coef-density") o.coef_density = std::max(1, std::atoi(next()));
     else if (a == "--pct-empty-block") o.pct_empty_block = std::atoi(next());
+    else if (a == "--pct-big-coef") o.pct_big_coef = std::atoi(next());
+    else if (a == "--pct-long-mv") o.pct_long_mv = std::atoi(next());
+    else if (a == "--prob-updates") o.prob_updates = std::atoi(next());
+    else if (a == "--no-skip-flag") o.no_skip_flag = 1;
     else if (a == "--out") o.out = next();
     else {
       std::fprintf(stderr,
@@ -630,7 +729,16 @@ int main(int argc, char **argv) {
                    "       [--sharpness S] [--filter-type 0|1] [--version 0..3] [--log2-parts 0..3] [--segmentation 0|1]\n"
                    "       [--lf-deltas 0|1] [--golden-period N] [--altref-period N] [--hidden-altref 0|1]\n"
                    "       [--pct-intra P] [--pct-split P] [--pct-new P] [--pct-skip P] [--pct-bpred P]\n"
-                   "       [--coef-density N] [--pct-empty-block P] --out file.ivf\n");
+                   "       [--coef-density N] [--pct-empty-block P] [--pct-big-coef P] [--pct-long-mv P]\n"
+                   "       [--prob-updates P] [--no-skip-flag] --out file.ivf\n"
+                   "  --pct-big-coef P   P %% of the non-zero coefficients become DCT_CAT6 magnitudes: half uniform over\n"
+                   "                     67..2114 (all 11 extra bits), half from {512, 1024, 1536, 2048}\n"
+                   "  --pct-long-mv P    P %% of the NEW deltas (macroblock and SPLIT partition) aim 64 px beyond a frame\n"
+                   "                     corner chosen per frame, clamped to +-1023, the range of the long form\n"
+                   "  --prob-updates P   each token and MV probability is updated with chance P %%; inter frames may\n"
+                   "                     update the 16x16 and chroma mode probabilities; P %% of the inter frames\n"
+                   "                     set refresh_entropy_probs = 0\n"
+                   "  --no-skip-flag     mb_no_skip_coeff = 0\n");
       return 2;
     }
   }
