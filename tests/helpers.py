@@ -179,16 +179,13 @@ def randomised_configs():
     return cfgs
 
 
-# Decode paths of the parity tests: engine settings (read when the engine is created), how the frames are parsed
-# (BatchDecoder's tokens_on_device / device_parse / depth) and VP8R_TOKENS (read at every launch of the token kernel).
+# Decode paths of the parity tests: engine settings (read when the engine is created) and how the frames are parsed
+# (BatchDecoder's tokens_on_device / device_parse / depth).
 DECODE_PATHS = {
     "auto": dict(env={}),
     "swar": dict(env={"VP8R_FILTER": "swar"}),
-    "ldg-one-launch": dict(env={"VP8R_INTER": "ldg", "VP8R_INTRA_ONE_LAUNCH": "1"}),
     "tokens-swar": dict(env={"VP8R_FILTER": "swar"}, tokens_on_device=True),
     "modes-swar": dict(env={"VP8R_FILTER": "swar"}, device_parse=True, depth=3),
-    "modes-warp": dict(env={"VP8R_FILTER": "swar"}, device_parse=True, depth=3, tokens="warp"),
-    "modes-lanes": dict(env={"VP8R_FILTER": "swar"}, device_parse=True, depth=3, tokens="lanes"),
     "half-device": dict(env={}, device_parse=0.5),
 }
 
@@ -204,19 +201,16 @@ class Engines:
         import vp8_b200
         key = tuple(sorted(env.items()))
         if key not in self._by_env:
-            names = ("VP8R_FILTER", "VP8R_INTER", "VP8R_INTRA_ONE_LAUNCH", "VP8R_FILTER_SWAR_MIN")
-            old = {k: os.environ.get(k) for k in names}
-            for k in names:
-                os.environ.pop(k, None)
+            old = os.environ.get("VP8R_FILTER")
+            os.environ.pop("VP8R_FILTER", None)
             os.environ.update(env)
             try:
                 self._by_env[key] = vp8_b200.Engine(0)
             finally:
-                for k, v in old.items():
-                    if v is None:
-                        os.environ.pop(k, None)
-                    else:
-                        os.environ[k] = v
+                if old is None:
+                    os.environ.pop("VP8R_FILTER", None)
+                else:
+                    os.environ["VP8R_FILTER"] = old
         return self._by_env[key]
 
     def close(self):
@@ -265,35 +259,23 @@ def decode_on_path(engine, payloads, want, path, names, last_frames=None):
     last frame byte for byte with last_frames[i].  Returns a list of mismatch descriptions
     naming the stream, the frame and the plane and (x, y) of the first differing sample."""
     import vp8_b200
-    tokens = path.get("tokens")
-    old = os.environ.get("VP8R_TOKENS")
-    if tokens:
-        os.environ["VP8R_TOKENS"] = tokens
-    else:
-        os.environ.pop("VP8R_TOKENS", None)
     bad = []
-    try:
-        dec = vp8_b200.BatchDecoder(engine, len(payloads), pinned=True, tokens_on_device=path.get("tokens_on_device", False),
-                                    device_parse=path.get("device_parse", False), depth=path.get("depth", 2))
+    dec = vp8_b200.BatchDecoder(engine, len(payloads), pinned=True, tokens_on_device=path.get("tokens_on_device", False),
+                                device_parse=path.get("device_parse", False), depth=path.get("depth", 2))
 
-        def on_step(t, live, frames):
-            sums = engine.checksum_batch([dec.streams[i] for i in live])
-            for i, s in zip(live, sums):
-                if s != want[i][t]:
-                    where = ""
-                    if len(bad) < 4:  # read the first few back and say where they differ
-                        img, w, h = oracle_frames(payloads[i][:t + 1])[t]
-                        where = f", first difference (plane, x, y) {first_difference(dec.streams[i].read_frame(), img, w, h)}"
-                    bad.append(f"{names[i]}: frame {t}{where}")
+    def on_step(t, live, frames):
+        sums = engine.checksum_batch([dec.streams[i] for i in live])
+        for i, s in zip(live, sums):
+            if s != want[i][t]:
+                where = ""
+                if len(bad) < 4:  # read the first few back and say where they differ
+                    img, w, h = oracle_frames(payloads[i][:t + 1])[t]
+                    where = f", first difference (plane, x, y) {first_difference(dec.streams[i].read_frame(), img, w, h)}"
+                bad.append(f"{names[i]}: frame {t}{where}")
 
-        dec.decode(payloads, on_step=on_step)
-        for i, img in enumerate(last_frames or []):
-            if dec.streams[i].read_frame() != img:
-                bad.append(f"{names[i]}: last frame differs byte for byte")
-        dec.close()
-    finally:
-        if old is None:
-            os.environ.pop("VP8R_TOKENS", None)
-        else:
-            os.environ["VP8R_TOKENS"] = old
+    dec.decode(payloads, on_step=on_step)
+    for i, img in enumerate(last_frames or []):
+        if dec.streams[i].read_frame() != img:
+            bad.append(f"{names[i]}: last frame differs byte for byte")
+    dec.close()
     return bad

@@ -338,14 +338,12 @@ def engines(built):
 
 
 HOST = dict(env={})
-TOKEN_FORMS = [None, "warp", "lanes"]
 
 
 def device_paths(env=None):
-    """Tokens on the device and macroblock headers + tokens on the device, each in the three token-kernel forms."""
+    """Tokens on the device, and macroblock headers + tokens on the device."""
     env = env or {}
-    return ([dict(env=env, tokens_on_device=True, tokens=t) for t in TOKEN_FORMS] +
-            [dict(env=env, device_parse=True, depth=3, tokens=t) for t in TOKEN_FORMS])
+    return [dict(env=env, tokens_on_device=True), dict(env=env, device_parse=True, depth=3)]
 
 
 def check_paths(engines, named_args, paths, check_last=False):
@@ -364,27 +362,26 @@ def check_paths(engines, named_args, paths, check_last=False):
 @pytest.mark.parametrize("parts", [1, 4])
 def test_wrap_to_zero_contexts_on_every_token_path(engines, parts):
     """Blocks that dequantise to zero hand "zero" to their neighbours, and the whole CAT6 range decodes, on the host
-    parse and in every form of the device token decoder."""
+    parse and in the device token decoder."""
     streams = {k: v for k, v in WRAP.items() if k.endswith(f"-p{parts}")}
     check_paths(engines, streams, [HOST] + device_paths())
 
 
 @pytest.mark.gpu
 def test_long_vectors(engines):
-    """Vectors beyond the frame and chroma sums that wrap in int16: TMA and ldg motion compensation, host and device
-    parse; the 4K frames by checksum, the last frame byte for byte."""
+    """Vectors beyond the frame and chroma sums that wrap in int16, host and device parse; the 4K frames by checksum,
+    the last frame byte for byte."""
     streams = {"4k": LONG_4K, **LONG_SMALL}
-    paths = [dict(env=env, **parse) for env in ({}, {"VP8R_INTER": "ldg"}) for parse in ({}, dict(device_parse=True, depth=3))]
+    paths = [HOST, dict(env={}, device_parse=True, depth=3)]
     check_paths(engines, streams, paths, check_last=True)
 
 
 @pytest.mark.gpu
 def test_intra_level_boundary(engines):
-    """47, 48, 49 and 50 intra levels in one batch: per-level launches and one launch on the host-parsed records, the
-    device-built level table against the wavefront fallback on the device-parsed ones."""
+    """47, 48, 49 and 50 intra levels in one batch: per-level launches on the host-parsed records, the device-built
+    level table (IntraLevelsKernel) against the wavefront fallback on the device-parsed ones."""
     streams = {f"{c}-bpred{b}": level_args(c, b) for c in LEVEL_COLS for b in (0, 100)}
-    paths = [HOST, dict(env={"VP8R_INTRA_ONE_LAUNCH": "1"}), dict(env={}, device_parse=True, depth=3),
-             dict(env={"VP8R_INTRA_ONE_LAUNCH": "1"}, device_parse=True, depth=3)]
+    paths = [HOST, dict(env={}, device_parse=True, depth=3)]
     check_paths(engines, streams, paths)
 
 
@@ -403,7 +400,7 @@ def test_filter_bands_and_groups(engines, rows):
 @pytest.mark.gpu
 def test_probability_updates_and_no_skip_flag_on_device_parse(engines):
     """Updated token, MV and mode probabilities (and frames that drop their updates) and frames without the skip flag,
-    decoded with the macroblock headers and tokens on the device in every token-kernel form, and on the host."""
+    decoded with the macroblock headers and tokens on the device, and on the host."""
     for args in PROBS.values():
         assert all(prob_stats(args)[:3])
     check_paths(engines, {f"probs-{k}": v for k, v in PROBS.items()}, [HOST] + device_paths({"VP8R_FILTER": "swar"}))

@@ -450,48 +450,6 @@ def test_device_tokens_batched_and_truncated(engine):
     st.close()
 
 
-@pytest.mark.parametrize("form", ["warp", "lanes"])
-def test_token_kernel_forms_agree(engine, monkeypatch, form):
-    """The other two forms of the token kernel (VP8R_TOKENS=warp: 32 partitions per warp as a lock-step automaton;
-    lanes: a frame's partitions as diverging lanes of one warp) against the default one-warp-per-partition form:
-    ragged batch (three sizes, 1/2/4/8 partitions, so lanes of one warp carry frames of different geometry),
-    device checksums of every time step, with and without the macroblock headers on the device; then a truncated
-    partition has to be flagged."""
-    import vp8_b200
-    from vp8_b200._capi import Vp8rError
-    sizes = ["--width 320 --height 192", "--width 176 --height 144", "--width 640 --height 368"]
-    ivfs = [helpers.synth_stream(f"{sizes[k % 3]} --frames 5 --seed {170 + k} --log2-parts {k % 4}") for k in range(13)]
-    payloads = [vp8_b200.read_ivf(d)[1] for d in ivfs]
-
-    def run(par):
-        dec = vp8_b200.BatchDecoder(engine, len(ivfs), pinned=True, tokens_on_device=not par, device_parse=par)
-        per_step = []
-        dec.decode(payloads, on_step=lambda t, live, frames: per_step.append(engine.checksum_batch([dec.streams[i] for i in live])))
-        dec.close()
-        return per_step
-
-    monkeypatch.delenv("VP8R_TOKENS", raising=False)
-    want = [run(False), run(True)]
-    assert want[0] == want[1]
-    monkeypatch.setenv("VP8R_TOKENS", form)
-    assert run(False) == want[0]
-    assert run(True) == want[0]
-    ps = vp8_b200.Parser()
-    ps.set_defer_tokens(True)
-    st = engine.open_stream()
-    key = payloads[0][0]
-    first_size = (key[0] | key[1] << 8 | key[2] << 16) >> 5
-    keep = 10 + first_size + (len(key) - 10 - first_size) // 3
-    fr = ps.parse(key[:keep], pinned=True)
-    engine.reconstruct_batch([st], [fr])
-    with pytest.raises(Vp8rError) as ei:
-        engine.sync()
-    assert ei.value.code == 4
-    engine.sync()
-    fr.close()
-    st.close()
-
-
 def test_passes_without_draining_and_resident_replays(engine):
     """decode(drain=False) hands the pipeline over to the next pass (new streams after reset, same ring): the frames
     that arrive in the pinned ring are those of a drained pass.  And frames kept resident with a deferred parse

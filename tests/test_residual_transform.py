@@ -1,6 +1,6 @@
 """The residual transform of the reconstruction kernels on its edges: the DC-only shortcut for Y blocks fed by
-Y2 alone, and macroblocks with more coded blocks than one pass of the warp transforms (8), decoded with both
-forms of the inter kernel and compared with the oracle frame by frame."""
+Y2 alone, and macroblocks with more coded blocks than one pass of the warp transforms (8), decoded and compared
+with the oracle frame by frame."""
 import ctypes as C
 
 import numpy as np
@@ -60,15 +60,9 @@ def test_dense_streams_need_a_second_pass(built, args):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("form", ["tma", "ldg"])
-def test_dense_residuals_match_oracle(built, monkeypatch, form):
-    """Every frame of the dense streams, decoded with reference windows by TMA and by the lanes' loads
-    (VP8R_INTER=ldg, read when the engine is created), equals the oracle's."""
+def test_dense_residuals_match_oracle(built):
+    """Every frame of the dense streams equals the oracle's."""
     import vp8_b200
-    if form == "ldg":
-        monkeypatch.setenv("VP8R_INTER", "ldg")
-    else:
-        monkeypatch.delenv("VP8R_INTER", raising=False)
     eng = vp8_b200.Engine(0)
     try:
         for args in DENSE:

@@ -19,33 +19,10 @@
 //
 // Measured (B200, 512 1080p frames per launch): 2.61 ms against 4.11 ms of the scalar kernel; ~1350 warp
 // instructions per step of 8 macroblocks (luma) + ~750 (chroma) = ~260 per macroblock against 796.
-#include <cstdio>
-#include <algorithm>
-#include <cstdlib>
-
 #include "lf_swar.h"
 #include "recon_kernels.h"
 
 namespace vp8r {
-
-#ifdef VP8R_SWAR_PROF
-// Development aid (build with -DVP8R_SWAR_PROF): cycles per phase of the macroblock step, summed over all
-// warps by lane 0; read back and printed by SwarProfDump().
-__device__ unsigned long long g_swar_prof[16];
-__device__ unsigned long long g_swar_rows[2][128][4];  // group 0: [kind][row][start, end] in ns (globaltimer)
-__device__ __forceinline__ unsigned long long GlobalTimerNs() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
-#define PROF_T(var) const long long var = clock64()
-#define PROF_ADD(slot, a, b) prof_acc[(slot) & 7] += (b) - (a)
-#define PROF_COUNT(slot) prof_acc[7] += 1
-#else
-#define PROF_T(var)
-#define PROF_ADD(slot, a, b)
-#define PROF_COUNT(slot)
-#endif
 
 namespace {
 
@@ -114,19 +91,15 @@ __device__ __forceinline__ int LoadFlagAcquireSwar(const int *p) {
   return v;
 }
 
-// One band (rows r0..r1-1 of the group's frames) of one plane kind.  NB = 4x4 blocks per macroblock side:
-// 4 for luma, 2 for chroma.
-struct SwarTune {
-  int sleep_base, sleep_slope;  // ns: a waiting row sleeps base + slope * (macroblocks still missing - 1)
-  int relaxed_poll;             // poll the band flag with a relaxed load, fence once it is reached
-  int band_stride;              // steps between device-scope publications of a band's last row
-};
-
-__device__ __forceinline__ int LoadFlagRelaxedSwar(const int *p) {
-  int v;
-  asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
+// A waiting row sleeps kSwarSleepBase + kSwarSleepSlope * (macroblocks still missing - 1) ns, at most kSwarSleepMax;
+// the last row of a band publishes its progress device-wide at every kSwarBandStride-th flush.
+constexpr int kSwarSleepBase = 400, kSwarSleepSlope = 1500, kSwarSleepMax = 40000;
+constexpr int kSwarBandStride = 4;
+// CTA shape: kSwarWarps warps = macroblock rows per band, one CTA per SM.  Measured at 512 1080p frames per launch
+// (profiles/r2_filter_swar.md): 12 x 1 = 2.61 ms, 10 x 1 = 2.67, 8 x 1 = 2.72, 6 x 2 = 2.77, 16 x 1 = 3.66,
+// 17 x 1 = 3.99, 4 x 5 = 4.19 (the scalar kernel: 4.11).  More resident warps lose: 12.5 KB of shared memory
+// per warp leave little L1 for the row loads (each 32-byte sector is read in two consecutive steps).
+constexpr int kSwarWarps = 12;
 
 // Output staging.  Finished pixel rows do not go to global memory word by word (a warp-wide 32-bit store of
 // this kernel touches 8..32 different sectors, and every hand-over fence has to wait for all of them): the
@@ -153,10 +126,12 @@ constexpr int kSwarRingBytes = 8 * SwarRing<4>::kSlotBytes;  // per warp; the lu
 constexpr int kSwarTileBytes = 8 * 20 * 16;                  // per warp; exchange tiles (luma: 8 slots x 4 regions x 5 chunks)
 constexpr int kSwarPtrBytes = 8 * 2 * 8;                     // per warp; plane pointers of the 8 slots
 
-template <int NB, int kSwarWarps>
+// One band (rows r0..r1-1 of the group's frames) of one plane kind.  NB = 4x4 blocks per macroblock side:
+// 4 for luma, 2 for chroma.
+template <int NB>
 __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ jobs, const FilterGroup &grp, int band, int n_bands,
                                                int *gflag, volatile int *lprog, uint4 *tiles, unsigned char *rings,
-                                               unsigned long long *ptrs, const SwarTune tune) {
+                                               unsigned long long *ptrs) {
   using Ring = SwarRing<NB>;
   constexpr int kN = 4 * NB;            // macroblock size in this plane
   constexpr int kRegion = NB + 1;       // 16-byte chunks between the regions of a slot (one pad chunk)
@@ -209,9 +184,10 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
     a_half[j] = NB == 4 ? (rem & 1) : 0;
   }
 
+  const int publish_row = band + 1 < n_bands ? r1 - 1 : -1;  // the band's last row, read by the next band (none after the last)
   for (int lr = warp; lr < r1 - r0; lr += kSwarWarps) {
     const int r = r0 + lr;
-    const bool last_of_band = (r == r1 - 1) && (band + 1 < n_bands);
+    const bool last_of_band = r == publish_row;
     const bool has_above = r > 0;
     const bool above_local = lr > 0;
     const uint8_t *rowp = plane + (ptrdiff_t)(r * kN + 4 * sub) * pitch;         // row group: first of my four rows, x = 0
@@ -259,13 +235,7 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
       }
     };
 
-#ifdef VP8R_SWAR_PROF
-    if (lane == 0 && grp.frame[0] == 0 && r < 128) g_swar_rows[NB == 4 ? 0 : 1][r][0] = GlobalTimerNs();
-    long long row_wait = 0, row_pub = 0;
-    long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#endif
     for (int c = 0; c < cols; ++c) {
-      PROF_T(t0);
       uint32_t W[4 + 4 * NB];
 #pragma unroll
       for (int k = 0; k < NB; ++k)
@@ -290,7 +260,6 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
 #pragma unroll
       for (int k = 0; k < NB; ++k) swar::Transpose4(W[4 + 4 * k], W[5 + 4 * k], W[6 + 4 * k], W[7 + 4 * k]);
       FilterEdgesSwar<NB>(W, K, c > 0, any_inner, simple);
-      PROF_T(t1);
       if (c > 0) {  // the previous macroblock's last four columns are final for these rows now: into its ring place
         uint32_t t[4] = {W[0], W[1], W[2], W[3]};
         swar::Transpose4(t[0], t[1], t[2], t[3]);
@@ -311,7 +280,6 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
         tslot[(pl * NB + k) * kRegion + sub] = make_uint4(W[4 + 4 * k], W[5 + 4 * k], W[6 + 4 * k], W[7 + 4 * k]);
       }
       __syncwarp();
-      PROF_T(t2);
 
       // ---- horizontal edges: words = pixel rows of my four columns ----
 #pragma unroll
@@ -321,26 +289,19 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
       }
 #pragma unroll
       for (int i = 0; i < 4; ++i) W[i] = a4n[i];
-      PROF_T(t3);
       if (has_above && !have_above) {  // not prefetched: wait for the row above, then fetch
         if (above_local) {
           for (int got = lprog[lr - 1]; got < need; got = lprog[lr - 1])
-            __nanosleep(min(tune.sleep_base + tune.sleep_slope * (need - got - 1), 40000));
+            __nanosleep(min(kSwarSleepBase + kSwarSleepSlope * (need - got - 1), kSwarSleepMax));
           __threadfence_block();
-        } else if (tune.relaxed_poll) {
-          for (gseen = LoadFlagRelaxedSwar(gflag - 1); gseen < need; gseen = LoadFlagRelaxedSwar(gflag - 1))
-            __nanosleep(min(tune.sleep_base + tune.sleep_slope * (need - gseen - 1), 40000));
-          gseen = LoadFlagAcquireSwar(gflag - 1);
         } else {
           for (gseen = LoadFlagAcquireSwar(gflag - 1); gseen < need; gseen = LoadFlagAcquireSwar(gflag - 1))
-            __nanosleep(min(tune.sleep_base + tune.sleep_slope * (need - gseen - 1), 40000));
+            __nanosleep(min(kSwarSleepBase + kSwarSleepSlope * (need - gseen - 1), kSwarSleepMax));
         }
 #pragma unroll
         for (int y = 0; y < 4; ++y) W[y] = __ldcg(reinterpret_cast<const uint32_t *>(colp + c * kN + (ptrdiff_t)(y - 4) * pitch));
       }
-      PROF_T(t4);
       FilterEdgesSwar<NB>(W, K, has_above, any_inner, simple);
-      PROF_T(t5);
       {  // into the ring: rows above (1..3 of W) and the macroblock's rows, my four columns
         const int off = (c % Ring::kRingMbs) * kN + 4 * sub;
         const int chunk = off >> 4, low = off & 15;
@@ -367,7 +328,6 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
         __syncwarp();
       }
 
-      PROF_T(t6);
       // rows above of the next macroblock: fetch now if the row above is far enough already
       have_above = false;
       if (has_above && c + 1 < cols && seen >= min(c + 2, cols)) {
@@ -389,7 +349,7 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
           flush(c - Ring::kG);
         }
         const int stored = last ? cols : c;
-        if (last_of_band && (last || ((c / Ring::kG) % tune.band_stride) == 0)) {
+        if (last_of_band && (last || ((c / Ring::kG) % kSwarBandStride) == 0)) {
           __threadfence();
           __syncwarp();
           if (lane == 0) atomicExch(gflag, stored);
@@ -399,38 +359,15 @@ __device__ __forceinline__ void FilterBandSwar(const DevFrameJob *__restrict__ j
         __syncwarp();
         if (lane == 0) lprog[lr] = stored;
       }
-      PROF_T(t7);
-      PROF_ADD(NB == 4 ? 0 : 8, t0, t1);  // load hand-over, transposes, vertical edges
-      PROF_ADD(NB == 4 ? 1 : 9, t1, t2);  // carry into the ring, transposes back, tile write, warp barrier
-      PROF_ADD(NB == 4 ? 2 : 10, t2, t3);  // tile read
-      PROF_ADD(NB == 4 ? 3 : 11, t3, t4);  // wait for the row above + its rows
-      PROF_ADD(NB == 4 ? 4 : 12, t4, t5);  // horizontal edges
-      PROF_ADD(NB == 4 ? 5 : 13, t5, t6);  // ring writes + carry hand-over
-      PROF_ADD(NB == 4 ? 6 : 14, t6, t7);  // prefetch of rows above, flush, fence, publish
-      PROF_COUNT(NB == 4 ? 7 : 15);
-#ifdef VP8R_SWAR_PROF
-      row_wait += t4 - t3;
-      row_pub += t7 - t6;
-#endif
     }
-#ifdef VP8R_SWAR_PROF
-    if (lane == 0 && grp.frame[0] == 0 && r < 128) {
-      g_swar_rows[NB == 4 ? 0 : 1][r][1] = GlobalTimerNs();
-      g_swar_rows[NB == 4 ? 0 : 1][r][2] = row_wait;
-      g_swar_rows[NB == 4 ? 0 : 1][r][3] = row_pub;
-    }
-    if (lane == 0)
-      for (int i = 0; i < 8; ++i) atomicAdd(&g_swar_prof[(NB == 4 ? 0 : 8) + i], (unsigned long long)prof_acc[i]);
-#endif
   }
 }
 
 }  // namespace
 
-template <int kSwarWarps, int kMinBlocks>
-__global__ void __launch_bounds__(kSwarWarps * 32, kMinBlocks) FilterSwarKernel(const DevFrameJob *__restrict__ jobs,
-                                                                     const FilterGroup *__restrict__ groups, int n_groups,
-                                                                     int n_bands, int *__restrict__ sync, const SwarTune tune) {
+__global__ void __launch_bounds__(kSwarWarps * 32, 1) FilterSwarKernel(const DevFrameJob *__restrict__ jobs,
+                                                        const FilterGroup *__restrict__ groups, int n_groups, int n_bands,
+                                                        int *__restrict__ sync) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_ticket;
   if (threadIdx.x == 0) s_ticket = atomicAdd(&sync[0], 1);
@@ -454,39 +391,13 @@ __global__ void __launch_bounds__(kSwarWarps * 32, kMinBlocks) FilterSwarKernel(
   for (int i = threadIdx.x; i < rpb; i += blockDim.x) lprog[i] = 0;
   __syncthreads();
   int *gflag = sync + 1 + (g * 2 + chroma) * n_bands + band;
-  if (chroma) FilterBandSwar<2, kSwarWarps>(jobs, grp, band, n_bands, gflag, lprog, tiles, rings, ptrs, tune);
-  else FilterBandSwar<4, kSwarWarps>(jobs, grp, band, n_bands, gflag, lprog, tiles, rings, ptrs, tune);
+  if (chroma) FilterBandSwar<2>(jobs, grp, band, n_bands, gflag, lprog, tiles, rings, ptrs);
+  else FilterBandSwar<4>(jobs, grp, band, n_bands, gflag, lprog, tiles, rings, ptrs);
 }
 
-#ifdef VP8R_SWAR_PROF
-void SwarProfDump() {
-  unsigned long long h[16];
-  if (cudaMemcpyFromSymbol(h, g_swar_prof, sizeof(h)) != cudaSuccess) return;
-  static const char *names[7] = {"vertical", "carry-store+tile-write", "tile-read", "wait-above", "horizontal", "stores+carry", "publish"};
-  for (int kind = 0; kind < 2; ++kind) {
-    const unsigned long long steps = h[kind * 8 + 7];
-    if (!steps) continue;
-    unsigned long long total = 0;
-    for (int i = 0; i < 7; ++i) total += h[kind * 8 + i];
-    fprintf(stderr, "[swar prof] %s: %llu steps, %.0f cycles per step\n", kind ? "chroma" : "luma", steps, double(total) / steps);
-    for (int i = 0; i < 7; ++i) fprintf(stderr, "[swar prof]   %-24s %8.0f\n", names[i], double(h[kind * 8 + i]) / steps);
-  }
-  static unsigned long long rows[2][128][4];
-  if (cudaMemcpyFromSymbol(rows, g_swar_rows, sizeof(rows)) != cudaSuccess) return;
-  for (int kind = 0; kind < 2; ++kind) {
-    fprintf(stderr, "[swar prof] %s rows of the last launch, group with frame 0: row, start(us), end(us), waiting(us at 1.9 GHz), publishing(us)\n", kind ? "chroma" : "luma");
-    const unsigned long long t0 = rows[kind][0][0];
-    for (int r = 0; r < 128 && rows[kind][r][1]; ++r)
-      if (r < 5 || r % 8 == 7 || !rows[kind][r + 1 < 128 ? r + 1 : r][1]) fprintf(stderr, "[swar prof]   %3d %9.1f %9.1f\n", r, (rows[kind][r][0] - t0) / 1e3, (rows[kind][r][1] - rows[kind][r][0]) / 1e3);
-  }
-}
-#else
-void SwarProfDump() {}
-#endif
-
-template <int kSwarWarps, int kMinBlocks>
-static cudaError_t LaunchSwarVariant(const DevFrameJob *jobs, const FilterGroup *groups, int n_groups, int max_rows, int *sync,
-                                     int sync_ints, cudaStream_t st, const SwarTune &tune) {
+cudaError_t LaunchFilterSwar(const DevFrameJob *jobs, const FilterGroup *groups, int n_groups, int max_rows, int *sync,
+                             int sync_ints, cudaStream_t st) {
+  if (n_groups <= 0) return cudaSuccess;
   int n_bands = (max_rows + kSwarWarps - 1) / kSwarWarps;
   if (n_bands > 64) n_bands = 64;
   const int n_flags = 1 + 2 * n_groups * n_bands;
@@ -496,34 +407,11 @@ static cudaError_t LaunchSwarVariant(const DevFrameJob *jobs, const FilterGroup 
   const int rpb = (max_rows + n_bands - 1) / n_bands;
   const size_t smem = ((size_t(rpb) * 4 + 15) & ~size_t(15)) + size_t(kSwarWarps) * (kSwarTileBytes + kSwarRingBytes + kSwarPtrBytes);
   if (smem > 48 * 1024) {
-    e = cudaFuncSetAttribute(FilterSwarKernel<kSwarWarps, kMinBlocks>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    e = cudaFuncSetAttribute(FilterSwarKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
-  FilterSwarKernel<kSwarWarps, kMinBlocks><<<2 * n_groups * n_bands, kSwarWarps * 32, smem, st>>>(jobs, groups, n_groups, n_bands, sync, tune);
+  FilterSwarKernel<<<2 * n_groups * n_bands, kSwarWarps * 32, smem, st>>>(jobs, groups, n_groups, n_bands, sync);
   return cudaGetLastError();
-}
-
-cudaError_t LaunchFilterSwar(const DevFrameJob *jobs, const FilterGroup *groups, int n_groups, int max_rows, int *sync,
-                             int sync_ints, cudaStream_t st) {
-  if (n_groups <= 0) return cudaSuccess;
-  static SwarTune tune = [] {
-    SwarTune t{400, 1500, 0, 4};
-    if (const char *v = std::getenv("VP8R_SWAR_SLEEP")) std::sscanf(v, "%d,%d", &t.sleep_base, &t.sleep_slope);
-    if (const char *v = std::getenv("VP8R_SWAR_RELAXED")) t.relaxed_poll = std::atoi(v);
-    if (const char *v = std::getenv("VP8R_SWAR_STRIDE")) t.band_stride = std::max(1, std::atoi(v));
-    return t;
-  }();
-  static const int variant = [] { const char *v = std::getenv("VP8R_SWAR_VARIANT"); return v ? std::atoi(v) : 0; }();
-  // CTA shape (warps = macroblock rows per band, CTAs per SM).  Measured at 512 1080p frames per launch
-  // (profiles/r2_filter_swar.md): 12 x 1 = 2.61 ms, 10 x 1 = 2.67, 8 x 1 = 2.72, 6 x 2 = 2.77, 16 x 1 = 3.66,
-  // 17 x 1 = 3.99, 4 x 5 = 4.19 (the scalar kernel: 4.11).  More resident warps lose: 12.5 KB of shared memory
-  // per warp leave little L1 for the row loads (each 32-byte sector is read in two consecutive steps).
-  switch (variant) {
-    case 1: return LaunchSwarVariant<8, 1>(jobs, groups, n_groups, max_rows, sync, sync_ints, st, tune);
-    case 2: return LaunchSwarVariant<4, 5>(jobs, groups, n_groups, max_rows, sync, sync_ints, st, tune);
-    case 3: return LaunchSwarVariant<16, 1>(jobs, groups, n_groups, max_rows, sync, sync_ints, st, tune);
-    default: return LaunchSwarVariant<12, 1>(jobs, groups, n_groups, max_rows, sync, sync_ints, st, tune);
-  }
 }
 
 }  // namespace vp8r

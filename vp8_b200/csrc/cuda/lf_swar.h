@@ -21,14 +21,6 @@
 #else
 #define VP8R_HD inline
 #endif
-// The three edge routines are big (120-175 instructions each).  A kernel that runs them eight times per
-// macroblock step can ask for ONE copy each (VP8R_SWAR_EDGE_NOINLINE): many warps at different places of
-// a fully inlined step miss the instruction cache on every fetch.
-#if defined(__CUDACC__) && defined(VP8R_SWAR_EDGE_NOINLINE)
-#define VP8R_EDGE __device__ __noinline__
-#else
-#define VP8R_EDGE VP8R_HD
-#endif
 
 namespace vp8r {
 namespace swar {
@@ -170,7 +162,7 @@ VP8R_HD uint32_t Apply(uint32_t pixel, uint32_t biased, int bias) { return AddCl
 VP8R_HD uint32_t Hi(uint32_t lanes) { return Prmt(lanes, 0u, 0x4341u); }  // upper byte of each lane
 
 // Sub-block (inner) edge of the normal filter, src/filter.cc:37-44.  P3/P2/Q2/Q3 only enter the decision.
-VP8R_EDGE void NormalInner(uint32_t P3, uint32_t P2, uint32_t &P1, uint32_t &P0, uint32_t &Q0, uint32_t &Q1, uint32_t Q2,
+VP8R_HD void NormalInner(uint32_t P3, uint32_t P2, uint32_t &P1, uint32_t &P0, uint32_t &Q0, uint32_t &Q1, uint32_t Q2,
                          uint32_t Q3, const EdgeK &k) {
   const Flags f = NormalFlags(P3, P2, P1, P0, Q0, Q1, Q2, Q3, k.k_int, k.k_hev, k.k_sb);
   const uint32_t m_off = ByteMask(f.off_e, f.off_o);
@@ -199,7 +191,7 @@ VP8R_EDGE void NormalInner(uint32_t P3, uint32_t P2, uint32_t &P1, uint32_t &P0,
 }
 
 // Macroblock edge of the normal filter, src/filter.cc:46-67.
-VP8R_EDGE void NormalMbEdge(uint32_t P3, uint32_t &P2, uint32_t &P1, uint32_t &P0, uint32_t &Q0, uint32_t &Q1, uint32_t &Q2,
+VP8R_HD void NormalMbEdge(uint32_t P3, uint32_t &P2, uint32_t &P1, uint32_t &P0, uint32_t &Q0, uint32_t &Q1, uint32_t &Q2,
                           uint32_t Q3, const EdgeK &k) {
   const Flags f = NormalFlags(P3, P2, P1, P0, Q0, Q1, Q2, Q3, k.k_int, k.k_hev, k.k_mb);
   const uint32_t m_off = ByteMask(f.off_e, f.off_o);
@@ -237,7 +229,7 @@ VP8R_EDGE void NormalMbEdge(uint32_t P3, uint32_t &P2, uint32_t &P1, uint32_t &P
 }
 
 // Simple filter (luma only), src/filter.cc:14-16,69-71: the edge limit alone decides, p0 / q0 move.
-VP8R_EDGE void SimpleEdge(uint32_t P1, uint32_t &P0, uint32_t &Q0, uint32_t Q1, uint32_t k_e) {
+VP8R_HD void SimpleEdge(uint32_t P1, uint32_t &P0, uint32_t &Q0, uint32_t Q1, uint32_t k_e) {
   uint32_t se, so;
   EdgeTest(P1, P0, Q0, Q1, k_e, se, so);
   const uint32_t m_off = ByteMask(se, so);

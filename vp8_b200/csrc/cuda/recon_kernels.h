@@ -43,7 +43,7 @@ struct DevFrameJob {
   const int16_t *payload;
   DevPlanes cur;
   DevPlanes ref[4];  // indexed by reference frame id 1..3 (last, golden, altref)
-  const DevTensorMap *ref_tmap[4];  // per reference frame: descriptors of its Y, U, V planes (nullptr: no TMA path)
+  const DevTensorMap *ref_tmap[4];  // per reference frame: descriptors of its Y, U, V planes
   int pitch_y, pitch_c;
   int mb_cols, mb_rows;
   int n_intra, n_inter;
@@ -51,7 +51,6 @@ struct DevFrameJob {
   const uint32_t *intra_levels;     // n_intra_levels+1 offsets, then MB indices sorted by level
   int16_t dq[4][6];
   uint8_t key_frame, version, filter_type, lf_level, sharpness;
-  uint8_t levels_in_one_launch;  // host-built level table walked by IntraLevelsKernel instead of one launch per level
   uint8_t pack_layout;           // PackKernel: VP8R_LAYOUT_I420 / _NV12; ConvertRgbKernel: VP8R_LAYOUT_RGB24 / _RGB_PLANAR;
                                  // StageSourceKernel: the layout of stage_src (any of the four)
   uint8_t enc_flags;             // K_encode: VP8R_ENC_*
@@ -117,10 +116,9 @@ cudaError_t InitEncodeTables(const unsigned short *bpred_lut);  // enc_kernels.c
 cudaError_t LaunchIntraLevels(const DevFrameJob *jobs, int n_frames, cudaStream_t st);
 // Blocks (32 B) of device coefficient area a frame with deferred tokens needs.
 inline size_t TokenCoefBlocks(int mb_cols, int mb_rows) { return size_t(mb_cols) * mb_rows * 25; }
-// K_inter: dequant + IWHT/IDCT + motion compensation + residual add for every inter MB.
-// `tma`: reference windows of macroblocks with one motion vector are staged in shared memory by bulk tensor
-// loads (every job must carry ref_tmap); otherwise by 32-bit loads of the lanes.
-cudaError_t LaunchInter(const DevFrameJob *jobs, int n_frames, int max_cols, int max_rows, cudaStream_t st, bool tma = false);
+// K_inter: dequant + IWHT/IDCT + motion compensation + residual add for every inter MB.  Reference windows of
+// macroblocks with one motion vector are staged in shared memory by bulk tensor loads through the job's ref_tmap.
+cudaError_t LaunchInter(const DevFrameJob *jobs, int n_frames, int max_cols, int max_rows, cudaStream_t st);
 // K_intra: dequant + IWHT/IDCT + intra prediction as a per-frame macroblock wavefront.
 cudaError_t LaunchIntra(const DevFrameJob *jobs, int n_frames, int max_rows, cudaStream_t st);
 // Flat intra: every intra MB of dependency level `level` (frames with n_intra_levels > 0).
@@ -149,7 +147,6 @@ cudaError_t LaunchFilter(const DevFrameJob *jobs, int n_frames, int max_rows, in
 cudaError_t LaunchBorder(const DevFrameJob *jobs, int n_frames, cudaStream_t st);
 cudaError_t LaunchFilterSwar(const DevFrameJob *jobs, const FilterGroup *groups, int n_groups, int max_rows, int *sync,
                              int sync_ints, cudaStream_t st);
-void SwarProfDump();  // development aid, see filter_swar.cu (no-op in normal builds)
 // Ints of `sync` scratch LaunchFilter needs for a batch.
 inline int FilterSyncInts(int n_frames) { return 1 + n_frames * 128; }
 // Host->device staging without the copy engines (which the packed read-back keeps busy): `src` is

@@ -146,14 +146,11 @@ struct vp8r_engine {
   uint64_t fence_head = 0;
   // first failure of a device-side parse that has been found but not yet reported
   std::string deferred_error;
-  // intra scheduling of host-parsed inter frames: one launch per dependency level (default) or one
-  // level-walking launch (VP8R_INTRA_ONE_LAUNCH=1)
-  bool intra_one_launch = false;
-  // loop filter form: 0 = by batch size (batch form from `swar_min_frames` filtered frames on), 1 = always
-  // the scalar form, 2 = always the batch form (VP8R_FILTER=scalar|swar, VP8R_FILTER_SWAR_MIN=<frames>)
-  bool inter_tma = true;  // reference windows by TMA (VP8R_INTER=ldg: by the lanes' 32-bit loads)
+  // loop filter form: 0 = by batch size (the batch form from kSwarMinFrames filtered frames on), 1 = always the
+  // scalar form, 2 = always the batch form.  VP8R_FILTER=scalar|swar forces one, so that tests can run both forms
+  // on the same batch.
   int filter_mode = 0;
-  int swar_min_frames = 128;  // measured: 64 frames 1.22 ms (batch) vs 1.06 (scalar); 256: 1.67 vs 2.23; 512: 2.61 vs 4.11
+  static constexpr int kSwarMinFrames = 128;  // measured: 64 frames 1.22 ms (batch) vs 1.06 (scalar); 256: 1.67 vs 2.23; 512: 2.61 vs 4.11
   // timing
   bool timing = false;
   std::vector<EventPair> live;
@@ -278,6 +275,9 @@ int ConfigureStream(vp8r_stream *s, const vp8r_frame_hdr &h) {
   CU_TRY(SyncParseStreams(s->eng));
   CU_TRY(cudaStreamSynchronize(s->eng->st));
   FreeSurfaces(s);
+  // until the new pool is complete the stream has no geometry and no frame: a failure below leaves nothing to decode
+  s->mb_cols = s->mb_rows = 0;
+  s->have_frame = false;
   const int B = vp8r::kBorder;
   const int wa = h.mb_cols * 16, ha = h.mb_rows * 16;
   s->pitch_y = wa + 2 * B;
@@ -297,25 +297,25 @@ int ConfigureStream(vp8r_stream *s, const vp8r_frame_hdr &h) {
     sf.planes.u = sf.base + ysz + size_t(B) * s->pitch_c + B;
     sf.planes.v = sf.base + ysz + csz + size_t(B) * s->pitch_c + B;
   }
-  {  // TMA descriptors of the padded planes (motion compensation fetches its reference windows with them)
+  {  // TMA descriptors of the padded planes: motion compensation fetches its reference windows with them
     vp8r::DevTensorMap h_maps[15];
-    bool ok = true;
-    for (int k = 0; k < 5 && ok; ++k) {
+    for (int k = 0; k < 5; ++k) {
       uint8_t *base = s->surf[k].base;
-      ok = EncodePlaneMap(&h_maps[3 * k + 0], base, s->pitch_y, ha + 2 * B, s->pitch_y, vp8r::kTmaLumaBoxW, vp8r::kTmaLumaBoxH) &&
-           EncodePlaneMap(&h_maps[3 * k + 1], base + ysz, s->pitch_c, ha / 2 + 2 * B, s->pitch_c, vp8r::kTmaChromaBoxW, vp8r::kTmaChromaBoxH) &&
-           EncodePlaneMap(&h_maps[3 * k + 2], base + ysz + csz, s->pitch_c, ha / 2 + 2 * B, s->pitch_c, vp8r::kTmaChromaBoxW, vp8r::kTmaChromaBoxH);
-    }
-    if (ok) {
-      void *p = nullptr;
-      if (cudaMalloc(&p, sizeof(h_maps)) != cudaSuccess) {
-        SetError("cudaMalloc(tensor maps) failed");
-        return VP8R_ERR_NOMEM;
+      if (!EncodePlaneMap(&h_maps[3 * k + 0], base, s->pitch_y, ha + 2 * B, s->pitch_y, vp8r::kTmaLumaBoxW, vp8r::kTmaLumaBoxH) ||
+          !EncodePlaneMap(&h_maps[3 * k + 1], base + ysz, s->pitch_c, ha / 2 + 2 * B, s->pitch_c, vp8r::kTmaChromaBoxW, vp8r::kTmaChromaBoxH) ||
+          !EncodePlaneMap(&h_maps[3 * k + 2], base + ysz + csz, s->pitch_c, ha / 2 + 2 * B, s->pitch_c, vp8r::kTmaChromaBoxW, vp8r::kTmaChromaBoxH)) {
+        SetError("cuTensorMapEncodeTiled failed for a reference plane (no driver entry point, or the descriptor was refused)");
+        return VP8R_ERR_CUDA;
       }
-      s->d_tmaps = static_cast<vp8r::DevTensorMap *>(p);
-      CU_TRY(cudaMemcpyAsync(p, h_maps, sizeof(h_maps), cudaMemcpyHostToDevice, s->eng->st));
-      CU_TRY(cudaStreamSynchronize(s->eng->st));  // h_maps is on the stack
     }
+    void *p = nullptr;
+    if (cudaMalloc(&p, sizeof(h_maps)) != cudaSuccess) {
+      SetError("cudaMalloc(tensor maps) failed");
+      return VP8R_ERR_NOMEM;
+    }
+    s->d_tmaps = static_cast<vp8r::DevTensorMap *>(p);
+    CU_TRY(cudaMemcpyAsync(p, h_maps, sizeof(h_maps), cudaMemcpyHostToDevice, s->eng->st));
+    CU_TRY(cudaStreamSynchronize(s->eng->st));  // h_maps is on the stack
   }
   {
     const size_t n_mb = size_t(h.mb_cols) * h.mb_rows;
@@ -333,7 +333,6 @@ int ConfigureStream(vp8r_stream *s, const vp8r_frame_hdr &h) {
   s->width = h.width;
   s->height = h.height;
   s->ref[0] = s->ref[1] = s->ref[2] = s->ref[3] = -1;
-  s->have_frame = false;
   return VP8R_OK;
 }
 
@@ -498,7 +497,7 @@ void FillJobSurfaces(const vp8r_stream *s, int cur, DevFrameJob *j) {
   j->cur = s->surf[cur].planes;
   for (int k = 1; k < 4; ++k) {
     j->ref[k] = s->ref[k] >= 0 ? s->surf[s->ref[k]].planes : vp8r::DevPlanes{};
-    j->ref_tmap[k] = (s->ref[k] >= 0 && s->d_tmaps) ? s->d_tmaps + 3 * s->ref[k] : nullptr;
+    j->ref_tmap[k] = s->ref[k] >= 0 ? s->d_tmaps + 3 * s->ref[k] : nullptr;
   }
   j->ref[0] = vp8r::DevPlanes{};
   j->ref_tmap[0] = nullptr;
@@ -572,13 +571,13 @@ int PickCurrent(const vp8r_stream *s) {
 
 // Filter groups for FilterSwarKernel, behind the batch's n jobs in the slot's table: the filtered jobs with the same
 // geometry and filter type, eight to a warp, in batch order within a group (filter_swar.cu).  There are none when the
-// scalar FilterKernel runs (fewer than swar_min_frames filtered frames, or VP8R_FILTER).  Returns their number.
+// scalar FilterKernel runs (fewer than kSwarMinFrames filtered frames, or VP8R_FILTER=scalar).  Returns their number.
 int BuildFilterGroups(const vp8r_engine *e, Slot &sl, int n) {
   const DevFrameJob *jobs = sl.h_jobs;
   std::vector<int> order;
   for (int i = 0; i < n; ++i)
     if (jobs[i].lf_level != 0) order.push_back(i);
-  const bool swar = e->filter_mode == 2 || (e->filter_mode == 0 && int(order.size()) >= e->swar_min_frames);
+  const bool swar = e->filter_mode == 2 || (e->filter_mode == 0 && int(order.size()) >= vp8r_engine::kSwarMinFrames);
   if (!swar || order.empty()) return 0;
   auto key = [&](int i) {
     return (uint64_t(jobs[i].mb_cols) << 32) | (uint64_t(jobs[i].mb_rows) << 8) | uint64_t(jobs[i].filter_type != 0);
@@ -901,11 +900,9 @@ int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const 
   std::vector<int> cur;
   rc = StageEncoderSources(e, sl, n, streams, src, L, &cur);
   if (rc) return rc;
-  bool tma = e->inter_tma;
   for (int i = 0; i < n; ++i) {
     sl.h_jobs[i].n_inter = int(L.n_mb);
     sl.h_jobs[i].enc_search_range = search_range;
-    tma = tma && streams[i]->d_tmaps != nullptr;
   }
   int n_groups = 0;
   rc = SubmitEncoderJobs(e, sl, n, src, L, &n_groups);
@@ -913,7 +910,7 @@ int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const 
   {
     ScopedTimer t(e, 0);
     CU_TRY(vp8r::LaunchEncodeInter(sl.d_jobs, n, cols, rows, e->st));
-    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st, tma));
+    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st));
     e->acc.launches_inter += 2;
   }
   rc = LaunchFilterAndBorder(e, sl, n, rows, n_groups);
@@ -968,10 +965,7 @@ VP8R_API int vp8r_engine_create(int device, void *cuda_stream, vp8r_engine **out
   }
   if (!e) return VP8R_ERR_NOMEM;
   e->device = device;
-  if (const char *v = std::getenv("VP8R_INTRA_ONE_LAUNCH")) e->intra_one_launch = v[0] == '1';
   if (const char *v = std::getenv("VP8R_FILTER")) e->filter_mode = std::strcmp(v, "scalar") == 0 ? 1 : (std::strcmp(v, "swar") == 0 ? 2 : 0);
-  if (const char *v = std::getenv("VP8R_INTER")) e->inter_tma = std::strcmp(v, "ldg") != 0;
-  if (const char *v = std::getenv("VP8R_FILTER_SWAR_MIN")) e->swar_min_frames = std::max(1, std::atoi(v));
   if (cuda_stream) {
     e->st = static_cast<cudaStream_t>(cuda_stream);
   } else {
@@ -1012,7 +1006,6 @@ VP8R_API void vp8r_engine_destroy(vp8r_engine *e) {
   if (!e) return;
   cudaSetDevice(e->device);
   cudaStreamSynchronize(e->st);
-  vp8r::SwarProfDump();
   if (e->st_copy) {
     cudaStreamSynchronize(e->st_copy);
     cudaStreamDestroy(e->st_copy);
@@ -1191,7 +1184,7 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
 
   // Pass 2: jobs + host->device staging.
   int max_mbs = 0, max_rows = 0, max_cols = 0, max_cols_all = 0, max_parts = 1;
-  bool any_inter = false, any_intra = false, any_wave = false, any_tokens = false, any_modes = false, any_level_walk = false;
+  bool any_inter = false, any_intra = false, any_wave = false, any_tokens = false, any_modes = false;
   std::vector<int> level_max;  // per dependency level: most intra MBs of that level in any frame
   size_t at = 0, gather_max = 0;
   int n_groups = 0;
@@ -1235,11 +1228,7 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
       j.n_inter = int(h.n_inter_mbs);
       j.n_intra = n_mb - j.n_inter;
       j.n_intra_levels = int(h.n_intra_levels);
-      if (h.n_intra_levels && e->intra_one_launch) {
-        j.intra_levels = reinterpret_cast<const uint32_t *>(j.payload + size_t(h.intra_levels_at) * 16);
-        j.levels_in_one_launch = 1;
-        any_level_walk = true;  // launches IntraLevelsKernel
-      } else if (h.n_intra_levels) {
+      if (h.n_intra_levels) {
         j.intra_levels = reinterpret_cast<const uint32_t *>(j.payload + size_t(h.intra_levels_at) * 16);
         if (level_max.size() < h.n_intra_levels) level_max.resize(h.n_intra_levels, 0);
         if (f->blob) {
@@ -1323,9 +1312,7 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
   }
   if (any_inter) {
     ScopedTimer t(e, 0);
-    bool tma = e->inter_tma;
-    for (int i = 0; i < n && tma; ++i) tma = streams[i]->d_tmaps != nullptr;
-    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, max_cols_all, max_rows, e->st, tma));
+    CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, max_cols_all, max_rows, e->st));
     e->acc.launches_inter++;
   }
   if (any_intra) {
@@ -1334,7 +1321,7 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
       CU_TRY(vp8r::LaunchIntraFlat(sl.d_jobs, n, int(L), level_max[L], e->st));
       e->acc.launches_intra++;
     }
-    if (any_modes || any_level_walk) {
+    if (any_modes) {
       CU_TRY(vp8r::LaunchIntraLevels(sl.d_jobs, n, e->st));
       e->acc.launches_intra++;
     }
