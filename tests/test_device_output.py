@@ -316,8 +316,9 @@ def test_consumer_on_another_stream(built, engine_stream):
 
 @pytest.mark.gpu
 def test_rejections_leave_the_engine_working(engine):
-    """Host memory (pinned or pageable), a stride below a frame, a stream without a frame, and tensors of the wrong
-    dtype / device / shape are refused; the engine decodes correctly afterwards."""
+    """Host memory (pinned or pageable), a stride below a frame, a stream without a frame, tensors of the wrong
+    dtype / device / shape and a packed read-back whose staging the allocator refuses are refused; the engine reads back
+    and decodes correctly afterwards."""
     import torch
     import vp8_b200
     lib = engine._lib
@@ -347,6 +348,15 @@ def test_rejections_leave_the_engine_working(engine):
                 engine.read_batch_device([st], bad, "rgb")
         with pytest.raises(ValueError):
             engine.read_batch_device([st], dev, "bgr")
+        # a stride of 1 TiB asks for 8 TiB of staging, which the allocator refuses at once; the next packed read-back
+        # allocates its staging anew and delivers the same bytes
+        ib = helpers.i420_bytes(w, h)
+        before, after = (C.c_uint8 * ib)(), (C.c_uint8 * ib)()
+        assert lib.vp8r_read_batch_packed(engine.handle, 1, sa, C.addressof(before), ib, 0) == 0
+        assert lib.vp8r_read_batch_packed(engine.handle, 1, sa, C.addressof(after), 1 << 40, 0) != 0
+        assert lib.vp8r_read_batch_packed(engine.handle, 1, sa, C.addressof(after), ib, 0) == 0
+        assert bytes(after) == bytes(before)
+        assert lib.vp8r_engine_sync(engine.handle) == 0
     finally:
         st.close()
         empty.close()

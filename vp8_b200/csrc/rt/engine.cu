@@ -8,7 +8,9 @@
 #include <atomic>
 #include <cstdio>
 #include <cstdlib>
+#include <cstdint>
 #include <cstring>
+#include <initializer_list>
 #include <mutex>
 #include <new>
 #include <string>
@@ -81,9 +83,11 @@ struct vp8r_stream {
 };
 
 namespace {
+// What a timer measures: the vp8r_timers field its time goes to (kNone: not timed).
+enum class Timer { kInter, kIntra, kFilter, kH2D, kD2H, kTokens, kBorder, kNone };
 struct EventPair {
   cudaEvent_t a, b;
-  int cls;
+  Timer cls;
 };
 struct Slot {
   DevFrameJob *h_jobs = nullptr, *d_jobs = nullptr;
@@ -132,8 +136,8 @@ struct vp8r_engine {
   cudaStream_t st_segments = nullptr;
   cudaEvent_t pack_done[kPackBufs] = {}, copy_done[kPackBufs] = {};
   bool copy_busy[kPackBufs] = {};
-  bool kernel_busy[kPackBufs] = {};  // pack_done of the part marks a device read-back (vp8r_read_batch_device) not yet waited for
-  cudaEvent_t consumer_ev = nullptr;  // vp8r_read_batch_device: the caller's stream, before the conversion
+  bool kernel_busy[kPackBufs] = {};  // pack_done of the part marks an output kernel (RunOutputJobs) not yet waited for
+  cudaEvent_t consumer_ev = nullptr;  // WaitForCaller: the caller's stream, before the engine's work
   cudaEvent_t fence_copy_ev[16] = {};
   bool fence_has_copy[16] = {};
   // checksum scratch
@@ -336,41 +340,68 @@ int ConfigureStream(vp8r_stream *s, const vp8r_frame_hdr &h) {
   return VP8R_OK;
 }
 
+// A buffer that Regrow replaces: device memory, or pinned host memory (mapped into the device's address space when
+// `mapped` receives its device pointer).
+struct GrownBuffer {
+  void **p;
+  size_t bytes;
+  bool host;
+  void **mapped;
+};
+template <class T>
+GrownBuffer DeviceBuf(T **p, size_t bytes) {
+  return {reinterpret_cast<void **>(p), bytes, false, nullptr};
+}
+template <class T>
+GrownBuffer PinnedBuf(T **p, size_t bytes, T **mapped = nullptr) {
+  return {reinterpret_cast<void **>(p), bytes, true, reinterpret_cast<void **>(mapped)};
+}
+
+// Replaces buffers that share one capacity by larger ones.  *capacity becomes `cap` only once every buffer is in
+// place.  A refused allocation leaves it 0 and the refused buffer null, so that the next call allocates again, and
+// clears the runtime's last error, which the next launch check would otherwise report as a failure of its own.
+template <class Cap>
+cudaError_t Regrow(Cap *capacity, Cap cap, std::initializer_list<GrownBuffer> bufs) {
+  *capacity = 0;
+  for (const GrownBuffer &b : bufs) {
+    if (*b.p) b.host ? cudaFreeHost(*b.p) : cudaFree(*b.p);
+    *b.p = nullptr;
+    if (b.mapped) *b.mapped = nullptr;
+  }
+  for (const GrownBuffer &b : bufs) {
+    cudaError_t err = b.host ? cudaHostAlloc(b.p, b.bytes, b.mapped ? cudaHostAllocMapped : cudaHostAllocDefault)
+                             : cudaMalloc(b.p, b.bytes);
+    if (err == cudaSuccess && b.mapped) err = cudaHostGetDevicePointer(b.mapped, *b.p, 0);
+    if (err != cudaSuccess) {
+      cudaGetLastError();
+      return err;
+    }
+  }
+  *capacity = cap;
+  return cudaSuccess;
+}
+
 int GrowSlot(vp8r_engine *e, Slot &sl, int n_jobs, size_t arena_bytes) {
   if (n_jobs > sl.cap_jobs) {
     int cap = std::max(n_jobs, sl.cap_jobs * 2);
     cap = std::max(cap, 16);
     CU_TRY(cudaStreamSynchronize(e->st));
-    if (sl.h_jobs) cudaFreeHost(sl.h_jobs);
-    if (sl.d_jobs) cudaFree(sl.d_jobs);
-    sl.h_jobs = nullptr;
-    sl.d_jobs = nullptr;
     // the batch's filter groups (at most one per job) follow the jobs in the same table
     const size_t table = (sizeof(DevFrameJob) + sizeof(vp8r::FilterGroup)) * cap + 16;
-    CU_TRY(cudaHostAlloc(reinterpret_cast<void **>(&sl.h_jobs), table, cudaHostAllocDefault));
-    CU_TRY(cudaMalloc(reinterpret_cast<void **>(&sl.d_jobs), table));
-    if (sl.h_status) cudaFreeHost(sl.h_status);
-    sl.h_status = sl.d_status = nullptr;
-    CU_TRY(cudaHostAlloc(reinterpret_cast<void **>(&sl.h_status), sizeof(int) * cap, cudaHostAllocMapped));
-    CU_TRY(cudaHostGetDevicePointer(reinterpret_cast<void **>(&sl.d_status), sl.h_status, 0));
+    CU_TRY(Regrow(&sl.cap_jobs, cap, {PinnedBuf(&sl.h_jobs, table), DeviceBuf(&sl.d_jobs, table),
+                                      PinnedBuf(&sl.h_status, sizeof(int) * cap, &sl.d_status),
+                                      DeviceBuf(&sl.d_status_dev, sizeof(int) * cap)}));
     std::memset(sl.h_status, 0, sizeof(int) * cap);
-    if (sl.d_status_dev) cudaFree(sl.d_status_dev);
-    sl.d_status_dev = nullptr;
-    CU_TRY(cudaMalloc(reinterpret_cast<void **>(&sl.d_status_dev), sizeof(int) * cap));
-    sl.cap_jobs = cap;
   }
   if (arena_bytes > sl.arena_cap) {
-    size_t cap = std::max(arena_bytes + arena_bytes / 4, size_t(1) << 20);
+    const size_t cap = std::max(arena_bytes + arena_bytes / 4, size_t(1) << 20);
     CU_TRY(cudaStreamSynchronize(e->st));
-    if (sl.d_arena) cudaFree(sl.d_arena);
-    sl.d_arena = nullptr;
-    CU_TRY(cudaMalloc(reinterpret_cast<void **>(&sl.d_arena), cap));
-    sl.arena_cap = cap;
+    CU_TRY(Regrow(&sl.arena_cap, cap, {DeviceBuf(&sl.d_arena, cap)}));
   }
   return VP8R_OK;
 }
 
-EventPair GetPair(vp8r_engine *e, int cls) {
+EventPair GetPair(vp8r_engine *e, Timer cls) {
   EventPair p;
   if (!e->pool.empty()) {
     p = e->pool.back();
@@ -388,8 +419,8 @@ struct ScopedTimer {
   EventPair p;
   bool on;
   cudaStream_t stream;
-  ScopedTimer(vp8r_engine *eng, int cls, cudaStream_t on_stream = nullptr)
-      : e(eng), on(eng->timing), stream(on_stream ? on_stream : eng->st) {
+  ScopedTimer(vp8r_engine *eng, Timer cls, cudaStream_t on_stream = nullptr)
+      : e(eng), on(eng->timing && cls != Timer::kNone), stream(on_stream ? on_stream : eng->st) {
     if (on) {
       p = GetPair(e, cls);
       cudaEventRecord(p.a, stream);
@@ -408,13 +439,14 @@ void DrainTimers(vp8r_engine *e) {
     float ms = 0;
     if (cudaEventElapsedTime(&ms, p.a, p.b) == cudaSuccess) {
       switch (p.cls) {
-        case 0: e->acc.ms_inter += ms; break;
-        case 1: e->acc.ms_intra += ms; break;
-        case 2: e->acc.ms_filter += ms; break;
-        case 3: e->acc.ms_h2d += ms; break;
-        case 5: e->acc.ms_tokens += ms; break;
-        case 6: e->acc.ms_border += ms; break;
-        default: e->acc.ms_d2h += ms; break;
+        case Timer::kInter: e->acc.ms_inter += ms; break;
+        case Timer::kIntra: e->acc.ms_intra += ms; break;
+        case Timer::kFilter: e->acc.ms_filter += ms; break;
+        case Timer::kH2D: e->acc.ms_h2d += ms; break;
+        case Timer::kD2H: e->acc.ms_d2h += ms; break;
+        case Timer::kTokens: e->acc.ms_tokens += ms; break;
+        case Timer::kBorder: e->acc.ms_border += ms; break;
+        case Timer::kNone: break;
       }
     } else {
       cudaGetLastError();
@@ -428,27 +460,17 @@ void DrainTimers(vp8r_engine *e) {
 int EnsureScratchJobs(vp8r_engine *e, int n) {
   if (n <= e->cap_cjobs) return VP8R_OK;
   CU_TRY(cudaStreamSynchronize(e->st));
-  if (e->h_cjobs) cudaFreeHost(e->h_cjobs);
-  if (e->d_cjobs) cudaFree(e->d_cjobs);
-  if (e->h_sums) cudaFreeHost(e->h_sums);
-  if (e->d_sums) cudaFree(e->d_sums);
-  e->h_cjobs = e->d_cjobs = nullptr;
-  e->h_sums = e->d_sums = nullptr;
-  e->cap_cjobs = 0;
   const int cap = std::max(n, 64);
   const size_t table = sizeof(DevFrameJob) * cap * vp8r_engine::kPackBufs + 16;
-  CU_TRY(cudaHostAlloc(reinterpret_cast<void **>(&e->h_cjobs), table, cudaHostAllocDefault));
-  CU_TRY(cudaMalloc(reinterpret_cast<void **>(&e->d_cjobs), table));
-  CU_TRY(cudaHostAlloc(reinterpret_cast<void **>(&e->h_sums), sizeof(uint64_t) * cap, cudaHostAllocDefault));
-  CU_TRY(cudaMalloc(reinterpret_cast<void **>(&e->d_sums), sizeof(uint64_t) * cap));
-  e->cap_cjobs = cap;
+  CU_TRY(Regrow(&e->cap_cjobs, cap, {PinnedBuf(&e->h_cjobs, table), DeviceBuf(&e->d_cjobs, table),
+                                     PinnedBuf(&e->h_sums, sizeof(uint64_t) * cap), DeviceBuf(&e->d_sums, sizeof(uint64_t) * cap)}));
   return VP8R_OK;
 }
 
 // Takes the next of the kPackBufs rotating parts of the scratch job table (and of the packed staging buffer) for a
 // read-back.  LaunchCopy reads a part from pinned host memory while its kernel runs, so the host rewrites the part
 // only after the work that last read it has finished: the D2H copy of a packed read-back (which follows its pack
-// kernel), or the kernel of a device read-back.
+// kernel), or the kernel of any other output.
 int AcquirePart(vp8r_engine *e, int *part) {
   e->pack_flip = (e->pack_flip + 1) % vp8r_engine::kPackBufs;
   const int k = e->pack_flip;
@@ -462,6 +484,50 @@ int AcquirePart(vp8r_engine *e, int *part) {
   }
   *part = k;
   return VP8R_OK;
+}
+
+// Makes the engine's stream wait for the work queued so far on a caller's stream.  A null stream, or the engine's own,
+// asks for nothing; torch's default stream arrives as cudaStreamLegacy and is waited for like any other.
+int WaitForCaller(vp8r_engine *e, cudaStream_t caller) {
+  if (!caller || caller == e->st) return VP8R_OK;
+  CU_TRY(cudaEventRecord(e->consumer_ev, caller));
+  CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
+  return VP8R_OK;
+}
+
+// Makes a caller's stream wait for `ev`, recorded on the engine's stream (the same rules as WaitForCaller).
+int CallerWaitsFor(vp8r_engine *e, cudaStream_t caller, cudaEvent_t ev) {
+  if (!caller || caller == e->st) return VP8R_OK;
+  CU_TRY(cudaStreamWaitEvent(caller, ev, 0));
+  return VP8R_OK;
+}
+
+// The path of every output that runs one kernel over a scratch job table (packed, device, conversion, checksum): n jobs
+// in the next rotating part (*part, set before fill runs), each cleared and then set by fill(i, job).  The part goes to
+// the device with LaunchCopy and launch(device jobs) queues the kernel, timed as `cls`, on the engine's stream behind
+// the work queued on `caller` so far (nullptr: none).  pack_done[part] marks the part busy until the kernel has
+// finished, and the caller's stream waits for it.
+template <class Fill, class Launch>
+int RunOutputJobs(vp8r_engine *e, int n, Timer cls, cudaStream_t caller, int *part, Fill fill, Launch launch) {
+  int rc = EnsureScratchJobs(e, n);
+  if (!rc) rc = AcquirePart(e, part);
+  if (rc) return rc;
+  DevFrameJob *hj = e->h_cjobs + size_t(*part) * e->cap_cjobs, *dj = e->d_cjobs + size_t(*part) * e->cap_cjobs;
+  for (int i = 0; i < n; ++i) {
+    std::memset(&hj[i], 0, sizeof(DevFrameJob));
+    fill(i, hj[i]);
+  }
+  rc = WaitForCaller(e, caller);
+  if (rc) return rc;
+  {
+    ScopedTimer t(e, cls);
+    CU_TRY(vp8r::LaunchCopy(dj, hj, sizeof(DevFrameJob) * n, e->st));
+    CU_TRY(launch(dj));
+    e->acc.launches_other++;
+  }
+  CU_TRY(cudaEventRecord(e->pack_done[*part], e->st));
+  e->kernel_busy[*part] = true;
+  return CallerWaitsFor(e, caller, e->pack_done[*part]);
 }
 
 // Error words of a batch whose kernels have finished: a stream with a truncated frame stops decoding (its frame
@@ -596,23 +662,20 @@ int BuildFilterGroups(const vp8r_engine *e, Slot &sl, int n) {
   return n_groups;
 }
 
-// Loop filter (timer class 2) and border extension (class 6) of a batch whose jobs and filter groups are on the device.
+// Loop filter and border extension of a batch whose jobs and filter groups are on the device.
 int LaunchFilterAndBorder(vp8r_engine *e, const Slot &sl, int n, int max_rows, int n_groups) {
   {
-    ScopedTimer t(e, 2);
+    ScopedTimer t(e, Timer::kFilter);
     const int need_sync = vp8r::FilterSyncInts(n);
     if (need_sync > e->sync_cap) {
       CU_TRY(cudaStreamSynchronize(e->st));
-      if (e->d_sync) cudaFree(e->d_sync);
-      e->d_sync = nullptr;
-      CU_TRY(cudaMalloc(reinterpret_cast<void **>(&e->d_sync), sizeof(int) * size_t(need_sync) * 2));
-      e->sync_cap = need_sync * 2;
+      CU_TRY(Regrow(&e->sync_cap, need_sync * 2, {DeviceBuf(&e->d_sync, sizeof(int) * size_t(need_sync) * 2)}));
     }
     CU_TRY(vp8r::LaunchFilter(sl.d_jobs, n, max_rows, e->d_sync, e->sync_cap, e->st,
                               reinterpret_cast<const vp8r::FilterGroup *>(sl.d_jobs + n), n_groups));
     e->acc.launches_filter++;
   }
-  ScopedTimer t(e, 6);
+  ScopedTimer t(e, Timer::kBorder);
   CU_TRY(vp8r::LaunchBorder(sl.d_jobs, n, e->st));
   e->acc.launches_other++;
   return VP8R_OK;
@@ -660,14 +723,67 @@ bool IsEngineDeviceMemory(const vp8r_engine *e, const void *p) {
   return attr.type == cudaMemoryTypeDevice && attr.device == e->device;
 }
 
-// The arguments both encoders take.
-int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, vp8r_frame *const *out,
-                     int width, int height, int q_index, int loop_filter_level, int sharpness) {
-  if (!e || n <= 0 || !streams || !(src.host || src.dev) || !out || width < 1 || height < 1 || width > 16383 ||
-      height > 16383 || q_index < 0 || q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 ||
-      sharpness > 7)
+// A layout of include/vp8r.h and a frame size VP8 can code.  `call` names the refused call.
+int CheckLayoutAndSize(const std::string &call, int layout, int width, int height) {
+  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
+    SetError(call + ": unknown layout " + std::to_string(layout));
     return VP8R_ERR_INVALID_ARG;
-  int rc = EnsureDevice(e);
+  }
+  if (width < 1 || height < 1 || width > 16383 || height > 16383) {
+    SetError(call + ": frame size outside 1..16383");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  return VP8R_OK;
+}
+
+// The distance of two frames of a batch holds a width x height frame in `layout`.  `what` names the stride.
+int CheckStride(const std::string &what, size_t stride, int layout, int width, int height) {
+  if (stride >= LayoutBytes(layout, width, height)) return VP8R_OK;
+  SetError(what + " smaller than a frame");
+  return VP8R_ERR_INVALID_ARG;
+}
+
+// The streams of an output: each of this engine with a reconstructed frame, which fits `stride` in `layout`.
+int CheckFrameStreams(const vp8r_engine *e, int n, vp8r_stream *const *streams, size_t stride = SIZE_MAX,
+                      int layout = VP8R_LAYOUT_I420) {
+  for (int i = 0; i < n; ++i) {
+    const vp8r_stream *s = streams[i];
+    if (!s || s->eng != e || !s->have_frame) {
+      SetError("stream has no reconstructed frame");
+      return VP8R_ERR_STATE;
+    }
+    const int rc = CheckStride("stride", stride, layout, s->width, s->height);
+    if (rc) return rc;
+  }
+  return VP8R_OK;
+}
+
+// The arguments of the four encoder calls, with a message naming the call for each refusal.  search_range < 0: a key-
+// frame call, which takes none.  The checks that need neither the engine nor a stream come first.
+int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, vp8r_frame *const *out,
+                     int width, int height, int q_index, int loop_filter_level, int sharpness, int search_range) {
+  const std::string call = std::string(search_range < 0 ? "vp8r_encode_key_frames" : "vp8r_encode_inter_frames") +
+                           (src.dev ? "_device" : "");
+  if (!e || !streams || !(src.host || src.dev) || !out) {
+    SetError(call + ": null engine, streams, src or out");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (n <= 0) {
+    SetError(call + ": n <= 0");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  int rc = CheckLayoutAndSize(call, src.layout, width, height);
+  if (rc) return rc;
+  if (q_index < 0 || q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 || sharpness > 7) {
+    SetError(call + ": q_index, loop_filter_level or sharpness out of range");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (src.dev && (rc = CheckStride(call + ": stride", src.stride, src.layout, width, height))) return rc;
+  if (search_range >= 0 && (search_range < 4 || search_range > 24)) {
+    SetError(call + ": search_range outside 4..24");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  rc = EnsureDevice(e);
   if (rc) return rc;
   rc = CheckBatchStreams(e, n, streams);
   if (rc) return rc;
@@ -678,39 +794,6 @@ int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const E
     }
   if (src.dev && !IsEngineDeviceMemory(e, src.dev)) {
     SetError("src is not device memory of the engine's device (pinned, pageable and managed memory are refused)");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  return VP8R_OK;
-}
-
-// The checks of an encoder call with its source in device memory that need no device, with a message for each;
-// `what` names the call.  The encoder's other argument checks follow in CheckEncoderArgs.
-int CheckDeviceSourceArgs(const char *what, const vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src,
-                          size_t stride, int layout, vp8r_frame *const *out, int width, int height, int q_index,
-                          int loop_filter_level, int sharpness) {
-  const std::string call(what);
-  if (!e || !streams || !src || !out) {
-    SetError(call + ": null engine, streams, src or out");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (n <= 0) {
-    SetError(call + ": n <= 0");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
-    SetError(call + ": unknown layout " + std::to_string(layout));
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (width < 1 || height < 1 || width > 16383 || height > 16383) {
-    SetError(call + ": frame size outside 1..16383");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (q_index < 0 || q_index > 127 || loop_filter_level < 0 || loop_filter_level > 63 || sharpness < 0 || sharpness > 7) {
-    SetError(call + ": q_index, loop_filter_level or sharpness out of range");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (stride < LayoutBytes(layout, width, height)) {
-    SetError(call + ": stride smaller than a frame");
     return VP8R_ERR_INVALID_ARG;
   }
   return VP8R_OK;
@@ -796,11 +879,9 @@ int SubmitEncoderJobs(vp8r_engine *e, Slot &sl, int n, const EncoderSource &src,
   *n_groups = BuildFilterGroups(e, sl, n);
   CU_TRY(vp8r::LaunchCopy(sl.d_jobs, sl.h_jobs, sizeof(DevFrameJob) * n + sizeof(vp8r::FilterGroup) * *n_groups, e->st));
   if (!src.dev) return VP8R_OK;
-  if (src.producer && src.producer != e->st) {
-    CU_TRY(cudaEventRecord(e->consumer_ev, src.producer));
-    CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
-  }
-  ScopedTimer t(e, 3);
+  const int rc = WaitForCaller(e, src.producer);
+  if (rc) return rc;
+  ScopedTimer t(e, Timer::kH2D);
   CU_TRY(vp8r::LaunchStageSource(sl.d_jobs, n, src.layout, L.h.mb_cols * 16, L.h.mb_rows * 16, e->st));
   e->acc.launches_other++;
   return VP8R_OK;
@@ -839,7 +920,7 @@ int FinishEncoderBatch(vp8r_engine *e, const Slot &sl, int n, vp8r_stream *const
 // Row f4: closed-loop key-frame encoder (vp8r_encode_key_frames, _device).
 int EncodeKeyFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, int width, int height,
                     int q_index, int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out) {
-  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness);
+  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness, -1);
   if (rc) return rc;
   EncodeLayout L = MakeEncodeLayout(width, height, q_index, loop_filter_level, sharpness);
   L.h.key_frame = 1;
@@ -864,7 +945,7 @@ int EncodeKeyFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const En
   rc = SubmitEncoderJobs(e, sl, n, src, L, &n_groups);
   if (rc) return rc;
   {
-    ScopedTimer t(e, 1);
+    ScopedTimer t(e, Timer::kIntra);
     CU_TRY(vp8r::LaunchEncodeIntra(sl.d_jobs, n, L.h.mb_rows, e->st));
     e->acc.launches_intra++;
   }
@@ -877,8 +958,7 @@ int EncodeKeyFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const En
 // K_inter reconstructs from the records, then the loop filter and the border as for a decoded frame.
 int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, int width, int height,
                       int q_index, int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out) {
-  if (search_range < 4 || search_range > 24) return VP8R_ERR_INVALID_ARG;
-  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness);
+  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness, search_range);
   if (rc) return rc;
   for (int i = 0; i < n; ++i) {
     const vp8r_stream *s = streams[i];
@@ -908,7 +988,7 @@ int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const 
   rc = SubmitEncoderJobs(e, sl, n, src, L, &n_groups);
   if (rc) return rc;
   {
-    ScopedTimer t(e, 0);
+    ScopedTimer t(e, Timer::kInter);
     CU_TRY(vp8r::LaunchEncodeInter(sl.d_jobs, n, cols, rows, e->st));
     CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st));
     e->acc.launches_inter += 2;
@@ -1195,7 +1275,7 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
   for (int i = 0; i < n; ++i) deferred |= frames[i]->hdr.tokens_deferred != 0;
   cudaStream_t front = deferred ? e->st_parse[slot_index] : e->st;
   {
-    ScopedTimer t(e, 3, front);
+    ScopedTimer t(e, Timer::kH2D, front);
     for (int i = 0; i < n; ++i) {
       vp8r_stream *s = streams[i];
       vp8r_frame *f = frames[i];
@@ -1292,7 +1372,7 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
 
   if (any_tokens) {
     CU_TRY(cudaMemsetAsync(sl.d_status_dev, 0, sizeof(int) * n, front));
-    ScopedTimer t(e, 5, front);
+    ScopedTimer t(e, Timer::kTokens, front);
     if (any_modes) {
       // K_modes here, K_segments in batch order on its own stream, then back (see token_kernel.cu)
       CU_TRY(vp8r::LaunchModes(sl.d_jobs, n, max_cols, max_mbs, front));
@@ -1311,12 +1391,12 @@ VP8R_API int vp8r_reconstruct_batch(vp8r_engine *e, int n, vp8r_stream *const *s
     CU_TRY(cudaStreamWaitEvent(e->st, sl.parsed, 0));
   }
   if (any_inter) {
-    ScopedTimer t(e, 0);
+    ScopedTimer t(e, Timer::kInter);
     CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, max_cols_all, max_rows, e->st));
     e->acc.launches_inter++;
   }
   if (any_intra) {
-    ScopedTimer t(e, 1);
+    ScopedTimer t(e, Timer::kIntra);
     for (size_t L = 0; L < level_max.size(); ++L) {
       CU_TRY(vp8r::LaunchIntraFlat(sl.d_jobs, n, int(L), level_max[L], e->st));
       e->acc.launches_intra++;
@@ -1354,9 +1434,6 @@ VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *s
 VP8R_API int vp8r_encode_key_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
                                            int layout, void *producer_stream, int width, int height, int q_index,
                                            int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out) {
-  int rc = CheckDeviceSourceArgs("vp8r_encode_key_frames_device", e, n, streams, src, stride, layout, out, width, height,
-                                 q_index, loop_filter_level, sharpness);
-  if (rc) return rc;
   EncoderSource s;
   s.dev = static_cast<const uint8_t *>(src);
   s.stride = stride;
@@ -1376,13 +1453,6 @@ VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const 
 VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
                                              int layout, void *producer_stream, int width, int height, int q_index,
                                              int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out) {
-  int rc = CheckDeviceSourceArgs("vp8r_encode_inter_frames_device", e, n, streams, src, stride, layout, out, width, height,
-                                 q_index, loop_filter_level, sharpness);
-  if (rc) return rc;
-  if (search_range < 4 || search_range > 24) {
-    SetError("vp8r_encode_inter_frames_device: search_range outside 4..24");
-    return VP8R_ERR_INVALID_ARG;
-  }
   EncoderSource s;
   s.dev = static_cast<const uint8_t *>(src);
   s.stride = stride;
@@ -1394,78 +1464,48 @@ VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream 
 VP8R_API int vp8r_convert_to_i420_device(vp8r_engine *e, int n, const void *src, size_t src_stride, int layout, int width,
                                          int height, void *dst, size_t dst_stride, void *stream) {
   // argument checks that need no device come first
+  const std::string call = "vp8r_convert_to_i420_device";
   if (!e || !src || !dst) {
-    SetError("vp8r_convert_to_i420_device: null engine, src or dst");
+    SetError(call + ": null engine, src or dst");
     return VP8R_ERR_INVALID_ARG;
   }
   if (n <= 0) {
-    SetError("vp8r_convert_to_i420_device: n <= 0");
+    SetError(call + ": n <= 0");
     return VP8R_ERR_INVALID_ARG;
   }
-  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
-    SetError("vp8r_convert_to_i420_device: unknown layout " + std::to_string(layout));
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (width < 1 || height < 1 || width > 16383 || height > 16383) {
-    SetError("vp8r_convert_to_i420_device: frame size outside 1..16383");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (src_stride < LayoutBytes(layout, width, height)) {
-    SetError("vp8r_convert_to_i420_device: stride smaller than a frame");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  if (dst_stride < LayoutBytes(VP8R_LAYOUT_I420, width, height)) {
-    SetError("vp8r_convert_to_i420_device: dst_stride smaller than an I420 frame");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  int rc = EnsureDevice(e);
+  int rc = CheckLayoutAndSize(call, layout, width, height);
+  if (!rc) rc = CheckStride(call + ": stride", src_stride, layout, width, height);
+  if (!rc) rc = CheckStride(call + ": dst_stride", dst_stride, VP8R_LAYOUT_I420, width, height);
+  if (!rc) rc = EnsureDevice(e);
   if (rc) return rc;
   if (!IsEngineDeviceMemory(e, src) || !IsEngineDeviceMemory(e, dst)) {
-    SetError("vp8r_convert_to_i420_device: src or dst is not device memory of the engine's device (pinned, pageable "
-             "and managed memory are refused)");
+    SetError(call + ": src or dst is not device memory of the engine's device (pinned, pageable and managed memory are "
+                    "refused)");
     return VP8R_ERR_INVALID_ARG;
   }
-  rc = EnsureScratchJobs(e, n);
-  if (rc) return rc;
-  int part = 0;
-  rc = AcquirePart(e, &part);
-  if (rc) return rc;
-  DevFrameJob *hj = e->h_cjobs + size_t(part) * e->cap_cjobs;
-  DevFrameJob *dj = e->d_cjobs + size_t(part) * e->cap_cjobs;
   const size_t cw = size_t(width + 1) / 2, ch = size_t(height + 1) / 2;
-  for (int i = 0; i < n; ++i) {
-    DevFrameJob &j = hj[i];
-    std::memset(&j, 0, sizeof(j));
-    uint8_t *d = static_cast<uint8_t *>(dst) + size_t(i) * dst_stride;
-    j.stage_src = static_cast<const uint8_t *>(src) + size_t(i) * src_stride;
-    j.pack_layout = uint8_t(layout);
-    j.width = j.stage_w = width;
-    j.height = j.stage_h = height;
-    j.enc_src[0] = d;
-    j.enc_src[1] = d + size_t(width) * height;
-    j.enc_src[2] = j.enc_src[1] + cw * ch;
-    j.enc_src_pitch_y = width;
-    j.enc_src_pitch_c = int(cw);
-  }
-  cudaStream_t user = static_cast<cudaStream_t>(stream);
-  const bool cross = user && user != e->st;
-  if (cross) {  // the source is written, and earlier work may still read dst, on the caller's stream
-    CU_TRY(cudaEventRecord(e->consumer_ev, user));
-    CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
-  }
-  CU_TRY(vp8r::LaunchCopy(dj, hj, sizeof(DevFrameJob) * n, e->st));
-  CU_TRY(vp8r::LaunchStageSource(dj, n, layout, width, height, e->st));
-  e->acc.launches_other++;
-  CU_TRY(cudaEventRecord(e->pack_done[part], e->st));
-  e->kernel_busy[part] = true;
-  if (cross) CU_TRY(cudaStreamWaitEvent(user, e->pack_done[part], 0));
-  return VP8R_OK;
+  int part;
+  // the source is written, and earlier work may still read dst, on the caller's stream
+  return RunOutputJobs(
+      e, n, Timer::kNone, static_cast<cudaStream_t>(stream), &part,
+      [&](int i, DevFrameJob &j) {
+        uint8_t *d = static_cast<uint8_t *>(dst) + size_t(i) * dst_stride;
+        j.stage_src = static_cast<const uint8_t *>(src) + size_t(i) * src_stride;
+        j.pack_layout = uint8_t(layout);
+        j.width = j.stage_w = width;
+        j.height = j.stage_h = height;
+        j.enc_src[0] = d;
+        j.enc_src[1] = d + size_t(width) * height;
+        j.enc_src[2] = j.enc_src[1] + cw * ch;
+        j.enc_src_pitch_y = width;
+        j.enc_src_pitch_c = int(cw);
+      },
+      [&](DevFrameJob *dj) { return vp8r::LaunchStageSource(dj, n, layout, width, height, e->st); });
 }
 
 VP8R_API size_t vp8r_stream_frame_bytes(const vp8r_stream *s) {
   if (!s || !s->have_frame) return 0;
-  size_t cw = size_t(s->width + 1) / 2, ch = size_t(s->height + 1) / 2;
-  return size_t(s->width) * s->height + 2 * cw * ch;
+  return LayoutBytes(VP8R_LAYOUT_I420, s->width, s->height);
 }
 
 VP8R_API int vp8r_stream_dims(const vp8r_stream *s, int *width, int *height) {
@@ -1479,13 +1519,14 @@ VP8R_API int vp8r_read_batch(vp8r_engine *e, int n, vp8r_stream *const *streams,
                              const size_t *cap, int async) {
   if (!e || n < 0 || (n > 0 && (!streams || !dst))) return VP8R_ERR_INVALID_ARG;
   int rc = EnsureDevice(e);
+  if (!rc) rc = CheckFrameStreams(e, n, streams);
   if (rc) return rc;
   {
-    ScopedTimer t(e, 4);
+    ScopedTimer t(e, Timer::kD2H);
     for (int i = 0; i < n; ++i) {
       const vp8r_stream *s = streams[i];
-      if (!s || s->eng != e || !s->have_frame || !dst[i]) {
-        SetError("stream has no reconstructed frame");
+      if (!dst[i]) {
+        SetError("null destination");
         return VP8R_ERR_STATE;
       }
       const size_t need = vp8r_stream_frame_bytes(s);
@@ -1515,62 +1556,37 @@ VP8R_API int vp8r_read_batch_packed_as(vp8r_engine *e, int n, vp8r_stream *const
                                        int async, int layout) {
   if (!e || n <= 0 || !streams || !dst || (layout != VP8R_LAYOUT_I420 && layout != VP8R_LAYOUT_NV12)) return VP8R_ERR_INVALID_ARG;
   int rc = EnsureDevice(e);
+  if (!rc) rc = CheckFrameStreams(e, n, streams, stride, layout);
   if (rc) return rc;
-  for (int i = 0; i < n; ++i) {
-    const vp8r_stream *s = streams[i];
-    if (!s || s->eng != e || !s->have_frame) {
-      SetError("stream has no reconstructed frame");
-      return VP8R_ERR_STATE;
-    }
-    if (vp8r_stream_frame_bytes(s) > stride) {
-      SetError("stride smaller than a frame");
-      return VP8R_ERR_INVALID_ARG;
-    }
-  }
   const size_t bytes = size_t(n) * stride;
   if (bytes > e->pack_cap) {
     CU_TRY(cudaStreamSynchronize(e->st));
     CU_TRY(cudaStreamSynchronize(e->st_copy));
     for (bool &b : e->copy_busy) b = false;
     for (bool &b : e->kernel_busy) b = false;
-    if (e->d_pack) cudaFree(e->d_pack);
-    e->d_pack = nullptr;
     const size_t half = (bytes + 255) & ~size_t(255);
-    CU_TRY(cudaMalloc(reinterpret_cast<void **>(&e->d_pack), vp8r_engine::kPackBufs * half + 256));
-    e->pack_cap = half;
+    CU_TRY(Regrow(&e->pack_cap, half, {DeviceBuf(&e->d_pack, vp8r_engine::kPackBufs * half + 256)}));
   }
-  rc = EnsureScratchJobs(e, n);
-  if (rc) return rc;
   // kPackBufs parts of the job table and of the staging buffer rotate: the pack kernel of this call
   // runs on the engine's stream while the D2H copy of the previous call may still be in flight on
   // the copy stream.
-  int half = 0;
-  rc = AcquirePart(e, &half);
+  int part = 0;
+  rc = RunOutputJobs(
+      e, n, Timer::kD2H, nullptr, &part,
+      [&](int i, DevFrameJob &j) {
+        FillJobSurfaces(streams[i], streams[i]->ref[0], &j);
+        j.pack_dst = e->d_pack + size_t(part) * e->pack_cap + size_t(i) * stride;
+        j.pack_layout = uint8_t(layout);
+      },
+      [&](DevFrameJob *dj) { return vp8r::LaunchPack(dj, n, e->st); });
   if (rc) return rc;
-  uint8_t *stage = e->d_pack + size_t(half) * e->pack_cap;
-  DevFrameJob *hj = e->h_cjobs + size_t(half) * e->cap_cjobs;
-  DevFrameJob *dj = e->d_cjobs + size_t(half) * e->cap_cjobs;
-  for (int i = 0; i < n; ++i) {
-    DevFrameJob &j = hj[i];
-    std::memset(&j, 0, sizeof(j));
-    FillJobSurfaces(streams[i], streams[i]->ref[0], &j);
-    j.pack_dst = stage + size_t(i) * stride;
-    j.pack_layout = uint8_t(layout);
-  }
-  {
-    ScopedTimer t(e, 4);
-    CU_TRY(vp8r::LaunchCopy(dj, hj, sizeof(DevFrameJob) * n, e->st));
-    CU_TRY(vp8r::LaunchPack(dj, n, e->st));
-    e->acc.launches_other++;
-  }
-  CU_TRY(cudaEventRecord(e->pack_done[half], e->st));
-  CU_TRY(cudaStreamWaitEvent(e->st_copy, e->pack_done[half], 0));
-  CU_TRY(cudaMemcpyAsync(dst, stage, bytes, cudaMemcpyDeviceToHost, e->st_copy));
-  CU_TRY(cudaEventRecord(e->copy_done[half], e->st_copy));
-  e->copy_busy[half] = true;
+  CU_TRY(cudaStreamWaitEvent(e->st_copy, e->pack_done[part], 0));
+  CU_TRY(cudaMemcpyAsync(dst, e->d_pack + size_t(part) * e->pack_cap, bytes, cudaMemcpyDeviceToHost, e->st_copy));
+  CU_TRY(cudaEventRecord(e->copy_done[part], e->st_copy));
+  e->copy_busy[part] = true;
   if (!async) {
     CU_TRY(cudaStreamSynchronize(e->st_copy));
-    e->copy_busy[half] = false;
+    e->copy_busy[part] = false;
   }
   return VP8R_OK;
 }
@@ -1578,74 +1594,38 @@ VP8R_API int vp8r_read_batch_packed_as(vp8r_engine *e, int n, vp8r_stream *const
 VP8R_API int vp8r_read_batch_device(vp8r_engine *e, int n, vp8r_stream *const *streams, void *dst, size_t stride,
                                     int layout, void *consumer_stream) {
   // argument checks that need no device come first
+  const std::string call = "vp8r_read_batch_device";
   if (!e || !streams || !dst) {
-    SetError("vp8r_read_batch_device: null engine, streams or destination");
+    SetError(call + ": null engine, streams or destination");
     return VP8R_ERR_INVALID_ARG;
   }
   if (n <= 0) {
-    SetError("vp8r_read_batch_device: n <= 0");
+    SetError(call + ": n <= 0");
     return VP8R_ERR_INVALID_ARG;
   }
-  if (layout < VP8R_LAYOUT_I420 || layout > VP8R_LAYOUT_RGB_PLANAR) {
-    SetError("vp8r_read_batch_device: unknown layout " + std::to_string(layout));
+  int rc = CheckLayoutAndSize(call, layout, 1, 1);  // the frames' sizes are the streams', checked as they were parsed
+  if (!rc) rc = CheckFrameStreams(e, n, streams, stride, layout);
+  if (!rc) rc = EnsureDevice(e);
+  if (rc) return rc;
+  if (!IsEngineDeviceMemory(e, dst)) {
+    SetError(call + ": dst is not device memory of the engine's device (pinned, pageable and managed memory are refused)");
     return VP8R_ERR_INVALID_ARG;
   }
   const bool rgb = layout == VP8R_LAYOUT_RGB24 || layout == VP8R_LAYOUT_RGB_PLANAR;
-  int max_w = 0, max_h = 0;
-  for (int i = 0; i < n; ++i) {
-    const vp8r_stream *s = streams[i];
-    if (!s || s->eng != e || !s->have_frame) {
-      SetError("stream has no reconstructed frame");
-      return VP8R_ERR_STATE;
-    }
-    const size_t bytes = rgb ? 3 * size_t(s->width) * s->height : vp8r_stream_frame_bytes(s);
-    if (bytes > stride) {
-      SetError("stride smaller than a frame");
-      return VP8R_ERR_INVALID_ARG;
-    }
-    max_w = std::max(max_w, s->width);
-    max_h = std::max(max_h, s->height);
-  }
-  int rc = EnsureDevice(e);
-  if (rc) return rc;
-  cudaPointerAttributes attr{};
-  if (cudaPointerGetAttributes(&attr, dst) != cudaSuccess) {
-    cudaGetLastError();
-    attr.type = cudaMemoryTypeUnregistered;
-  }
-  if (attr.type != cudaMemoryTypeDevice || attr.device != e->device) {
-    SetError("vp8r_read_batch_device: dst is not device memory of the engine's device (pinned, pageable and managed "
-             "memory are refused)");
-    return VP8R_ERR_INVALID_ARG;
-  }
-  rc = EnsureScratchJobs(e, n);
-  if (rc) return rc;
-  int part = 0;
-  rc = AcquirePart(e, &part);
-  if (rc) return rc;
-  DevFrameJob *hj = e->h_cjobs + size_t(part) * e->cap_cjobs;
-  DevFrameJob *dj = e->d_cjobs + size_t(part) * e->cap_cjobs;
-  for (int i = 0; i < n; ++i) {
-    DevFrameJob &j = hj[i];
-    std::memset(&j, 0, sizeof(j));
-    FillJobSurfaces(streams[i], streams[i]->ref[0], &j);
-    j.pack_dst = static_cast<uint8_t *>(dst) + size_t(i) * stride;
-    j.pack_layout = uint8_t(layout);
-  }
-  cudaStream_t consumer = static_cast<cudaStream_t>(consumer_stream);
-  const bool cross = consumer && consumer != e->st;
-  if (cross) {  // earlier consumer work may still read dst
-    CU_TRY(cudaEventRecord(e->consumer_ev, consumer));
-    CU_TRY(cudaStreamWaitEvent(e->st, e->consumer_ev, 0));
-  }
-  CU_TRY(vp8r::LaunchCopy(dj, hj, sizeof(DevFrameJob) * n, e->st));
-  if (rgb) CU_TRY(vp8r::LaunchConvertRgb(dj, n, max_w, max_h, e->st));
-  else CU_TRY(vp8r::LaunchPack(dj, n, e->st));
-  e->acc.launches_other++;
-  CU_TRY(cudaEventRecord(e->pack_done[part], e->st));
-  e->kernel_busy[part] = true;
-  if (cross) CU_TRY(cudaStreamWaitEvent(consumer, e->pack_done[part], 0));
-  return VP8R_OK;
+  int max_w = 0, max_h = 0, part;
+  // earlier consumer work may still read dst
+  return RunOutputJobs(
+      e, n, Timer::kNone, static_cast<cudaStream_t>(consumer_stream), &part,
+      [&](int i, DevFrameJob &j) {
+        FillJobSurfaces(streams[i], streams[i]->ref[0], &j);
+        j.pack_dst = static_cast<uint8_t *>(dst) + size_t(i) * stride;
+        j.pack_layout = uint8_t(layout);
+        max_w = std::max(max_w, j.width);
+        max_h = std::max(max_h, j.height);
+      },
+      [&](DevFrameJob *dj) {
+        return rgb ? vp8r::LaunchConvertRgb(dj, n, max_w, max_h, e->st) : vp8r::LaunchPack(dj, n, e->st);
+      });
 }
 
 VP8R_API int vp8r_stream_read_frame(vp8r_stream *s, uint8_t *dst, size_t cap) {
@@ -1659,26 +1639,21 @@ VP8R_API int vp8r_stream_read_frame(vp8r_stream *s, uint8_t *dst, size_t cap) {
 VP8R_API int vp8r_checksum_batch(vp8r_engine *e, int n, vp8r_stream *const *streams, uint64_t *out) {
   if (!e || n <= 0 || !streams || !out) return VP8R_ERR_INVALID_ARG;
   int rc = EnsureDevice(e);
+  if (!rc) rc = CheckFrameStreams(e, n, streams);
+  int part;
+  if (!rc)
+    rc = RunOutputJobs(
+        e, n, Timer::kNone, nullptr, &part,
+        [&](int i, DevFrameJob &j) {
+          FillJobSurfaces(streams[i], streams[i]->ref[0], &j);
+          j.checksum = e->d_sums + i;
+        },
+        [&](DevFrameJob *dj) {
+          const cudaError_t err = cudaMemsetAsync(e->d_sums, 0, sizeof(uint64_t) * n, e->st);
+          return err != cudaSuccess ? err : vp8r::LaunchChecksum(dj, n, e->st);
+        });
   if (rc) return rc;
-  // synchronous call: nothing queued may still read part 0 of the scratch job table
-  CU_TRY(cudaStreamSynchronize(e->st));
-  rc = EnsureScratchJobs(e, n);
-  if (rc) return rc;
-  for (int i = 0; i < n; ++i) {
-    const vp8r_stream *s = streams[i];
-    if (!s || s->eng != e || !s->have_frame) {
-      SetError("stream has no reconstructed frame");
-      return VP8R_ERR_STATE;
-    }
-    DevFrameJob &j = e->h_cjobs[i];
-    std::memset(&j, 0, sizeof(j));
-    FillJobSurfaces(s, s->ref[0], &j);
-    j.checksum = e->d_sums + i;
-  }
-  CU_TRY(cudaMemsetAsync(e->d_sums, 0, sizeof(uint64_t) * n, e->st));
-  CU_TRY(cudaMemcpyAsync(e->d_cjobs, e->h_cjobs, sizeof(DevFrameJob) * n, cudaMemcpyHostToDevice, e->st));
-  CU_TRY(vp8r::LaunchChecksum(e->d_cjobs, n, e->st));
-  e->acc.launches_other++;
+  // the checksum words are the engine's, not a part's: each call waits for its own
   CU_TRY(cudaMemcpyAsync(e->h_sums, e->d_sums, sizeof(uint64_t) * n, cudaMemcpyDeviceToHost, e->st));
   CU_TRY(cudaStreamSynchronize(e->st));
   for (int i = 0; i < n; ++i) out[i] = e->h_sums[i];
