@@ -320,7 +320,7 @@ VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *s
 /* vp8r_encode_inter_frames: one INTER frame for each of n different streams, from cropped I420 images in host memory
  * (the same conventions as vp8r_encode_key_frames).  Every macroblock predicts from the stream's current LAST frame
  * (made by vp8r_encode_key_frames, by an earlier inter encode or by decoding) with one motion vector; there are no
- * intra or SPLIT macroblocks.  On the device, one warp per macroblock: full-pel search over +-search_range whole pixels
+ * SPLIT macroblocks, and intra ones only with vp8r_encode_inter_frames_ex and VP8R_ENC_INTRA_MBS.  On the device, one warp per macroblock: full-pel search over +-search_range whole pixels
  * around the zero vector, then half-pel and quarter-pel refinement, by cost = luma SAD + lambda(q) * bits(vector)
  * (the lowest candidate index wins a tie), residual, forward DCT / WHT and quantisation; the decoder's own inter
  * reconstruction, loop filter and border extension then run on the records, so that stream k afterwards holds exactly
@@ -333,6 +333,27 @@ VP8R_API int vp8r_encode_key_frames(vp8r_engine *e, int n, vp8r_stream *const *s
 VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
                                       int width, int height, int q_index, int loop_filter_level, int sharpness,
                                       int search_range, vp8r_frame *const *out);
+/* vp8r_encode_inter_frames_ex / vp8r_encode_inter_frames_device_ex: vp8r_encode_inter_frames / _device with `flags`
+ * (flags 0: exactly those calls).
+ * VP8R_ENC_INTRA_MBS lets a macroblock be coded intra where prediction from LAST fails (scene cuts, objects entering
+ * the picture, content uncovered by motion).  Per macroblock, after the motion search and the inter reconstruction:
+ *   inter_err = luma sum of squared errors of the chosen vector's prediction against the source;
+ *   intra_err = the same for the best 16x16 mode (V, H, DC, TM, a later one only when strictly better), or, with
+ *               VP8R_ENC_BPRED, the B_PRED trial's total when that is strictly below it; predicted, as on a key frame,
+ *               from the frame's unfiltered reconstruction as it stands: inter neighbours as reconstructed, intra
+ *               neighbours as coded in this pass (127 above row 0, 129 left of column 0);
+ *   the macroblock is coded intra iff intra_err + bias(q) < inter_err (a tie stays inter), bias = vp8r_enc_intra_bias
+ *   of the luma AC factor (vp8_b200/csrc/cuda/enc_cost.h).
+ * The chroma mode of an intra macroblock is chosen as on a key frame; chroma plays no part in the decision.  An intra
+ * macroblock's record is exactly a key frame's: no VP8R_MB_IS_INTER, reference 0, vector 0, the luma and chroma modes,
+ * VP8R_MB_HAS_Y2 unless B_PRED (sub-modes in aux), the frame's filter level, VP8R_MB_LF_INNER iff it has coefficients
+ * or is B_PRED, blocks at 25*mb.  The other macroblocks get their modes as without the flag; n_inter_mbs counts them.
+ * VP8R_ENC_BPRED (only together with VP8R_ENC_INTRA_MBS) makes B_PRED a candidate for those intra macroblocks.
+ * VP8R_ERR_INVALID_ARG: the calls' checks, unknown flag bits, or VP8R_ENC_BPRED without VP8R_ENC_INTRA_MBS. */
+#define VP8R_ENC_INTRA_MBS 2u
+VP8R_API int vp8r_encode_inter_frames_ex(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
+                                         int width, int height, int q_index, int loop_filter_level, int sharpness,
+                                         int search_range, unsigned flags, vp8r_frame *const *out);
 /* ---- encoder input from device memory ----
  * Frames already on the GPU (decoded frames, a model's output, rendered images) encode without crossing PCIe.  The
  * source layouts are the VP8R_LAYOUT_* constants read as input formats: VP8R_LAYOUT_I420 (cropped Y, U, V planes back to
@@ -361,6 +382,10 @@ VP8R_API int vp8r_encode_key_frames_device(vp8r_engine *e, int n, vp8r_stream *c
 VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
                                              int layout, void *producer_stream, int width, int height, int q_index,
                                              int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out);
+VP8R_API int vp8r_encode_inter_frames_device_ex(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src,
+                                                size_t stride, int layout, void *producer_stream, int width, int height,
+                                                int q_index, int loop_filter_level, int sharpness, int search_range,
+                                                unsigned flags, vp8r_frame *const *out);
 /* The cropped I420 image (w*h + 2*ceil(w/2)*ceil(h/2) bytes) the encoder codes for each of n frames at src + i*src_stride
  * in `layout`, written to dst + i*dst_stride; src and dst device memory of the engine's device.  For PSNR against the
  * reconstruction of an RGB / NV12 source.  Asynchronous on the engine's stream, ordered against `stream` (the caller's

@@ -19,6 +19,10 @@ Reports, in one JSON document (--out):
 same bytes) or "rgb" (a CUDA tensor of RGB24 pictures, made from the I420 pictures in numpy by include/vp8r.h's
 YUV -> RGB formula).  A device input is uploaded before each call, outside the timed window; with "rgb" the PSNR is
 measured against the I420 the encoder codes (Engine.convert_to_i420).
+--intra-mbs lets the inter frames code macroblocks intra (Engine.encode_inter_frames(intra_mbs=True), B_PRED among the
+candidates); the time of that pass per call is read from the engine's intra timer during the profiled calls.
+--cut-every N replaces the picture of every stream with an unrelated scene (the texture turned by 180 degrees, and back)
+every N frames.
 --dry-run builds the pictures of the first two time steps and prints the plan without touching a device.
 """
 import argparse
@@ -37,7 +41,7 @@ import numpy as np  # noqa: E402
 class Scene:
     """Seeded moving scene of n streams: picture(s, t) is cropped I420 bytes."""
 
-    def __init__(self, n, w, h, steps, seed=2024):
+    def __init__(self, n, w, h, steps, seed=2024, cut_every=0):
         rng = np.random.default_rng(seed)
         self.w, self.h, self.n = w, h, n
         self.margin = 2 * steps + 40
@@ -45,6 +49,8 @@ class Scene:
         t = rng.integers(0, 256, (th + 2, tw + 2)).astype(np.float32)
         t = (t[:-2, :-2] + t[1:-1, :-2] + t[2:, :-2] + t[:-2, 1:-1] + 2 * t[1:-1, 1:-1] + t[2:, 1:-1] + t[:-2, 2:] + t[1:-1, 2:] + t[2:, 2:]) / 10
         self.tex = np.clip((t - 128) * 2.0 + 128, 0, 255).astype(np.uint8)
+        self.tex_cut = np.ascontiguousarray(self.tex[::-1, ::-1])
+        self.cut_every = cut_every
         self.vel = [(int(rng.integers(-2, 3)), int(rng.integers(-2, 3))) for _ in range(n)]
         self.off = [(int(rng.integers(0, 20)), int(rng.integers(0, 20))) for _ in range(n)]
         self.noise = [rng.integers(-2, 3, (h, w)).astype(np.int16) for _ in range(4)]
@@ -56,7 +62,8 @@ class Scene:
     def picture(self, s, t):
         (vy, vx), (oy, ox) = self.vel[s], self.off[s]
         y0, x0 = self.margin + oy + vy * t - 20, self.margin + ox + vx * t - 20
-        y = self.tex[y0:y0 + self.h, x0:x0 + self.w].astype(np.int16) + self.noise[(s + t) % 4]
+        tex = self.tex_cut if self.cut_every and (t // self.cut_every) % 2 else self.tex
+        y = tex[y0:y0 + self.h, x0:x0 + self.w].astype(np.int16) + self.noise[(s + t) % 4]
         rh, rw = self.h // 6, self.w // 6
         ry, rx = (self.h // 3 + 5 * t) % (self.h - rh), (self.w // 4 + 7 * t + 31 * s) % (self.w - rw)
         y[ry:ry + rh, rx:rx + rw] = 60 + 40 * ((np.arange(rw) // 6) % 2)
@@ -99,17 +106,19 @@ def main():
     ap.add_argument("--compare-streams", type=int, default=4, help="streams whose key-frame sizes and PSNR are measured")
     ap.add_argument("--profile-steps", type=int, default=3)
     ap.add_argument("--input", choices=("host", "i420", "rgb"), default="host", help="where the pictures come from")
+    ap.add_argument("--intra-mbs", action="store_true", help="intra macroblocks in inter frames")
+    ap.add_argument("--cut-every", type=int, default=0, help="an unrelated scene every N frames (0: never)")
     ap.add_argument("--out", default=None)
     ap.add_argument("--dry-run", action="store_true", help="build the pictures of two steps and print the plan; no device")
     args = ap.parse_args()
     if args.warmup >= args.inter:
         raise SystemExit("--warmup must be smaller than --inter")
     n, w, h = args.streams, args.width, args.height
-    scene = Scene(n, w, h, args.inter + 1)
+    scene = Scene(n, w, h, args.inter + 1, cut_every=args.cut_every)
     ncmp = min(args.compare_streams, n)
     plan = {"streams": n, "width": w, "height": h, "inter_frames_per_stream": args.inter, "timed_steps": args.inter - args.warmup,
             "q_index": args.q, "loop_filter_level": args.lf, "search_range": args.search_range, "compare_streams": ncmp,
-            "input": args.input}
+            "input": args.input, "intra_mbs": args.intra_mbs, "cut_every": args.cut_every}
     if args.dry_run:
         t0 = time.perf_counter()
         pics = [scene.picture(s, t) for t in range(2) for s in range(n)]
@@ -142,6 +151,7 @@ def main():
     key_streams = [eng.open_stream() for _ in range(ncmp)]
     fb_y = w * h
     step_s, inter_bytes, key_bytes, psnr = [], [], [], []
+    intra_mbs = all_mbs = 0
     try:
         src, _, layout = source([scene.picture(s, 0) for s in range(n)])
         for f in eng.encode_key_frames(streams, src, w, h, args.q, args.lf, layout=layout):
@@ -149,10 +159,15 @@ def main():
         for t in range(1, args.inter + 1):
             src, pics, layout = source([scene.picture(s, t) for s in range(n)])
             t0 = time.perf_counter()
-            frames = eng.encode_inter_frames(streams, src, w, h, args.q, args.lf, search_range=args.search_range, layout=layout)
+            frames = eng.encode_inter_frames(streams, src, w, h, args.q, args.lf, search_range=args.search_range, layout=layout,
+                                             intra_mbs=args.intra_mbs)
             dt = time.perf_counter() - t0
             if t > args.warmup:
                 step_s.append(dt)
+            for f in frames:
+                d = f.desc().hdr
+                intra_mbs += d.mb_cols * d.mb_rows - d.n_inter_mbs
+                all_mbs += d.mb_cols * d.mb_rows
             for s in range(ncmp):
                 inter_bytes.append(len(frames[s].write_bitstream()))
                 psnr.append(psnr_y(streams[s].read_frame(), pics[s], fb_y))
@@ -166,13 +181,17 @@ def main():
         # separate run under the profiler: kernel times of --profile-steps inter calls
         from torch.profiler import ProfilerActivity, profile
         src, _, layout = source([scene.picture(s, args.inter + 1) for s in range(n)])
+        eng.set_timing(True)
+        eng.timers(reset=True)
         with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
             t0 = time.perf_counter()
             for _ in range(args.profile_steps):
                 for f in eng.encode_inter_frames(streams, src, w, h, args.q, args.lf, search_range=args.search_range,
-                                                 layout=layout):
+                                                 layout=layout, intra_mbs=args.intra_mbs):
                     f.close()
             prof_wall = time.perf_counter() - t0
+        tm = eng.timers()
+        eng.set_timing(False)
         kernels, copies = {}, {}
         for ev in prof.key_averages():
             dev_us = getattr(ev, "self_device_time_total", None)
@@ -197,6 +216,8 @@ def main():
                     "rest_ms_per_call": 1e3 * prof_wall / args.profile_steps - kernel_ms,
                     "note": "rest = host padding and staging copies (host input), read-back copies, mode assignment (wall under the "
                             "profiler minus kernel time)"},
+        "intra_timer_ms_per_call": tm.ms_intra / args.profile_steps,
+        "intra_mb_fraction": intra_mbs / max(all_mbs, 1),
         "bytes_per_inter_frame": float(np.mean(inter_bytes)),
         "bytes_per_key_frame_same_pictures": float(np.mean(key_bytes)),
         "inter_over_key": float(np.mean(inter_bytes) / np.mean(key_bytes)),

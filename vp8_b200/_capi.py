@@ -81,6 +81,11 @@ SIGNATURES = {
     "vp8r_encode_inter_frames_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t, C.c_int,
                                                   C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                                   C.POINTER(C.c_void_p)]),
+    "vp8r_encode_inter_frames_ex": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int, C.c_int,
+                                              C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint, C.POINTER(C.c_void_p)]),
+    "vp8r_encode_inter_frames_device_ex": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t, C.c_int,
+                                                     C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint,
+                                                     C.POINTER(C.c_void_p)]),
     "vp8r_convert_to_i420_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_int,
                                               C.c_void_p, C.c_size_t, C.c_void_p]),
     "vp8r_frame_write_bitstream": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),

@@ -273,209 +273,292 @@ __device__ __forceinline__ unsigned BpredTrial(const DevFrameJob &job, int r, in
   return total;
 }
 
+// What one lane of an intra warp owns for the whole frame: lane b < 24 the 4x4 block b (16 Y raster, 4 U, 4 V),
+// lane 24 the Y2 block; the plane it predicts into and the source plane it reads; its quantiser factors.
+struct IntraLane {
+  bool luma, is_block;
+  int n4, first, bi, bj, pitch, spitch, n, f_dc, f_ac;
+  uint8_t *plane;
+  const uint8_t *splane;
+};
+
+__device__ __forceinline__ IntraLane MakeIntraLane(const DevFrameJob &job, int lane) {
+  IntraLane L;
+  L.luma = lane < 16;
+  L.n4 = L.luma ? 4 : 2;
+  L.first = L.luma ? 0 : (lane < 20 ? 16 : 20);
+  const int b = lane - L.first;
+  L.bi = L.luma ? (b >> 2) : (b >> 1);
+  L.bj = L.luma ? (b & 3) : (b & 1);
+  L.pitch = L.luma ? job.pitch_y : job.pitch_c;
+  L.spitch = L.luma ? job.enc_src_pitch_y : job.enc_src_pitch_c;
+  L.plane = L.luma ? job.cur.y : (lane < 20 ? job.cur.u : job.cur.v);
+  L.splane = L.luma ? job.enc_src[0] : (lane < 20 ? job.enc_src[1] : job.enc_src[2]);
+  L.n = L.luma ? 16 : 8;
+  L.is_block = lane < 24;
+  const int16_t *dq = job.dq[0];
+  L.f_dc = lane == 24 ? dq[VP8R_DQ_Y2_DC] : (L.luma ? dq[VP8R_DQ_Y1_DC] : dq[VP8R_DQ_UV_DC]);
+  L.f_ac = lane == 24 ? dq[VP8R_DQ_Y2_AC] : (L.luma ? dq[VP8R_DQ_Y1_AC] : dq[VP8R_DQ_UV_AC]);
+  return L;
+}
+
+// One macroblock of the closed-loop intra coder, by one warp, once its left, above-left, above and above-right
+// neighbours are final in job.cur: the mode decision on those neighbours, then the commit (residual, forward
+// transforms, quantisation, record and blocks, the decoder's reconstruction in place).  kGated (intra macroblocks of
+// inter frames): the commit happens only when the macroblock's intra error plus vp8r_enc_intra_bias is strictly below
+// inter_err; otherwise nothing of the frame is touched.  Returns whether it committed.
+template <bool kGated>
+__device__ __forceinline__ bool EncodeIntraMb(const DevFrameJob &job, const IntraLane &L, int lane, int r, int c, bool try_bpred,
+                                              EncScratch &s, const unsigned short *lut, unsigned inter_err) {
+  const bool luma = L.luma, is_block = L.is_block;
+  const int n4 = L.n4, first = L.first, bi = L.bi, bj = L.bj, pitch = L.pitch, spitch = L.spitch, n = L.n;
+  const int f_dc = L.f_dc, f_ac = L.f_ac;
+  const int cols = job.mb_cols;
+  short *const y2_slot = s.y2;
+  const int16_t *dq = job.dq[0];
+  uint8_t *mbp = L.plane + (ptrdiff_t)(r * n) * pitch + c * n;
+  const uint8_t *sp = L.splane + (ptrdiff_t)(r * n + 4 * bi) * spitch + c * n + 4 * bj;
+  const bool have_above = r > 0, have_left = c > 0;
+  unsigned src[4] = {0, 0, 0, 0}, aw = 0x7f7f7f7fu;
+  int l[4] = {129, 129, 129, 129};
+  int P = have_above ? (have_left ? 0 : 129) : 127;
+  if (is_block) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) src[k] = *reinterpret_cast<const unsigned *>(sp + (ptrdiff_t)k * spitch);
+    if (have_above) aw = *reinterpret_cast<const volatile unsigned *>(mbp - pitch + 4 * bj);
+    if (have_left) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) l[k] = *reinterpret_cast<const volatile uint8_t *>(mbp + (ptrdiff_t)(4 * bi + k) * pitch - 1);
+    }
+    if (have_above && have_left) P = *reinterpret_cast<const volatile uint8_t *>(mbp - pitch - 1);
+  }
+  // DC value: sums over the whole top edge / left edge of the plane's macroblock
+  int dc = 128;
+  {
+    const int sum_a = (int)__dp4a(aw, 0x01010101u, 0u), sum_l = l[0] + l[1] + l[2] + l[3];
+    int tot_a = 0, tot_l = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int va = __shfl_sync(0xffffffffu, sum_a, first + (k < n4 ? k : 0));
+      const int vl = __shfl_sync(0xffffffffu, sum_l, first + (k < n4 ? k * n4 : 0));
+      if (k < n4) {
+        tot_a += va;
+        tot_l += vl;
+      }
+    }
+    if (have_above || have_left) {
+      const int shf = (luma ? 3 : 2) + (have_above ? 1 : 0) + (have_left ? 1 : 0);
+      dc = ((have_above ? tot_a : 0) + (have_left ? tot_l : 0) + (1 << (shf - 1))) >> shf;
+    }
+  }
+  // ---- mode decision: V, H, DC, TM in the reference's order, a later one only when strictly better ----
+  int ymode = 0, uvmode = 0;
+  unsigned best_y = 0xffffffffu;
+  {
+    unsigned best_c = 0xffffffffu;
+    const int order[4] = {1, 2, 0, 3};
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      unsigned rows4[4];
+      PredictRows(order[k], aw, l, P, dc, rows4);
+      const unsigned e = is_block ? Sse4(rows4, src) : 0u;
+      const unsigned ey = __reduce_add_sync(0xffffffffu, luma ? e : 0u);
+      const unsigned ec = __reduce_add_sync(0xffffffffu, luma ? 0u : e);
+      if (ey < best_y) best_y = ey, ymode = order[k];
+      if (ec < best_c) best_c = ec, uvmode = order[k];
+    }
+  }
+  // ---- B_PRED last, only when strictly better than the best 16x16 mode (src/encode_frame.cc:233-237) ----
+  bool bpred = false;
+  unsigned aux[2] = {0, 0};
+  unsigned intra_err = best_y;
+  if (try_bpred) {
+    const int y1_dc = dq[VP8R_DQ_Y1_DC], y1_ac = dq[VP8R_DQ_Y1_AC];
+    const unsigned total = BpredTrial(job, r, c, lane, src, y1_dc, y1_ac, s, lut, aux);
+    bpred = total < best_y;
+    if (bpred) ymode = 4, intra_err = total;
+  }
+  // ---- intra or inter: strict, so a tie stays inter (warp-uniform: both errors are warp sums) ----
+  if (kGated && !(intra_err + (unsigned)vp8r_enc_intra_bias(dq[VP8R_DQ_Y1_AC]) < inter_err)) return false;
+  // ---- residual, forward transform, quantisation ----
+  unsigned pred[4];
+  PredictRows(luma ? ymode : uvmode, aw, l, P, dc, pred);
+  int m[16];
+  if (bpred && lane <= 24) {  // luma blocks were quantised in the trial (DC in place); there is no Y2 block
+#pragma unroll
+    for (int i = 0; i < 16; ++i) m[i] = (luma) ? s.cand[lane][i] : 0;
+  }
+  if (!(bpred && (luma || lane == 24))) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+#pragma unroll
+      for (int x = 0; x < 4; ++x) m[4 * k + x] = (int)((src[k] >> (8 * x)) & 0xff) - (int)((pred[k] >> (8 * x)) & 0xff);
+    if (is_block) Fdct4x4(m);
+  }
+  if (!bpred) {
+    if (luma) y2_slot[lane] = (short)m[0];
+    __syncwarp();
+    if (lane == 24) {
+#pragma unroll
+      for (int i = 0; i < 16; ++i) m[i] = y2_slot[i];
+      Fwht4x4(m);
+    }
+    __syncwarp();
+  }
+  bool nz = false;
+  if (lane <= 24) {
+    if (!(bpred && (luma || lane == 24))) {
+      m[0] = luma ? 0 : s16e(m[0] / f_dc);  // a luma block's DC travels in the Y2 block
+#pragma unroll
+      for (int i = 1; i < 16; ++i) m[i] = s16e(m[i] / f_ac);
+    }
+#pragma unroll
+    for (int i = 0; i < 16; ++i) nz |= m[i] != 0;
+  }
+  const unsigned lanes_nz = __ballot_sync(0xffffffffu, nz);
+  const unsigned coef_mask = ((lanes_nz & 0x00ffffffu) << 1) | ((lanes_nz >> 24) & 1u);
+  const int mb_index = r * cols + c;
+  const unsigned coef_offset = (unsigned)mb_index * 25u;
+  if (nz) {
+    const int blk = lane < 24 ? lane + 1 : 0;
+    const int at = __popc(coef_mask & ((1u << blk) - 1u));
+    int4 *dst = reinterpret_cast<int4 *>(const_cast<int16_t *>(job.payload) + (size_t)(coef_offset + at) * 16);
+    unsigned w[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) w[i] = ((unsigned)m[2 * i] & 0xffffu) | ((unsigned)m[2 * i + 1] << 16);
+    dst[0] = make_int4((int)w[0], (int)w[1], (int)w[2], (int)w[3]);
+    dst[1] = make_int4((int)w[4], (int)w[5], (int)w[6], (int)w[7]);
+  }
+  if (lane == 0) {
+    const unsigned flags = ((unsigned)ymode << VP8R_MB_MODE_SHIFT) | ((unsigned)uvmode << VP8R_MB_UVMODE_SHIFT) |
+                           (bpred ? 0u : VP8R_MB_HAS_Y2) | ((unsigned)job.lf_level << VP8R_MB_LF_SHIFT) |
+                           ((coef_mask || bpred) ? VP8R_MB_LF_INNER : 0u);
+    int4 *rec = reinterpret_cast<int4 *>(const_cast<vp8r_mb_info *>(job.mbs) + mb_index);
+    rec[0] = make_int4((int)flags, (int)coef_mask, (int)coef_offset, 0);
+    rec[1] = make_int4(bpred ? (int)aux[0] : 0, bpred ? (int)aux[1] : 0, 0, 0);
+  }
+  // ---- reconstruction, exactly as the decoder does it from the stored blocks (WarpResidual) ----
+  if (lane <= 24) {
+    m[0] = s16e(m[0] * f_dc);
+#pragma unroll
+    for (int i = 1; i < 16; ++i) m[i] = s16e(m[i] * f_ac);
+  }
+  bool any = nz && is_block;
+  if (bpred) {  // the luma reconstruction stands in the trial's tile
+    if (lane < 16) {
+      const unsigned *t = reinterpret_cast<const unsigned *>(&s.tile[1 + lane][4]);
+      *reinterpret_cast<uint4 *>(mbp + (ptrdiff_t)lane * pitch) = make_uint4(t[0], t[1], t[2], t[3]);
+    }
+  }
+  if (coef_mask & 1u) {
+    if (lane == 24) {
+      IwhtE(m);
+#pragma unroll
+      for (int i = 0; i < 16; ++i) y2_slot[i] = (short)m[i];
+    }
+    __syncwarp();
+    if (luma) {
+      m[0] = y2_slot[lane];
+      any = true;
+    }
+    __syncwarp();
+  }
+  if (is_block && !(bpred && luma)) {
+    if (any) IdctE(m);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      unsigned v = pred[k];
+      if (any) {
+        unsigned o = 0;
+#pragma unroll
+        for (int x = 0; x < 4; ++x) o |= (unsigned)clamp255e(s16e((int)((v >> (8 * x)) & 0xff) + m[4 * k + x])) << (8 * x);
+        v = o;
+      }
+      *reinterpret_cast<unsigned *>(mbp + (ptrdiff_t)(4 * bi + k) * pitch + 4 * bj) = v;
+    }
+  }
+  return true;
+}
+
+// Shared memory of the intra wavefront kernels: one progress word per macroblock row, the B_PRED gather table, then
+// one EncScratch per warp.
+__device__ __forceinline__ void IntraWavefrontSetup(const DevFrameJob &job, unsigned char *smem, volatile int *&progress,
+                                                    unsigned short *&lut, EncScratch *&scratch) {
+  const int rows = job.mb_rows;
+  progress = reinterpret_cast<volatile int *>(smem);
+  lut = reinterpret_cast<unsigned short *>(smem + ((rows * 4 + 15) & ~15));
+  scratch = reinterpret_cast<EncScratch *>(reinterpret_cast<unsigned char *>(lut) + 320);
+  for (int i = threadIdx.x; i < rows; i += blockDim.x) progress[i] = 0;
+  for (int i = threadIdx.x; i < 160; i += blockDim.x) lut[i] = c_enc_bpred_lut[i];
+  __syncthreads();
+}
+
+// Row r may work on column c once row r-1 has finished column c+1 (its above-right neighbour).
+__device__ __forceinline__ void WaitForRowAbove(volatile int *progress, int r, int c, int cols) {
+  if (r > 0) {
+    const int need = min(c + 2, cols);
+    while (progress[r - 1] < need) __nanosleep(100);
+    __threadfence_block();
+  }
+}
+
+__device__ __forceinline__ void PublishColumn(volatile int *progress, int r, int c, int lane) {
+  __syncwarp();
+  __threadfence_block();
+  if (lane == 0) progress[r] = c + 1;
+}
+
 }  // namespace
 
 __global__ void __launch_bounds__(kEncWarps * 32) EncodeIntraKernel(const DevFrameJob *__restrict__ jobs) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const DevFrameJob &job = jobs[blockIdx.x];
   if (!job.enc_src[0]) return;
-  const int rows = job.mb_rows, cols = job.mb_cols;
-  volatile int *progress = reinterpret_cast<volatile int *>(smem_raw);
-  unsigned short *lut = reinterpret_cast<unsigned short *>(smem_raw + ((rows * 4 + 15) & ~15));
-  EncScratch *scratch = reinterpret_cast<EncScratch *>(reinterpret_cast<unsigned char *>(lut) + 320);
-  for (int i = threadIdx.x; i < rows; i += blockDim.x) progress[i] = 0;
-  for (int i = threadIdx.x; i < 160; i += blockDim.x) lut[i] = c_enc_bpred_lut[i];
-  __syncthreads();
+  volatile int *progress;
+  unsigned short *lut;
+  EncScratch *scratch;
+  IntraWavefrontSetup(job, smem_raw, progress, lut, scratch);
   const bool try_bpred = (job.enc_flags & VP8R_ENC_BPRED) != 0;
-
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;  // from lane 0: known to be warp-uniform
-  short *const y2_slot = scratch[warp].y2;
-  vp8r_mb_info *const mbs = const_cast<vp8r_mb_info *>(job.mbs);
-  int16_t *const payload = const_cast<int16_t *>(job.payload);
-  // this lane's block
-  const bool luma = lane < 16;
-  const int n4 = luma ? 4 : 2;
-  const int first = luma ? 0 : (lane < 20 ? 16 : 20);
-  const int b = lane - first, bi = luma ? (b >> 2) : (b >> 1), bj = luma ? (b & 3) : (b & 1);
-  const int pitch = luma ? job.pitch_y : job.pitch_c, spitch = luma ? job.enc_src_pitch_y : job.enc_src_pitch_c;
-  uint8_t *const plane = luma ? job.cur.y : (lane < 20 ? job.cur.u : job.cur.v);
-  const uint8_t *const splane = luma ? job.enc_src[0] : (lane < 20 ? job.enc_src[1] : job.enc_src[2]);
-  const int n = luma ? 16 : 8;
-  const bool is_block = lane < 24;
-  // quantiser (= dequantiser) factors of this lane's block
-  const int16_t *dq = job.dq[0];
-  const int f_dc = lane == 24 ? dq[VP8R_DQ_Y2_DC] : (luma ? dq[VP8R_DQ_Y1_DC] : dq[VP8R_DQ_UV_DC]);
-  const int f_ac = lane == 24 ? dq[VP8R_DQ_Y2_AC] : (luma ? dq[VP8R_DQ_Y1_AC] : dq[VP8R_DQ_UV_AC]);
-  const unsigned lf_bits = (unsigned)job.lf_level << VP8R_MB_LF_SHIFT;
-
+  const IntraLane L = MakeIntraLane(job, lane);
+  const int rows = job.mb_rows, cols = job.mb_cols;
   for (int r = warp; r < rows; r += kEncWarps) {
     for (int c = 0; c < cols; ++c) {
-      // neighbours above and to the left must be reconstructed
-      if (r > 0) {
-        const int need = min(c + 2, cols);
-        while (progress[r - 1] < need) __nanosleep(100);
-        __threadfence_block();
+      WaitForRowAbove(progress, r, c, cols);
+      EncodeIntraMb<false>(job, L, lane, r, c, try_bpred, scratch[warp], lut, 0u);
+      PublishColumn(progress, r, c, lane);
+    }
+  }
+}
+
+// K_encode_intra_mbs: the intra macroblocks of inter frames (VP8R_ENC_INTRA_MBS).  Runs after K_encode_inter and
+// K_inter, on the unfiltered reconstruction they left, in EncodeIntraKernel's wavefront: a macroblock is decided on
+// its final neighbours (inter ones as K_inter made them, intra ones as this pass made them) and, when it goes intra,
+// overwrites its inter record, blocks and reconstruction in place.  No inter macroblock reads pixels of its own frame,
+// so nothing else changes.
+__global__ void __launch_bounds__(kEncWarps * 32) EncodeIntraMbsKernel(const DevFrameJob *__restrict__ jobs) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const DevFrameJob &job = jobs[blockIdx.x];
+  if (!job.enc_src[0] || !(job.enc_flags & VP8R_ENC_INTRA_MBS)) return;
+  volatile int *progress;
+  unsigned short *lut;
+  EncScratch *scratch;
+  IntraWavefrontSetup(job, smem_raw, progress, lut, scratch);
+  const bool try_bpred = (job.enc_flags & VP8R_ENC_BPRED) != 0;
+  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
+  const IntraLane L = MakeIntraLane(job, lane);
+  const int rows = job.mb_rows, cols = job.mb_cols;
+  const unsigned bias = (unsigned)vp8r_enc_intra_bias(job.dq[0][VP8R_DQ_Y1_AC]);
+  for (int r = warp; r < rows; r += kEncWarps) {
+    for (int c = 0; c < cols; ++c) {
+      const unsigned inter_err = job.enc_inter_err[r * cols + c];
+      // Skip rule: intra_err + bias >= bias >= inter_err can never win the strict comparison, so such a macroblock
+      // stays inter without a decision, and it reads no neighbour, so it need not wait for the row above either.
+      if (!(inter_err <= bias)) {
+        WaitForRowAbove(progress, r, c, cols);
+        EncodeIntraMb<true>(job, L, lane, r, c, try_bpred, scratch[warp], lut, inter_err);
       }
-      uint8_t *mbp = plane + (ptrdiff_t)(r * n) * pitch + c * n;
-      const uint8_t *sp = splane + (ptrdiff_t)(r * n + 4 * bi) * spitch + c * n + 4 * bj;
-      const bool have_above = r > 0, have_left = c > 0;
-      unsigned src[4] = {0, 0, 0, 0}, aw = 0x7f7f7f7fu;
-      int l[4] = {129, 129, 129, 129};
-      int P = have_above ? (have_left ? 0 : 129) : 127;
-      if (is_block) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) src[k] = *reinterpret_cast<const unsigned *>(sp + (ptrdiff_t)k * spitch);
-        if (have_above) aw = *reinterpret_cast<const volatile unsigned *>(mbp - pitch + 4 * bj);
-        if (have_left) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k) l[k] = *reinterpret_cast<const volatile uint8_t *>(mbp + (ptrdiff_t)(4 * bi + k) * pitch - 1);
-        }
-        if (have_above && have_left) P = *reinterpret_cast<const volatile uint8_t *>(mbp - pitch - 1);
-      }
-      // DC value: sums over the whole top edge / left edge of the plane's macroblock
-      int dc = 128;
-      {
-        const int sum_a = (int)__dp4a(aw, 0x01010101u, 0u), sum_l = l[0] + l[1] + l[2] + l[3];
-        int tot_a = 0, tot_l = 0;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const int va = __shfl_sync(0xffffffffu, sum_a, first + (k < n4 ? k : 0));
-          const int vl = __shfl_sync(0xffffffffu, sum_l, first + (k < n4 ? k * n4 : 0));
-          if (k < n4) {
-            tot_a += va;
-            tot_l += vl;
-          }
-        }
-        if (have_above || have_left) {
-          const int shf = (luma ? 3 : 2) + (have_above ? 1 : 0) + (have_left ? 1 : 0);
-          dc = ((have_above ? tot_a : 0) + (have_left ? tot_l : 0) + (1 << (shf - 1))) >> shf;
-        }
-      }
-      // ---- mode decision: V, H, DC, TM in the reference's order, a later one only when strictly better ----
-      int ymode = 0, uvmode = 0;
-      unsigned best_y = 0xffffffffu;
-      {
-        unsigned best_c = 0xffffffffu;
-        const int order[4] = {1, 2, 0, 3};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          unsigned rows4[4];
-          PredictRows(order[k], aw, l, P, dc, rows4);
-          const unsigned e = is_block ? Sse4(rows4, src) : 0u;
-          const unsigned ey = __reduce_add_sync(0xffffffffu, luma ? e : 0u);
-          const unsigned ec = __reduce_add_sync(0xffffffffu, luma ? 0u : e);
-          if (ey < best_y) best_y = ey, ymode = order[k];
-          if (ec < best_c) best_c = ec, uvmode = order[k];
-        }
-      }
-      // ---- B_PRED last, only when strictly better than the best 16x16 mode (src/encode_frame.cc:233-237) ----
-      bool bpred = false;
-      unsigned aux[2] = {0, 0};
-      if (try_bpred) {
-        const int y1_dc = dq[VP8R_DQ_Y1_DC], y1_ac = dq[VP8R_DQ_Y1_AC];
-        bpred = BpredTrial(job, r, c, lane, src, y1_dc, y1_ac, scratch[warp], lut, aux) < best_y;
-        if (bpred) ymode = 4;
-      }
-      // ---- residual, forward transform, quantisation ----
-      unsigned pred[4];
-      PredictRows(luma ? ymode : uvmode, aw, l, P, dc, pred);
-      int m[16];
-      if (bpred && lane <= 24) {  // luma blocks were quantised in the trial (DC in place); there is no Y2 block
-#pragma unroll
-        for (int i = 0; i < 16; ++i) m[i] = (luma) ? scratch[warp].cand[lane][i] : 0;
-      }
-      if (!(bpred && (luma || lane == 24))) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-#pragma unroll
-          for (int x = 0; x < 4; ++x) m[4 * k + x] = (int)((src[k] >> (8 * x)) & 0xff) - (int)((pred[k] >> (8 * x)) & 0xff);
-        if (is_block) Fdct4x4(m);
-      }
-      if (!bpred) {
-        if (luma) y2_slot[lane] = (short)m[0];
-        __syncwarp();
-        if (lane == 24) {
-#pragma unroll
-          for (int i = 0; i < 16; ++i) m[i] = y2_slot[i];
-          Fwht4x4(m);
-        }
-        __syncwarp();
-      }
-      bool nz = false;
-      if (lane <= 24) {
-        if (!(bpred && (luma || lane == 24))) {
-          m[0] = luma ? 0 : s16e(m[0] / f_dc);  // a luma block's DC travels in the Y2 block
-#pragma unroll
-          for (int i = 1; i < 16; ++i) m[i] = s16e(m[i] / f_ac);
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) nz |= m[i] != 0;
-      }
-      const unsigned lanes_nz = __ballot_sync(0xffffffffu, nz);
-      const unsigned coef_mask = ((lanes_nz & 0x00ffffffu) << 1) | ((lanes_nz >> 24) & 1u);
-      const int mb_index = r * cols + c;
-      const unsigned coef_offset = (unsigned)mb_index * 25u;
-      if (nz) {
-        const int blk = lane < 24 ? lane + 1 : 0;
-        const int at = __popc(coef_mask & ((1u << blk) - 1u));
-        int4 *dst = reinterpret_cast<int4 *>(payload + (size_t)(coef_offset + at) * 16);
-        unsigned w[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) w[i] = ((unsigned)m[2 * i] & 0xffffu) | ((unsigned)m[2 * i + 1] << 16);
-        dst[0] = make_int4((int)w[0], (int)w[1], (int)w[2], (int)w[3]);
-        dst[1] = make_int4((int)w[4], (int)w[5], (int)w[6], (int)w[7]);
-      }
-      if (lane == 0) {
-        const unsigned flags = ((unsigned)ymode << VP8R_MB_MODE_SHIFT) | ((unsigned)uvmode << VP8R_MB_UVMODE_SHIFT) |
-                               (bpred ? 0u : VP8R_MB_HAS_Y2) | lf_bits | ((coef_mask || bpred) ? VP8R_MB_LF_INNER : 0u);
-        int4 *rec = reinterpret_cast<int4 *>(mbs + mb_index);
-        rec[0] = make_int4((int)flags, (int)coef_mask, (int)coef_offset, 0);
-        rec[1] = make_int4(bpred ? (int)aux[0] : 0, bpred ? (int)aux[1] : 0, 0, 0);
-      }
-      // ---- reconstruction, exactly as the decoder does it from the stored blocks (WarpResidual) ----
-      if (lane <= 24) {
-        m[0] = s16e(m[0] * f_dc);
-#pragma unroll
-        for (int i = 1; i < 16; ++i) m[i] = s16e(m[i] * f_ac);
-      }
-      bool any = nz && is_block;
-      if (bpred) {  // the luma reconstruction stands in the trial's tile
-        if (lane < 16) {
-          const unsigned *t = reinterpret_cast<const unsigned *>(&scratch[warp].tile[1 + lane][4]);
-          *reinterpret_cast<uint4 *>(mbp + (ptrdiff_t)lane * pitch) = make_uint4(t[0], t[1], t[2], t[3]);
-        }
-      }
-      if (coef_mask & 1u) {
-        if (lane == 24) {
-          IwhtE(m);
-#pragma unroll
-          for (int i = 0; i < 16; ++i) y2_slot[i] = (short)m[i];
-        }
-        __syncwarp();
-        if (luma) {
-          m[0] = y2_slot[lane];
-          any = true;
-        }
-        __syncwarp();
-      }
-      if (is_block && !(bpred && luma)) {
-        if (any) IdctE(m);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          unsigned v = pred[k];
-          if (any) {
-            unsigned o = 0;
-#pragma unroll
-            for (int x = 0; x < 4; ++x) o |= (unsigned)clamp255e(s16e((int)((v >> (8 * x)) & 0xff) + m[4 * k + x])) << (8 * x);
-            v = o;
-          }
-          *reinterpret_cast<unsigned *>(mbp + (ptrdiff_t)(4 * bi + k) * pitch + 4 * bj) = v;
-        }
-      }
-      // publish
-      __syncwarp();
-      __threadfence_block();
-      if (lane == 0) progress[r] = c + 1;
+      PublishColumn(progress, r, c, lane);
     }
   }
 }
@@ -668,6 +751,16 @@ __global__ void __launch_bounds__(kEncInterWarps * 32) EncodeInterKernel(const D
     }
   }
   __syncwarp();
+  if (job.enc_flags & VP8R_ENC_INTRA_MBS) {  // inter_err: the luma squared error of the prediction, for K_encode_intra_mbs
+    unsigned e = 0;
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const unsigned d = __vabsdiffu4(s.pred[lane + 32 * k], s.src[lane + 32 * k]);
+      e = __dp4a(d, d, e);
+    }
+    e = __reduce_add_sync(0xffffffffu, e);
+    if (lane == 0) job.enc_inter_err[mb_r * cols + mb_c] = e;
+  }
 
   // ---- residual, forward transform, quantisation (lane b < 24: block b; lane 24: Y2) ----
   const bool luma = lane < 16, is_block = lane < 24;
@@ -748,6 +841,12 @@ cudaError_t InitEncodeTables(const unsigned short *bpred_lut) {
 cudaError_t LaunchEncodeIntra(const DevFrameJob *jobs, int n_frames, int max_rows, cudaStream_t st) {
   const size_t smem = ((size_t(max_rows) * 4 + 15) & ~size_t(15)) + 320 + sizeof(EncScratch) * kEncWarps;
   EncodeIntraKernel<<<n_frames, kEncWarps * 32, smem, st>>>(jobs);
+  return cudaGetLastError();
+}
+
+cudaError_t LaunchEncodeIntraMbs(const DevFrameJob *jobs, int n_frames, int max_rows, cudaStream_t st) {
+  const size_t smem = ((size_t(max_rows) * 4 + 15) & ~size_t(15)) + 320 + sizeof(EncScratch) * kEncWarps;
+  EncodeIntraMbsKernel<<<n_frames, kEncWarps * 32, smem, st>>>(jobs);
   return cudaGetLastError();
 }
 

@@ -82,6 +82,7 @@ struct DevFrameJob {
   const uint8_t *enc_src[3];
   int enc_src_pitch_y, enc_src_pitch_c;
   int enc_search_range;          // K_encode_inter: full-pel search range (whole pixels, 4..24)
+  uint32_t *enc_inter_err;       // VP8R_ENC_INTRA_MBS: per macroblock, the luma squared error of the inter prediction
   // StageSourceKernel: a width x height frame in pack_layout at stage_src (device memory, any alignment) becomes the
   // I420 planes enc_src[0..2] over stage_w x stage_h luma pixels (source coordinates clamped to the frame)
   const uint8_t *stage_src;
@@ -130,6 +131,9 @@ cudaError_t LaunchEncodeIntra(const DevFrameJob *jobs, int n_frames, int max_row
 // macroblock of every job with enc_src set, one warp per macroblock; writes records (vector, coef_mask, flags
 // without mode bits) and coefficient blocks.  K_inter, the loop filter and the border follow as for a decoded frame.
 cudaError_t LaunchEncodeInter(const DevFrameJob *jobs, int n_frames, int max_cols, int max_rows, cudaStream_t st);
+// K_encode_intra_mbs: intra macroblocks of the inter frames of jobs with VP8R_ENC_INTRA_MBS in enc_flags, after
+// K_encode_inter and K_inter and before the loop filter; the key-frame coder's wavefront, one CTA per frame.
+cudaError_t LaunchEncodeIntraMbs(const DevFrameJob *jobs, int n_frames, int max_rows, cudaStream_t st);
 // Up to eight frames with the same geometry and filter type (and a non-zero frame filter level) that one
 // warp of the batch loop filter walks together; unused slots are -1, slot 0 is always used.
 struct FilterGroup {

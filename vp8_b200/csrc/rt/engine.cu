@@ -758,10 +758,12 @@ int CheckFrameStreams(const vp8r_engine *e, int n, vp8r_stream *const *streams, 
   return VP8R_OK;
 }
 
-// The arguments of the four encoder calls, with a message naming the call for each refusal.  search_range < 0: a key-
-// frame call, which takes none.  The checks that need neither the engine nor a stream come first.
+// The arguments of the encoder calls, with a message naming the call for each refusal.  search_range < 0: a key-frame
+// call, which takes none (and whose flags are not checked).  The checks that need neither the engine nor a stream come
+// first.
 int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, vp8r_frame *const *out,
-                     int width, int height, int q_index, int loop_filter_level, int sharpness, int search_range) {
+                     int width, int height, int q_index, int loop_filter_level, int sharpness, int search_range,
+                     unsigned flags) {
   const std::string call = std::string(search_range < 0 ? "vp8r_encode_key_frames" : "vp8r_encode_inter_frames") +
                            (src.dev ? "_device" : "");
   if (!e || !streams || !(src.host || src.dev) || !out) {
@@ -783,6 +785,14 @@ int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const E
     SetError(call + ": search_range outside 4..24");
     return VP8R_ERR_INVALID_ARG;
   }
+  if (search_range >= 0 && (flags & ~(VP8R_ENC_INTRA_MBS | VP8R_ENC_BPRED))) {
+    SetError(call + "_ex: unknown flag bits");
+    return VP8R_ERR_INVALID_ARG;
+  }
+  if (search_range >= 0 && (flags & VP8R_ENC_BPRED) && !(flags & VP8R_ENC_INTRA_MBS)) {
+    SetError(call + "_ex: VP8R_ENC_BPRED needs VP8R_ENC_INTRA_MBS");
+    return VP8R_ERR_INVALID_ARG;
+  }
   rc = EnsureDevice(e);
   if (rc) return rc;
   rc = CheckBatchStreams(e, n, streams);
@@ -801,11 +811,11 @@ int CheckEncoderArgs(vp8r_engine *e, int n, vp8r_stream *const *streams, const E
 
 // An encoder batch: the header of its frames (the fields both encoders share; the caller adds its own) and the
 // layout of its slot arena.  Per frame the arena holds the source image padded to whole macroblocks (Y of pitch
-// cols*16, then U and V of pitch cols*8), the records the kernels write and their blocks (25 per macroblock), each
-// part 256-byte aligned.
+// cols*16, then U and V of pitch cols*8), the records the kernels write and their blocks (25 per macroblock), and one
+// uint32 per macroblock for the inter prediction's error (VP8R_ENC_INTRA_MBS), each part 256-byte aligned.
 struct EncodeLayout {
   vp8r_frame_hdr h{};
-  size_t n_mb = 0, src_bytes = 0, mb_bytes = 0, pay_bytes = 0, per_frame = 0;
+  size_t n_mb = 0, src_bytes = 0, mb_bytes = 0, pay_bytes = 0, err_at = 0, per_frame = 0;
 };
 EncodeLayout MakeEncodeLayout(int width, int height, int q_index, int loop_filter_level, int sharpness) {
   EncodeLayout L;
@@ -825,7 +835,8 @@ EncodeLayout MakeEncodeLayout(int width, int height, int q_index, int loop_filte
   L.src_bytes = (cols * 16 * rows * 16 + 2 * cols * 8 * rows * 8 + 255) & ~size_t(255);
   L.mb_bytes = (L.n_mb * sizeof(vp8r_mb_info) + 255) & ~size_t(255);
   L.pay_bytes = L.n_mb * 25 * 32;
-  L.per_frame = L.src_bytes + L.mb_bytes + ((L.pay_bytes + 255) & ~size_t(255));
+  L.err_at = L.src_bytes + L.mb_bytes + ((L.pay_bytes + 255) & ~size_t(255));
+  L.per_frame = L.err_at + ((L.n_mb * sizeof(uint32_t) + 255) & ~size_t(255));
   return L;
 }
 
@@ -920,7 +931,7 @@ int FinishEncoderBatch(vp8r_engine *e, const Slot &sl, int n, vp8r_stream *const
 // Row f4: closed-loop key-frame encoder (vp8r_encode_key_frames, _device).
 int EncodeKeyFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, int width, int height,
                     int q_index, int loop_filter_level, int sharpness, unsigned flags, vp8r_frame *const *out) {
-  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness, -1);
+  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness, -1, flags);
   if (rc) return rc;
   EncodeLayout L = MakeEncodeLayout(width, height, q_index, loop_filter_level, sharpness);
   L.h.key_frame = 1;
@@ -955,10 +966,12 @@ int EncodeKeyFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const En
 }
 
 // Row f4, inter frames: every macroblock predicts from LAST with one vector (K_encode_inter), the decoder's own
-// K_inter reconstructs from the records, then the loop filter and the border as for a decoded frame.
+// K_inter reconstructs from the records; with VP8R_ENC_INTRA_MBS, K_encode_intra_mbs then recodes as intra the
+// macroblocks that LAST predicts badly; then the loop filter and the border as for a decoded frame.
 int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const EncoderSource &src, int width, int height,
-                      int q_index, int loop_filter_level, int sharpness, int search_range, vp8r_frame *const *out) {
-  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness, search_range);
+                      int q_index, int loop_filter_level, int sharpness, int search_range, unsigned flags,
+                      vp8r_frame *const *out) {
+  int rc = CheckEncoderArgs(e, n, streams, src, out, width, height, q_index, loop_filter_level, sharpness, search_range, flags);
   if (rc) return rc;
   for (int i = 0; i < n; ++i) {
     const vp8r_stream *s = streams[i];
@@ -981,8 +994,11 @@ int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const 
   rc = StageEncoderSources(e, sl, n, streams, src, L, &cur);
   if (rc) return rc;
   for (int i = 0; i < n; ++i) {
-    sl.h_jobs[i].n_inter = int(L.n_mb);
-    sl.h_jobs[i].enc_search_range = search_range;
+    DevFrameJob &j = sl.h_jobs[i];
+    j.n_inter = int(L.n_mb);
+    j.enc_search_range = search_range;
+    j.enc_flags = uint8_t(flags);
+    if (flags & VP8R_ENC_INTRA_MBS) j.enc_inter_err = reinterpret_cast<uint32_t *>(sl.d_arena + L.per_frame * size_t(i) + L.err_at);
   }
   int n_groups = 0;
   rc = SubmitEncoderJobs(e, sl, n, src, L, &n_groups);
@@ -992,6 +1008,11 @@ int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const 
     CU_TRY(vp8r::LaunchEncodeInter(sl.d_jobs, n, cols, rows, e->st));
     CU_TRY(vp8r::LaunchInter(sl.d_jobs, n, cols, rows, e->st));
     e->acc.launches_inter += 2;
+  }
+  if (flags & VP8R_ENC_INTRA_MBS) {
+    ScopedTimer t(e, Timer::kIntra);
+    CU_TRY(vp8r::LaunchEncodeIntraMbs(sl.d_jobs, n, rows, e->st));
+    e->acc.launches_intra++;
   }
   rc = LaunchFilterAndBorder(e, sl, n, rows, n_groups);
   if (rc) return rc;
@@ -1005,7 +1026,10 @@ int EncodeInterFrames(vp8r_engine *e, int n, vp8r_stream *const *streams, const 
       SetError(err);
       return rc;
     }
-    out[i]->hdr.n_inter_mbs = uint32_t(L.n_mb);
+    uint32_t n_inter = 0;
+    const vp8r_mb_info *mbs = out[i]->mbs();
+    for (size_t m = 0; m < L.n_mb; ++m) n_inter += (mbs[m].flags & VP8R_MB_IS_INTER) ? 1u : 0u;
+    out[i]->hdr.n_inter_mbs = n_inter;
   }
   return VP8R_OK;
 }
@@ -1447,7 +1471,15 @@ VP8R_API int vp8r_encode_inter_frames(vp8r_engine *e, int n, vp8r_stream *const 
                                       int search_range, vp8r_frame *const *out) {
   EncoderSource src;
   src.host = i420;
-  return EncodeInterFrames(e, n, streams, src, width, height, q_index, loop_filter_level, sharpness, search_range, out);
+  return EncodeInterFrames(e, n, streams, src, width, height, q_index, loop_filter_level, sharpness, search_range, 0u, out);
+}
+
+VP8R_API int vp8r_encode_inter_frames_ex(vp8r_engine *e, int n, vp8r_stream *const *streams, const uint8_t *const *i420,
+                                         int width, int height, int q_index, int loop_filter_level, int sharpness,
+                                         int search_range, unsigned flags, vp8r_frame *const *out) {
+  EncoderSource src;
+  src.host = i420;
+  return EncodeInterFrames(e, n, streams, src, width, height, q_index, loop_filter_level, sharpness, search_range, flags, out);
 }
 
 VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src, size_t stride,
@@ -1458,7 +1490,19 @@ VP8R_API int vp8r_encode_inter_frames_device(vp8r_engine *e, int n, vp8r_stream 
   s.stride = stride;
   s.layout = layout;
   s.producer = static_cast<cudaStream_t>(producer_stream);
-  return EncodeInterFrames(e, n, streams, s, width, height, q_index, loop_filter_level, sharpness, search_range, out);
+  return EncodeInterFrames(e, n, streams, s, width, height, q_index, loop_filter_level, sharpness, search_range, 0u, out);
+}
+
+VP8R_API int vp8r_encode_inter_frames_device_ex(vp8r_engine *e, int n, vp8r_stream *const *streams, const void *src,
+                                                size_t stride, int layout, void *producer_stream, int width, int height,
+                                                int q_index, int loop_filter_level, int sharpness, int search_range,
+                                                unsigned flags, vp8r_frame *const *out) {
+  EncoderSource s;
+  s.dev = static_cast<const uint8_t *>(src);
+  s.stride = stride;
+  s.layout = layout;
+  s.producer = static_cast<cudaStream_t>(producer_stream);
+  return EncodeInterFrames(e, n, streams, s, width, height, q_index, loop_filter_level, sharpness, search_range, flags, out);
 }
 
 VP8R_API int vp8r_convert_to_i420_device(vp8r_engine *e, int n, const void *src, size_t src_stride, int layout, int width,

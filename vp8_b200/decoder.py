@@ -13,6 +13,7 @@ from ._capi import check
 
 
 DEVICE_LAYOUTS = {"i420": 0, "nv12": 1, "rgb": 2, "rgb_planar": 3}  # VP8R_LAYOUT_*
+ENC_BPRED, ENC_INTRA_MBS = 1, 2  # VP8R_ENC_BPRED, VP8R_ENC_INTRA_MBS
 
 
 def _is_tensor(x):
@@ -130,17 +131,21 @@ class Engine:
         torch.uint8 CUDA tensor on the engine's device with one frame per stream along its first dimension, in `layout`
         (see _device_source); it is read on the device, ordered behind the work queued on torch's current stream."""
         return self._encode(self._lib.vp8r_encode_key_frames, self._lib.vp8r_encode_key_frames_device, streams, images,
-                            layout, width, height, q_index, loop_filter_level, sharpness, 1 if bpred else 0)
+                            layout, width, height, q_index, loop_filter_level, sharpness, ENC_BPRED if bpred else 0)
 
     def encode_inter_frames(self, streams, images, width, height, q_index, loop_filter_level=0, sharpness=0, search_range=16,
-                            layout="i420"):
+                            layout="i420", intra_mbs=False, bpred=True):
         """One inter frame per stream from cropped I420 images (bytes): every macroblock predicts from the stream's
         current LAST frame with one motion vector, searched on the device over +-search_range whole pixels (4..24) and
-        refined to quarter pel (vp8r_encode_inter_frames).  Returns the ParsedFrame objects (records with modes and
-        vectors, coefficient blocks; .write_bitstream() serialises them); every stream then holds the reconstructed
-        frame a decoder would produce.  `images` and `layout` as for encode_key_frames."""
-        return self._encode(self._lib.vp8r_encode_inter_frames, self._lib.vp8r_encode_inter_frames_device, streams, images,
-                            layout, width, height, q_index, loop_filter_level, sharpness, search_range)
+        refined to quarter pel (vp8r_encode_inter_frames_ex).  intra_mbs: a macroblock that LAST predicts worse than
+        intra prediction does, by more than a bias of the quantiser, is coded intra instead (VP8R_ENC_INTRA_MBS), with
+        B_PRED among its candidates when bpred is set (VP8R_ENC_BPRED); bpred is ignored without intra_mbs.  Returns the
+        ParsedFrame objects (records with modes and vectors, coefficient blocks; .write_bitstream() serialises them);
+        every stream then holds the reconstructed frame a decoder would produce.  `images` and `layout` as for
+        encode_key_frames."""
+        flags = (ENC_INTRA_MBS | (ENC_BPRED if bpred else 0)) if intra_mbs else 0
+        return self._encode(self._lib.vp8r_encode_inter_frames_ex, self._lib.vp8r_encode_inter_frames_device_ex, streams,
+                            images, layout, width, height, q_index, loop_filter_level, sharpness, search_range, flags)
 
     def _encode(self, fn, fn_device, streams, images, layout, width, height, *params):
         """Calls the C encoder entry point on one picture per stream: fn(engine, n, streams, images, width, height,
@@ -364,9 +369,11 @@ def decode_ivf(path_or_bytes, engine=None, layout=None):
 
 
 def encode_ivf(images, width, height, q_index, path=None, key_interval=0, loop_filter_level=0, sharpness=0, bpred=True,
-               search_range=16, engine=None, layout="i420"):
+               search_range=16, engine=None, layout="i420", intra_mbs=False):
     """Encodes one stream of cropped I420 images (bytes) into an IVF file, the mirror of decode_ivf: a key frame first
-    and then every key_interval frames (0: only the first), inter frames between them.  Returns the IVF bytes and
+    and then every key_interval frames (0: only the first), inter frames between them.  intra_mbs: the inter frames
+    may code macroblocks intra where LAST predicts them badly (see Engine.encode_inter_frames); bpred then applies to
+    those macroblocks as well.  Returns the IVF bytes and
     writes them to `path` when one is given.  `images` may instead be a (T, ...) torch.uint8 CUDA tensor of T frames in
     `layout` (see Engine.encode_key_frames), such as decode_ivf(..., layout="i420") returns: no pixel then crosses PCIe."""
     from .ivf import ivf_bytes
@@ -384,7 +391,7 @@ def encode_ivf(images, width, height, q_index, path=None, key_interval=0, loop_f
                                                 layout=layout)
             else:
                 (f,) = engine.encode_inter_frames([st], img, width, height, q_index, loop_filter_level, sharpness,
-                                                  search_range, layout=layout)
+                                                  search_range, layout=layout, intra_mbs=intra_mbs, bpred=bpred)
             payloads.append(f.write_bitstream())
             f.close()
     finally:
